@@ -10,6 +10,10 @@ Multi-GPU is STRONG scaling, the metric BASELINE.json states ("8 GPU, 200-config
 over the ranks exactly as mpcmmd_b200/driver.py::shard does (rank r solves k = r, r + W, ...), no data-path collective; the only
 exchange is the NCCL all_gather of the 26-float per-episode record.  `--scaling weak` (200 episodes per GPU) is kept as an option
 and its value is reported under `weak_scaling` in the same line.  Prints ONE JSON line on rank 0.
+
+`--dump-outputs DIR` writes what the timed path returned in its last timed step (cx, cy, cost_lane, cost_obs, beta, sigma, res_beta of
+every cost function) as DIR/<cost>_<field>.npy.  The inputs are generated from fixed seeds, so two builds run with the same arguments
+can be compared output for output.
 """
 from __future__ import annotations
 
@@ -28,6 +32,7 @@ ROOT = os.path.dirname(os.path.abspath(__file__))
 for p in (ROOT, os.path.join(ROOT, "mpc-mmd_b200")):
     if p not in sys.path:
         sys.path.insert(1, p)
+sys.dont_write_bytecode = True         # the benchmark writes nothing into the tree it runs from (which may be read-only)
 
 WORK = dict(num_reduced=5, num_obs=4, noise_level=0.3, num_prime=50, noise="beta", acc_const_noise=0.0, steer_const_noise=0.0)
 COSTS = ("cvar", "mmd_opt")
@@ -174,6 +179,25 @@ def traffic_per_launch():
         return None, None
 
 
+DUMP_CAP_BYTES = 64 << 20
+
+
+def write_outputs(out_dir, arrays, cap=DUMP_CAP_BYTES):
+    """--dump-outputs: each array (one row per episode, the same rows in all) as out_dir/<name>.npy in float32.  Above `cap` bytes in all,
+    every array keeps the same seeded sample of rows and the kept row indices go to out_dir/rows.npy (float64)."""
+    arrays = {k: np.ascontiguousarray(v, dtype=np.float32) for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > cap:
+        n = next(iter(arrays.values())).shape[0]
+        rows = np.sort(np.random.default_rng(0).choice(n, int(cap // (total / n + 8)), replace=False))
+        arrays = {k: a[rows] for k, a in arrays.items()}
+        arrays["rows"] = rows.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
+    return sorted(arrays)
+
+
 def main():
     # The contract is ONE JSON line on stdout.  Libraries write there too (NCCL prints its version banner to stdout), so everything
     # except the final line is routed to stderr: fd 1 is pointed at fd 2 for the run and the line goes to the saved descriptor.
@@ -198,7 +222,14 @@ def main():
     ap.add_argument("--workload", default="cfg2", choices=sorted(WORKLOADS))
     ap.add_argument("--projection", default="exact", choices=["exact", "tc"],
                     help="exact = k_project (bit-exact FP32, the default product path); tc = k_project_tc (tcgen05 kind::tf32 products, 1e-4 stage parity)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the solver returned in the last one as DIR/<cost>_<field>.npy (float32; row i = "
+                         "episode i of the sweep; with several ranks DIR/rank<r>/, row i = the rank's i-th episode)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "native":
+        ap.error("--dump-outputs writes the outputs of the native (CUDA) path")
     if args.projection == "tc":
         os.environ["MPCMMD_PROJ"] = "tc"          # read by mpcmmd_create
     else:
@@ -291,6 +322,7 @@ def main():
         def step_device(self):
             cur = torch.cuda.current_stream(dev)
             outs = {}
+            self.last_outs = outs                                       # what the solver handed back in this step (--dump-outputs)
             if not self.concurrent:
                 for cost in COSTS:
                     outs[cost] = self.probs[cost].solve_batch_device(cost, *[self.dev_in[k] for k in keys])
@@ -348,6 +380,9 @@ def main():
         ms_total, t_wall, recs, launches_per_step = arm.time_device(K, W)
     value = arm.total_solves * K / (ms_total * 1e-3)
     accepted = {c: int(recs[c][:, 1].sum().item()) for c in COSTS}
+    if args.dump_outputs:
+        write_outputs(args.dump_outputs if world == 1 else os.path.join(args.dump_outputs, "rank%d" % rank),
+                      {"%s_%s" % (c, f): v.cpu().numpy() for c, o in arm.last_outs.items() for f, v in o.items() if not f.startswith("_")})
 
     # ---- end to end through the host-buffer C ABI call (`e2e`): pinned host inputs, H2D + D2H inside the timed region
     for _ in range(2):

@@ -42,6 +42,34 @@ def test_reference_arm_prints_the_contract_line():
     assert d["e2e"] == {"value": d["value"], "unit": "solves/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
 
 
+def test_dump_outputs_writes_float32_and_samples_rows_above_the_cap(tmp_path):
+    """--dump-outputs: one float32 .npy per array; above the byte cap every array keeps the same seeded rows, listed in rows.npy"""
+    import numpy as np
+    b = _bench()
+    rng = np.random.default_rng(1)
+    arrays = {"cvar_cx": rng.normal(size=(200, 11)).astype(np.float32), "cvar_cost_obs": rng.normal(size=200).astype(np.float32)}
+    assert b.write_outputs(str(tmp_path / "all"), arrays) == ["cvar_cost_obs", "cvar_cx"]
+    for k, v in arrays.items():
+        got = np.load(tmp_path / "all" / (k + ".npy"))
+        assert got.dtype == np.float32 and np.array_equal(got, v)
+    cap = 2000
+    names = [b.write_outputs(str(tmp_path / d), arrays, cap=cap) for d in ("a", "b")]
+    assert names[0] == names[1] == ["cvar_cost_obs", "cvar_cx", "rows"]
+    rows = np.load(tmp_path / "a" / "rows.npy")
+    assert rows.dtype == np.float64 and np.array_equal(rows, np.load(tmp_path / "b" / "rows.npy"))
+    assert sum((tmp_path / "a" / (k + ".npy")).stat().st_size - 128 for k in names[0]) <= cap
+    r = rows.astype(int)
+    assert len(r) > 0 and np.all(np.diff(r) > 0)
+    for k, v in arrays.items():
+        assert np.array_equal(np.load(tmp_path / "a" / (k + ".npy")), v[r])
+
+
+def test_bad_arguments_are_refused():
+    for argv in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", "out"]):
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + argv, capture_output=True, text=True, timeout=120)
+        assert out.returncode == 2 and out.stdout.strip() == "", (argv, out.stderr[-500:])
+
+
 def test_reference_arm_other_ranks_exit_quietly():
     env = dict(os.environ, RANK="1", WORLD_SIZE="2")
     out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "1", "--warmup", "0"],
