@@ -126,6 +126,21 @@ int mpcmmd_validate_host(int device, int n_ep, int n_roll, int num_prime, int nu
                          const double *state0, const double *x_obs_traj, const double *y_obs_traj, int32_t *count,
                          int32_t *count_lane, double *x_roll, double *y_roll);
 
+/* The same validation with the noise drawn ON THE DEVICE (k_validate_noise): trajectory i's controls are perturbed with the draws of
+ * np.random.seed(seed[i]) in the order of validation.py:43-84, restated in csrc/dnprng.cuh (DESIGN.md section 3 item 6).  Stream
+ * consumption is NumPy's exactly; values differ from NumPy's only where CUDA's double pow / log / exp round differently from glibc's.
+ * noise_kind 0 gaussian, 1 beta.  acc_plan, steer_plan (n_ep, num_prime) are the planned controls; the other inputs and the counts as
+ * mpcmmd_validate_host.  Beta noise checks every shape parameter as np.random.beta does and fails with "a <= 0" / "b <= 0" before
+ * anything runs.  Optional outputs (NULL to skip): acc_out, steer_out (n_ep, n_roll, num_prime) the perturbed controls (both or
+ * neither); state_out (n_ep, 628) each stream after its last draw: key[624], pos, has_gauss, cached gauss as float64 bits (low word
+ * first) = np.random.get_state()[1:].  All pointers are HOST pointers.  Synchronous. */
+int mpcmmd_validate_seeded_host(int device, int n_ep, int n_roll, int num_prime, int num_obs, int obs_cost_f32, int noise_kind,
+                                double noise_level, double k_steer, double beta_a, double beta_b, double acc_const_noise,
+                                double steer_const_noise, double dt, double wheel_base, double a_obs, double b_obs, double y_lb,
+                                double y_ub, const uint32_t *seed, const double *acc_plan, const double *steer_plan,
+                                const double *state0, const double *x_obs_traj, const double *y_obs_traj, int32_t *count,
+                                int32_t *count_lane, double *acc_out, double *steer_out, uint32_t *state_out);
+
 /* Measured FP32 FMA throughput of the device (TFLOP/s, FMA = 2 flops): the roofline denominator of the FP32-bound kernels. */
 int mpcmmd_fp32_peak(int device, float *tflops, int *sm_count);
 /* Measured special-function-unit peaks (thread-level operations per second / 1e9): gops[0] = ex2.approx (MUFU.EX2), gops[1] = IEEE

@@ -21,6 +21,7 @@
 #include "k_inner_big.cuh"
 #include "k_select.cuh"
 #include "k_validate.cuh"
+#include "k_validate_noise.cuh"
 
 static thread_local std::string g_err;
 static int fail(const std::string& m) { g_err = m; return -1; }
@@ -946,6 +947,22 @@ extern "C" int mpcmmd_stage_noise(mpcmmd_handle h, int32_t idx_mpc, int32_t iter
 
 // ------------------------------------------------------------------------------------------------
 // Monte-Carlo validation (S/validation.py:134-171): host arrays in, counts out.  Not tied to a handle.
+// k_validate on device arrays: the rollout + counting half shared by both validation entry points (enqueue only).
+static cudaError_t launch_validate(int n_ep, int n_roll, int num_prime, int num_obs, int obs_cost_f32, double dt, double wheel_base, double a_obs,
+                                   double b_obs, double y_lb, double y_ub, size_t smem, const double* d_acc, const double* d_steer,
+                                   const double* d_s0, const double* d_xo, const double* d_yo, int32_t* d_cnt, int32_t* d_lane,
+                                   double* d_xr, double* d_yr) {
+    if (smem > 48 * 1024) {
+        const cudaError_t e = cudaFuncSetAttribute(k_validate, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (e != cudaSuccess) return e;
+    }
+    ValCfg c;
+    c.n_roll = n_roll; c.np = num_prime; c.O = num_obs; c.obs_f32 = obs_cost_f32; c.dt = dt; c.wheel_base = wheel_base;
+    c.a2 = a_obs * a_obs; c.b2 = b_obs * b_obs; c.y_lb = y_lb; c.y_ub = y_ub;
+    k_validate<<<n_ep, VAL_THREADS, smem>>>(c, d_acc, d_steer, d_s0, d_xo, d_yo, d_cnt, d_lane, d_xr, d_yr);
+    return cudaGetLastError();
+}
+
 extern "C" int mpcmmd_validate_host(int device, int n_ep, int n_roll, int num_prime, int num_obs, int obs_cost_f32, double dt, double wheel_base,
                                     double a_obs, double b_obs, double y_lb, double y_ub, const double* acc, const double* steer,
                                     const double* state0, const double* x_obs_traj, const double* y_obs_traj, int32_t* count,
@@ -959,7 +976,6 @@ extern "C" int mpcmmd_validate_host(int device, int n_ep, int n_roll, int num_pr
     const size_t smem = (size_t)(num_obs + 2) * num_prime * sizeof(int);
     if (smem > 200 * 1024) return fail("mpcmmd_validate_host: (num_obs + 2) * num_prime counters do not fit in shared memory");
     CK(cudaSetDevice(device));
-    if (smem > 48 * 1024) CK(cudaFuncSetAttribute(k_validate, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     const size_t nc = (size_t)n_ep * n_roll * num_prime, no = (size_t)n_ep * num_obs * num_prime;
     double *d_acc = nullptr, *d_steer = nullptr, *d_s0 = nullptr, *d_xo = nullptr, *d_yo = nullptr, *d_xr = nullptr, *d_yr = nullptr;
     int32_t *d_cnt = nullptr, *d_lane = nullptr;
@@ -971,17 +987,69 @@ extern "C" int mpcmmd_validate_host(int device, int n_ep, int n_roll, int num_pr
         CK(cudaMemcpy(d_acc, acc, nc * 8, cudaMemcpyHostToDevice)); CK(cudaMemcpy(d_steer, steer, nc * 8, cudaMemcpyHostToDevice));
         CK(cudaMemcpy(d_s0, state0, (size_t)n_ep * 5 * 8, cudaMemcpyHostToDevice));
         CK(cudaMemcpy(d_xo, x_obs_traj, no * 8, cudaMemcpyHostToDevice)); CK(cudaMemcpy(d_yo, y_obs_traj, no * 8, cudaMemcpyHostToDevice));
-        ValCfg c;
-        c.n_roll = n_roll; c.np = num_prime; c.O = num_obs; c.obs_f32 = obs_cost_f32; c.dt = dt; c.wheel_base = wheel_base;
-        c.a2 = a_obs * a_obs; c.b2 = b_obs * b_obs; c.y_lb = y_lb; c.y_ub = y_ub;
-        k_validate<<<n_ep, VAL_THREADS, smem>>>(c, d_acc, d_steer, d_s0, d_xo, d_yo, d_cnt, d_lane, d_xr, d_yr);
-        CK(cudaGetLastError());
+        CK(launch_validate(n_ep, n_roll, num_prime, num_obs, obs_cost_f32, dt, wheel_base, a_obs, b_obs, y_lb, y_ub, smem,
+                           d_acc, d_steer, d_s0, d_xo, d_yo, d_cnt, d_lane, d_xr, d_yr));
         CK(cudaMemcpy(count, d_cnt, (size_t)n_ep * 4, cudaMemcpyDeviceToHost)); CK(cudaMemcpy(count_lane, d_lane, (size_t)n_ep * 4, cudaMemcpyDeviceToHost));
         if (x_roll) { CK(cudaMemcpy(x_roll, d_xr, nc * 8, cudaMemcpyDeviceToHost)); CK(cudaMemcpy(y_roll, d_yr, nc * 8, cudaMemcpyDeviceToHost)); }
         return 0;
     };
     rc = body();
     cudaFree(d_acc); cudaFree(d_steer); cudaFree(d_s0); cudaFree(d_xo); cudaFree(d_yo); cudaFree(d_cnt); cudaFree(d_lane); cudaFree(d_xr); cudaFree(d_yr);
+    return rc;
+}
+
+// The same with the noise drawn on the device (k_validate_noise): planned controls and per-trajectory seeds in, counts out.
+extern "C" int mpcmmd_validate_seeded_host(int device, int n_ep, int n_roll, int num_prime, int num_obs, int obs_cost_f32, int noise_kind,
+                                           double noise_level, double k_steer, double beta_a, double beta_b, double acc_const_noise,
+                                           double steer_const_noise, double dt, double wheel_base, double a_obs, double b_obs, double y_lb,
+                                           double y_ub, const uint32_t* seed, const double* acc_plan, const double* steer_plan,
+                                           const double* state0, const double* x_obs_traj, const double* y_obs_traj, int32_t* count,
+                                           int32_t* count_lane, double* acc_out, double* steer_out, uint32_t* state_out) {
+    int ndev = 0;
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) return fail("mpcmmd_validate_seeded_host: no CUDA device (this library has no CPU fallback)");
+    if (device < 0 || device >= ndev) return fail("mpcmmd_validate_seeded_host: bad device index");
+    if (n_ep < 1 || n_roll < 1 || num_prime < 1 || num_prime > MPCMMD_T || num_obs < 1) return fail("mpcmmd_validate_seeded_host: bad sizes");
+    if (noise_kind != 0 && noise_kind != 1) return fail("mpcmmd_validate_seeded_host: noise_kind must be 0 (gaussian) or 1 (beta)");
+    if (!seed || !acc_plan || !steer_plan || !state0 || !x_obs_traj || !y_obs_traj || !count || !count_lane)
+        return fail("mpcmmd_validate_seeded_host: null pointer");
+    if ((acc_out == nullptr) != (steer_out == nullptr)) return fail("mpcmmd_validate_seeded_host: acc_out and steer_out must both be given or both be null");
+    if (noise_kind == 1) {                               // np.random.beta's argument check (NaN passes), before anything is drawn
+        for (size_t i = 0; i < (size_t)n_ep * num_prime; i++) {
+            if (beta_a * fabs(acc_plan[i]) <= 0.0 || beta_a * fabs(steer_plan[i]) + 1e-5 <= 0.0) return fail("mpcmmd_validate_seeded_host: a <= 0");
+            if (beta_b * fabs(acc_plan[i]) <= 0.0 || beta_b * fabs(steer_plan[i]) + 1e-5 <= 0.0) return fail("mpcmmd_validate_seeded_host: b <= 0");
+        }
+    }
+    const size_t smem = (size_t)(num_obs + 2) * num_prime * sizeof(int);
+    if (smem > 200 * 1024) return fail("mpcmmd_validate_seeded_host: (num_obs + 2) * num_prime counters do not fit in shared memory");
+    CK(cudaSetDevice(device));
+    const size_t nc = (size_t)n_ep * n_roll * num_prime, no = (size_t)n_ep * num_obs * num_prime, npl = (size_t)n_ep * num_prime;
+    double *d_ap = nullptr, *d_sp = nullptr, *d_acc = nullptr, *d_steer = nullptr, *d_s0 = nullptr, *d_xo = nullptr, *d_yo = nullptr;
+    uint32_t *d_seed = nullptr, *d_state = nullptr;
+    int32_t *d_cnt = nullptr, *d_lane = nullptr;
+    auto body = [&]() -> int {
+        CK(cudaMalloc(&d_seed, (size_t)n_ep * 4)); CK(cudaMalloc(&d_ap, npl * 8)); CK(cudaMalloc(&d_sp, npl * 8));
+        CK(cudaMalloc(&d_acc, nc * 8)); CK(cudaMalloc(&d_steer, nc * 8)); CK(cudaMalloc(&d_s0, (size_t)n_ep * 5 * 8));
+        CK(cudaMalloc(&d_xo, no * 8)); CK(cudaMalloc(&d_yo, no * 8)); CK(cudaMalloc(&d_cnt, (size_t)n_ep * 4)); CK(cudaMalloc(&d_lane, (size_t)n_ep * 4));
+        if (state_out) CK(cudaMalloc(&d_state, (size_t)n_ep * VALN_STATE_WORDS * 4));
+        CK(cudaMemcpy(d_seed, seed, (size_t)n_ep * 4, cudaMemcpyHostToDevice));
+        CK(cudaMemcpy(d_ap, acc_plan, npl * 8, cudaMemcpyHostToDevice)); CK(cudaMemcpy(d_sp, steer_plan, npl * 8, cudaMemcpyHostToDevice));
+        CK(cudaMemcpy(d_s0, state0, (size_t)n_ep * 5 * 8, cudaMemcpyHostToDevice));
+        CK(cudaMemcpy(d_xo, x_obs_traj, no * 8, cudaMemcpyHostToDevice)); CK(cudaMemcpy(d_yo, y_obs_traj, no * 8, cudaMemcpyHostToDevice));
+        ValNoiseCfg vn;
+        vn.n_roll = n_roll; vn.np = num_prime; vn.noise_kind = noise_kind; vn.nl = noise_level; vn.k_steer = k_steer;
+        vn.beta_a = beta_a; vn.beta_b = beta_b; vn.c_acc = acc_const_noise; vn.c_steer = steer_const_noise;
+        k_validate_noise<<<n_ep, VALN_THREADS>>>(vn, d_seed, d_ap, d_sp, d_acc, d_steer, d_state);
+        CK(cudaGetLastError());
+        CK(launch_validate(n_ep, n_roll, num_prime, num_obs, obs_cost_f32, dt, wheel_base, a_obs, b_obs, y_lb, y_ub, smem,
+                           d_acc, d_steer, d_s0, d_xo, d_yo, d_cnt, d_lane, nullptr, nullptr));
+        CK(cudaMemcpy(count, d_cnt, (size_t)n_ep * 4, cudaMemcpyDeviceToHost)); CK(cudaMemcpy(count_lane, d_lane, (size_t)n_ep * 4, cudaMemcpyDeviceToHost));
+        if (acc_out) { CK(cudaMemcpy(acc_out, d_acc, nc * 8, cudaMemcpyDeviceToHost)); CK(cudaMemcpy(steer_out, d_steer, nc * 8, cudaMemcpyDeviceToHost)); }
+        if (state_out) CK(cudaMemcpy(state_out, d_state, (size_t)n_ep * VALN_STATE_WORDS * 4, cudaMemcpyDeviceToHost));
+        return 0;
+    };
+    const int rc = body();
+    cudaFree(d_seed); cudaFree(d_ap); cudaFree(d_sp); cudaFree(d_acc); cudaFree(d_steer); cudaFree(d_s0); cudaFree(d_xo); cudaFree(d_yo);
+    cudaFree(d_cnt); cudaFree(d_lane); cudaFree(d_state);
     return rc;
 }
 

@@ -34,7 +34,8 @@ class MpcmmdOut(C.Structure):
 
 EXPORTS = ("mpcmmd_last_error", "mpcmmd_version", "mpcmmd_create", "mpcmmd_destroy", "mpcmmd_solve", "mpcmmd_solve_host",
            "mpcmmd_last_launch_count", "mpcmmd_inner_cem_path", "mpcmmd_profile_solve", "mpcmmd_fp32_peak", "mpcmmd_xu_peaks", "mpcmmd_selfcheck_ieee", "mpcmmd_math_vec", "mpcmmd_rng_normal", "mpcmmd_rng_beta", "mpcmmd_get_tables",
-           "mpcmmd_stage_project", "mpcmmd_stage_risk", "mpcmmd_stage_risk_injected", "mpcmmd_stage_init", "mpcmmd_stage_select", "mpcmmd_stage_noise", "mpcmmd_validate_host")
+           "mpcmmd_stage_project", "mpcmmd_stage_risk", "mpcmmd_stage_risk_injected", "mpcmmd_stage_init", "mpcmmd_stage_select", "mpcmmd_stage_noise", "mpcmmd_validate_host",
+           "mpcmmd_validate_seeded_host")
 
 _lib = None
 
@@ -76,6 +77,7 @@ def load():
     lib.mpcmmd_stage_select.argtypes = [V, C.c_int] + [V] * 8
     lib.mpcmmd_stage_noise.argtypes = [V, C.c_int32, C.c_int32] + [V] * 5
     lib.mpcmmd_validate_host.argtypes = [C.c_int] * 6 + [C.c_double] * 6 + [V] * 9
+    lib.mpcmmd_validate_seeded_host.argtypes = [C.c_int] * 7 + [C.c_double] * 12 + [V] * 11
     _lib = lib
     return lib
 

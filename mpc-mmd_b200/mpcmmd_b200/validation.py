@@ -5,6 +5,9 @@ What stays on the host, and why: the reference seeds NumPy's legacy global strea
 and draws `multivariate_normal` / `beta` from it (:65-84).  Bit-identical collision counts need those exact MT19937 draws, so the noise is
 drawn here with the same calls in the same order, the controls are perturbed in float64 exactly as the reference does, and the perturbed
 controls go to `mpcmmd_validate_host` (csrc/k_validate.cuh), which rolls the 1000 bicycle models out and counts intersections.
+Opt-in (`--rng device`, `compute_stats_batch(..., rng="device")`): the same legacy stream restated on the GPU (csrc/dnprng.cuh,
+k_validate_noise.cuh), one stream per trajectory.  Its stream consumption is NumPy's exactly; its values differ from NumPy's only where
+CUDA's double pow / log / exp round differently from glibc's (DESIGN.md section 3 item 6).  The host draws stay the default and the reference.
 
 Same command line as the reference, same input files (`./data/{noise}_noise/noise_{L}/ts_{np}/{cost}_{nr}_samples_{O}_obs.npz`), same output
 (`./stats/{noise}_noise/noise_{L}/ts_{np}/{nr}_samples_{O}_obs.npz` with coll_cvar, coll_cvar_lane, coll_mmd_opt, coll_mmd_opt_lane,
@@ -59,21 +62,16 @@ def perturbed_controls(prob, acc, steer, noise_level, num_prime, noise, key, n_r
     return acc + acc_pert + prob.acc_const_noise * z, steer + steer_pert + prob.steer_const_noise * z
 
 
-def compute_stats_batch(prob, items, num_prime, noise_level, noise, num_obs, want_rollouts=False, device=None, n_roll=NUM_ROLLOUTS):
-    """`compute_stats` (validation.py:134-171) for a list of trajectories in ONE device call.
-
-    items: dicts with cx, cy (11,), init_state (6,), key, and either x_obs, y_obs, vx_obs, vy_obs (static variant) or
-    x_obs_traj, y_obs_traj (num_obs, 100) (dynamic variant).  Returns count (n,), count_lane (n,) int arrays [, x_roll, y_roll]."""
+def _inputs(prob, items, num_prime, num_obs):
+    """per-trajectory inputs of the validation entry points: planned controls (n, num_prime) x2, state0 (n, 5), obstacle trajectories
+    (n, num_obs, num_prime) x2, and whether the obstacle cost is float32 (static variant)"""
     n = len(items)
-    if n == 0:
-        z = np.zeros(0, np.int64)
-        return (z, z, None, None) if want_rollouts else (z, z)
-    acc_all = np.empty((n, n_roll, num_prime)); steer_all = np.empty((n, n_roll, num_prime))
+    acc_p = np.empty((n, num_prime)); steer_p = np.empty((n, num_prime))
     state0 = np.empty((n, 5)); xo = np.empty((n, num_obs, num_prime)); yo = np.empty((n, num_obs, num_prime))
     static = "x_obs_traj" not in items[0]
     for i, it in enumerate(items):
         acc, steer = compute_controls(prob, it["cx"], it["cy"])
-        acc_all[i], steer_all[i] = perturbed_controls(prob, acc[0:num_prime], steer[0:num_prime], noise_level, num_prime, noise, it["key"], n_roll)
+        acc_p[i], steer_p[i] = acc[0:num_prime], steer[0:num_prime]
         s = np.asarray(it["init_state"], np.float64).reshape(-1)
         state0[i] = [s[0], s[1], s[2], s[3], np.arctan2(s[3], s[2])]
         if static:
@@ -83,6 +81,32 @@ def compute_stats_batch(prob, items, num_prime, noise_level, noise, num_obs, wan
         else:
             xt = np.asarray(it["x_obs_traj"]).reshape(num_obs, prob.num); yt = np.asarray(it["y_obs_traj"]).reshape(num_obs, prob.num)
         xo[i] = xt[:, 0:num_prime]; yo[i] = yt[:, 0:num_prime]
+    return acc_p, steer_p, state0, xo, yo, static
+
+
+def compute_stats_batch(prob, items, num_prime, noise_level, noise, num_obs, want_rollouts=False, device=None, n_roll=NUM_ROLLOUTS, rng="host"):
+    """`compute_stats` (validation.py:134-171) for a list of trajectories in ONE device call.
+
+    items: dicts with cx, cy (11,), init_state (6,), key, and either x_obs, y_obs, vx_obs, vy_obs (static variant) or
+    x_obs_traj, y_obs_traj (num_obs, 100) (dynamic variant).  Returns count (n,), count_lane (n,) int arrays [, x_roll, y_roll].
+
+    rng="host" (default) draws the noise from NumPy's legacy stream here, exactly as the reference does.  rng="device" draws the same
+    stream on the GPU (`seeded_stats_batch`): identical stream consumption, values within CUDA's libm rounding of NumPy's; it returns
+    no rollouts."""
+    if rng == "device":
+        if want_rollouts:
+            raise ValueError("compute_stats_batch: want_rollouts needs rng='host'")
+        return seeded_stats_batch(prob, items, num_prime, noise_level, noise, num_obs, device=device, n_roll=n_roll)[:2]
+    if rng != "host":
+        raise ValueError("compute_stats_batch: rng must be 'host' or 'device', not %r" % (rng,))
+    n = len(items)
+    if n == 0:
+        z = np.zeros(0, np.int64)
+        return (z, z, None, None) if want_rollouts else (z, z)
+    acc_p, steer_p, state0, xo, yo, static = _inputs(prob, items, num_prime, num_obs)
+    acc_all = np.empty((n, n_roll, num_prime)); steer_all = np.empty((n, n_roll, num_prime))
+    for i, it in enumerate(items):
+        acc_all[i], steer_all[i] = perturbed_controls(prob, acc_p[i], steer_p[i], noise_level, num_prime, noise, it["key"], n_roll)
     count = np.zeros(n, np.int32); lane = np.zeros(n, np.int32)
     xr = np.empty((n, n_roll, num_prime)) if want_rollouts else None
     yr = np.empty((n, n_roll, num_prime)) if want_rollouts else None
@@ -92,6 +116,67 @@ def compute_stats_batch(prob, items, num_prime, noise_level, noise, num_obs, wan
                                           float(prob.a_obs), float(prob.b_obs), float(prob.y_lb), float(prob.y_ub), p(acc_all), p(steer_all),
                                           p(state0), p(xo), p(yo), p(count), p(lane), p(xr), p(yr)))
     return (count, lane, xr, yr) if want_rollouts else (count, lane)
+
+
+STATE_WORDS = 628                 # key[624], pos, has_gauss, cached gauss as float64 bits (mpcmmd_validate_seeded_host's state_out)
+_IDENTITY_OK = {}
+
+
+def _mvn_identity_is_exact(num_prime):
+    """multivariate_normal(0, I) multiplies the standard normals by sqrt(s)[:, None] * vh of svd(I) (NumPy's legacy
+    multivariate_normal); the device path draws plain standard normals, which is the same stream only if that factor is exactly I.
+    Checked once per num_prime against the LAPACK NumPy runs on."""
+    if num_prime not in _IDENTITY_OK:
+        _, s, vh = np.linalg.svd(np.eye(num_prime))
+        _IDENTITY_OK[num_prime] = bool(np.array_equal(np.sqrt(s)[:, None] * vh, np.eye(num_prime)))
+    return _IDENTITY_OK[num_prime]
+
+
+def check_beta_params(prob, acc, steer):
+    """the argument check np.random.beta makes before it draws (NaN passes): ValueError("a <= 0") / ("b <= 0") for the first failing
+    call of perturbed_controls -- the acceleration draw, then the steering draw"""
+    for a, b in ((prob.beta_a * np.abs(acc), prob.beta_b * np.abs(acc)), (prob.beta_a * np.abs(steer) + 1e-5, prob.beta_b * np.abs(steer) + 1e-5)):
+        if np.any(np.less_equal(a, 0)):
+            raise ValueError("a <= 0")
+        if np.any(np.less_equal(b, 0)):
+            raise ValueError("b <= 0")
+
+
+def seeded_stats_batch(prob, items, num_prime, noise_level, noise, num_obs, want_draws=False, device=None, n_roll=NUM_ROLLOUTS):
+    """`compute_stats_batch` with the legacy-stream noise drawn on the GPU (mpcmmd_validate_seeded_host, csrc/k_validate_noise.cuh):
+    the planned controls are computed here, each trajectory's stream is np.random.seed(item["key"]) restated on the device.
+    Returns count, count_lane (n,) [, acc, steer (n, n_roll, num_prime) perturbed controls, state (n, 628) uint32 streams after the
+    last draw = np.random.get_state()[1:] packed as key[624], pos, has_gauss, gauss bits]."""
+    if noise not in B.NOISE_KINDS:
+        raise ValueError("noise must be one of %s, not %r" % (sorted(B.NOISE_KINDS), noise))
+    n = len(items)
+    if n == 0:
+        z = np.zeros(0, np.int64)
+        return (z, z, np.zeros((0, n_roll, num_prime)), np.zeros((0, n_roll, num_prime)), np.zeros((0, STATE_WORDS), np.uint32)) if want_draws else (z, z)
+    seeds = np.empty(n, np.uint32)
+    for i, it in enumerate(items):
+        k = int(it["key"])
+        if not 0 <= k <= 0xffffffff:
+            raise ValueError("Seed must be between 0 and 2**32 - 1")                  # np.random.seed's range
+        seeds[i] = k
+    if not _mvn_identity_is_exact(num_prime):
+        raise RuntimeError("multivariate_normal(0, eye(%d)) is not exactly standard_normal with this LAPACK: use rng='host'" % num_prime)
+    acc_p, steer_p, state0, xo, yo, static = _inputs(prob, items, num_prime, num_obs)
+    if noise == "beta":
+        for i in range(n):
+            check_beta_params(prob, acc_p[i], steer_p[i])
+    count = np.zeros(n, np.int32); lane = np.zeros(n, np.int32)
+    acc = np.empty((n, n_roll, num_prime)) if want_draws else None
+    steer = np.empty((n, n_roll, num_prime)) if want_draws else None
+    state = np.empty((n, STATE_WORDS), np.uint32) if want_draws else None
+    dev = prob.device.index if device is None else int(device)
+    p = lambda a: None if a is None else a.ctypes.data_as(C.c_void_p)
+    B.check(B.load().mpcmmd_validate_seeded_host(
+        dev or 0, n, n_roll, num_prime, num_obs, 1 if static else 0, B.NOISE_KINDS[noise], float(noise_level), float(prob.cem_helper.K_steer),
+        float(prob.beta_a), float(prob.beta_b), float(prob.acc_const_noise), float(prob.steer_const_noise), float(prob.t), float(prob.wheel_base),
+        float(prob.a_obs), float(prob.b_obs), float(prob.y_lb), float(prob.y_ub), p(seeds), p(acc_p), p(steer_p), p(state0), p(xo), p(yo),
+        p(count), p(lane), p(acc), p(steer), p(state)))
+    return (count, lane, acc, steer, state) if want_draws else (count, lane)
 
 
 def _load(root, noise, noise_level, num_prime, cost, num_reduced, num_obs):
@@ -143,7 +228,7 @@ def run_validation(args, variant="static", device=0, log=print):
                         log((len(pairs), _matrix(data_cvar, num_obs).shape[1]))                     # the reference prints eset.shape
                         # both costs of a scene share the seed k (validation.py:315-336)
                         items = [_item(data_mmd_opt, im, k, dynamic) for k, _, im in pairs] + [_item(data_cvar, ic, k, dynamic) for k, ic, _ in pairs]
-                        count, lane = compute_stats_batch(prob, items, num_prime, noise_level, noise, num_obs)
+                        count, lane = compute_stats_batch(prob, items, num_prime, noise_level, noise, num_obs, rng=args.rng)
                         m = len(pairs)
                         f = lambda a: np.asarray(a, np.float64)                                   # np.append([], int) yields float64 arrays
                         path = "{}/{}_noise/noise_{}/ts_{}/{}_samples_{}_obs".format(args.stats_root, noise, int(noise_level * 100), num_prime, num_reduced, num_obs)
@@ -167,6 +252,9 @@ def build_parser():
     p.add_argument("--root", type=str, default="./data")
     p.add_argument("--stats_root", type=str, default="./stats")
     p.add_argument("--variant", type=str, default="static", choices=["static", "dynamic"])
+    p.add_argument("--rng", type=str, default="host", choices=["host", "device"],
+                   help="host (default): NumPy's legacy stream, as the reference; device: the same stream drawn on the GPU (identical "
+                        "consumption, values within CUDA's pow / log / exp rounding)")
     return p
 
 
