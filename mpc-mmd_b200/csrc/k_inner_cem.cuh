@@ -12,6 +12,7 @@
 // Replaces beta_cem.compute_cem (S/compute_beta.py:93-157) + kernel_matrix.compute_kernel (S/kernel_computation.py:19-65)
 // + Costs.compute_mmd_obs / compute_mmd_lane (S/optimizer/costs.py:121-135, 173-186).
 #pragma once
+#include <type_traits>
 #include "k_risk.cuh"
 
 namespace pk {   // packed float32x2 arithmetic (sm_100a): each lane is an IEEE-754 round-to-nearest operation
@@ -402,79 +403,114 @@ __device__ __forceinline__ void icf_chol(float* __restrict__ C, int ldc, int lan
 }
 
 // Cholesky of the d x d covariance by ONE warp, left-looking by PANELS of four columns: lane r owns row r.  For panel j0 = 4p each lane first
-// accumulates its four entries (r, j0..j0+3) over the finished columns k < j0 -- four independent fma chains per lane that share one load of
-// L[r][k] and one broadcast float4 of L[j0..j0+3][k] (the factor is kept TRANSPOSED: LT[k][q] = L[q][k], so both are conflict-free) -- then the
-// 4 x 4 diagonal block is gathered with ten shuffles and factored REDUNDANTLY by every lane in registers (no exchange inside the panel), and each
-// lane finishes its own four entries with the block's columns.  Entry (r, j) accumulates fma(-L_rk, L_jk, .) for k = 0 .. j-1 ascending, then
-// the pivot's square root / reciprocal scaling: the contract's order, bit for bit the same as the column-by-column versions.  7 sync points
-// and ~1500 executed instructions instead of 26 and ~2400 for d = 26.  In place: LT lives in the upper triangle (and diagonal) of C while the
-// untouched part of C's lower triangle still holds the covariance; each lane zeroes its consumed sub-diagonal entries, which is the zero
-// fill the resampling loops rely on (LT[k][q] = 0 for q < k).
+// accumulates its four entries (r, j0..j0+3) over the finished columns k < j0 -- four independent fma chains per lane, two FFMA2, that share one load
+// of L[r][k] and the broadcast L[j0..j0+3][k] (the factor is kept TRANSPOSED: LT[k][q] = L[q][k], so both are conflict-free) -- then the
+// 4 x 4 diagonal block is gathered with ten shuffles and factored REDUNDANTLY by every lane in registers (no exchange inside the panel): the lanes of
+// the block store their row of it, the lanes below finish their own four entries with the block's columns and store them transposed.  The last
+// panel factors only the columns that exist (d = 26: two).  Entry (r, j) accumulates fma(-L_rk, L_jk, .) for k = 0 .. j-1 ascending, then
+// the pivot's square root / reciprocal scaling: the contract's order, bit for bit the same as the column-by-column versions.  In place: LT lives in
+// the upper triangle (and diagonal) of C while the untouched part of C's lower triangle still holds the covariance.  The resampling loops read
+// whole float4 groups from the diagonal's group on (icf_mvn_row_unrolled, icu_row_elem), so the only zero fill they need is the strict lower
+// triangle of each 4 x 4 diagonal block (LT[k][q] = 0 for 4 (k / 4) <= q < k); the rest of the lower triangle is never read again.
+// One panel of W <= 4 live columns j0 .. j0 + W - 1 (W < 4 only for the last panel of a d that is not a multiple of four).
+template <int d, int W, bool LAST>
+__device__ __forceinline__ void icf_chol_panel_step(float* __restrict__ C, const float* __restrict__ rowp, int r, int lane, int p) {
+    constexpr int ldc = (d + 3) & ~3;
+    const int j0 = 4 * p;
+    float a[4];
+    {
+        // a(r, j0..j0+3), then the k < j0 part on the packed pipe: each lane of an FFMA2 is the fma(-L_rk, L_jk, .) of one entry, k ascending
+        pk::f2 a01 = *reinterpret_cast<const pk::f2*>(rowp + j0), a23 = *reinterpret_cast<const pk::f2*>(rowp + j0 + 2);
+        const float* pr = C + r;                                       // LT[k][r] = L[r][k], k = 0, 1, ...
+        const float* pj = C + j0;                                      // L[j0..j0+3][k]
+#pragma unroll 1
+        for (int k4 = 0; k4 < p; k4++) {                               // j0 is a multiple of four: whole groups of four columns, fixed offsets
+#pragma unroll
+            for (int u = 0; u < 4; u++) {
+                const pk::f2 nl = pk::dup(-pr[u * ldc]);
+                if constexpr (W > 2) {
+                    const pk::f2 l01 = *reinterpret_cast<const pk::f2*>(pj + u * ldc), l23 = *reinterpret_cast<const pk::f2*>(pj + u * ldc + 2);
+                    a01 = pk::fma2(nl, l01, a01); a23 = pk::fma2(nl, l23, a23);
+                } else {
+                    const float2 lj = *reinterpret_cast<const float2*>(pj + u * ldc);
+                    a01 = pk::fma2(nl, pk::pack(lj.x, lj.y), a01);
+                }
+            }
+            pr += 4 * ldc; pj += 4 * ldc;
+        }
+        pk::unpack(a01, a[0], a[1]); pk::unpack(a23, a[2], a[3]);
+    }
+    // diagonal block b(i, j), j <= i < W, from lanes j0 + i, factored redundantly by every lane (the columns that exist only).  The pivots take the
+    // branch-free fast path of sqrt_rcp with one range check for the whole block; the block is the same on every lane, so is the check, and a block
+    // with a pivot outside the fast path's range is factored again with sqrt_rcp -- the same bits either way.
+    float b[4][4], l[4][4], dv[4], rv[4];
+#pragma unroll
+    for (int i = 0; i < W; i++)
+#pragma unroll
+        for (int j = 0; j <= i; j++) b[i][j] = __shfl_sync(FULL, a[j], j0 + i);
+    auto factor = [&](auto fast) {
+        bool ok = true;
+#pragma unroll
+        for (int j = 0; j < W; j++) {
+            float acc = b[j][j];
+#pragma unroll
+            for (int k = 0; k < j; k++) acc = fmaf(-l[j][k], l[j][k], acc);
+            if constexpr (decltype(fast)::value) ok &= dm::sqrt_rcp_fast(acc, dv[j], rv[j]);
+            else dm::sqrt_rcp(acc, dv[j], rv[j]);
+#pragma unroll
+            for (int i = j + 1; i < W; i++) {
+                float s = b[i][j];
+#pragma unroll
+                for (int k = 0; k < j; k++) s = fmaf(-l[i][k], l[j][k], s);
+                l[i][j] = s * rv[j];
+            }
+        }
+        return ok;
+    };
+    if (!factor(std::true_type{})) factor(std::false_type{});
+    if (lane >= j0 && lane < j0 + W) {
+        // row v = lane - j0 of the block of LT: zeros left of the diagonal, the pivot, then L[j0 + u][j0 + v] = l[u][v] (the padding columns of the last panel get zeros)
+        const int v = lane - j0;
+        float o[4];
+#pragma unroll
+        for (int u = 0; u < 4; u++) {
+            float x = 0.0f;
+            if (u < W) {
+                x = u == W - 1 ? dv[u] : 0.0f;                     // v <= W - 1: the last column needs no test for its pivot
+#pragma unroll
+                for (int w = 0; w < u; w++) x = v == w ? l[u][w] : x;
+                if (u < W - 1) x = v == u ? dv[u] : x;
+            }
+            o[u] = x;
+        }
+        *reinterpret_cast<float4*>(C + lane * ldc + j0) = make_float4(o[0], o[1], o[2], o[3]);
+    }
+    if constexpr (!LAST) {
+        // rows below the block: own entries L[r][j0 + u], stored transposed as column r of LT rows j0..j0+3
+        float e[4];
+#pragma unroll
+        for (int u = 0; u < 4; u++) {
+            float s = a[u];
+#pragma unroll
+            for (int k = 0; k < u; k++) s = fmaf(-e[k], l[u][k], s);
+            e[u] = s * rv[u];
+        }
+        if (lane >= j0 + 4 && lane < d) {
+#pragma unroll
+            for (int u = 0; u < 4; u++) C[(j0 + u) * ldc + lane] = e[u];
+        }
+    }
+    __syncwarp();                                                  // the next panel (or the caller) reads these rows of LT
+}
 template <int d>
 __device__ __forceinline__ void icf_chol_panel(float* __restrict__ C, int ldc_, int lane) {
     constexpr int NG = (d + 3) / 4, ldc = (d + 3) & ~3;    // the row stride is a compile-time constant (every caller passes al4(d)): immediate load offsets
     (void)ldc_;
     const int r = lane < d ? lane : d - 1;                 // lanes >= d shadow the last row (no stores)
-    float* rowp = C + r * ldc;
+    const float* rowp = C + r * ldc;
 #pragma unroll 1
-    for (int p = 0; p < NG; p++) {
-        const int j0 = 4 * p;
-        float4 av = *reinterpret_cast<const float4*>(rowp + j0);          // a(r, j0..j0+3)
-        float a0 = av.x, a1 = av.y, a2 = av.z, a3 = av.w;
-        {
-            const float* pr = C + r;                                       // LT[k][r] = L[r][k], k = 0, 1, ...
-            const float* pj = C + j0;                                      // L[j0..j0+3][k]
-#pragma unroll 1
-            for (int k4 = 0; k4 < p; k4++) {                               // j0 is a multiple of four: whole groups of four columns, fixed offsets
-#pragma unroll
-                for (int u = 0; u < 4; u++) {
-                    const float lr = pr[u * ldc];
-                    const float4 lj = *reinterpret_cast<const float4*>(pj + u * ldc);
-                    a0 = fmaf(-lr, lj.x, a0); a1 = fmaf(-lr, lj.y, a1); a2 = fmaf(-lr, lj.z, a2); a3 = fmaf(-lr, lj.w, a3);
-                }
-                pr += 4 * ldc; pj += 4 * ldc;
-            }
-        }
-        // diagonal block b(u', u), u <= u', from lanes j0 + u'
-        const float b00 = __shfl_sync(FULL, a0, j0);
-        const float b10 = __shfl_sync(FULL, a0, j0 + 1), b11 = __shfl_sync(FULL, a1, j0 + 1);
-        const float b20 = __shfl_sync(FULL, a0, j0 + 2), b21 = __shfl_sync(FULL, a1, j0 + 2), b22 = __shfl_sync(FULL, a2, j0 + 2);
-        const float b30 = __shfl_sync(FULL, a0, j0 + 3), b31 = __shfl_sync(FULL, a1, j0 + 3), b32 = __shfl_sync(FULL, a2, j0 + 3), b33 = __shfl_sync(FULL, a3, j0 + 3);
-        float d0, r0, d1, r1, d2, r2, d3, r3;
-        dm::sqrt_rcp(b00, d0, r0);
-        const float l10 = b10 * r0, l20 = b20 * r0, l30 = b30 * r0;
-        dm::sqrt_rcp(fmaf(-l10, l10, b11), d1, r1);
-        const float l21 = fmaf(-l20, l10, b21) * r1, l31 = fmaf(-l30, l10, b31) * r1;
-        dm::sqrt_rcp(fmaf(-l21, l21, fmaf(-l20, l20, b22)), d2, r2);
-        const float l32 = fmaf(-l31, l21, fmaf(-l30, l20, b32)) * r2;
-        dm::sqrt_rcp(fmaf(-l32, l32, fmaf(-l31, l31, fmaf(-l30, l30, b33))), d3, r3);
-        // own row: L[r][j0 + u]; on the diagonal the pivot itself, above it nothing
-        float e0 = a0 * r0;
-        a1 = fmaf(-e0, l10, a1); float e1 = a1 * r1;
-        a2 = fmaf(-e1, l21, fmaf(-e0, l20, a2)); float e2 = a2 * r2;
-        a3 = fmaf(-e2, l32, fmaf(-e1, l31, fmaf(-e0, l30, a3))); float e3 = a3 * r3;
-        if (lane == j0) e0 = d0;
-        if (lane == j0 + 1) e1 = d1;
-        if (lane == j0 + 2) e2 = d2;
-        if (lane == j0 + 3) e3 = d3;
-        if (lane < d) {
-            // consumed covariance entries below the diagonal become the zero fill; then column r of LT rows j0..j0+3 (q = r >= k only)
-            float4 z = av;
-            if (j0 + 0 < lane) z.x = 0.0f;
-            if (j0 + 1 < lane) z.y = 0.0f;
-            if (j0 + 2 < lane) z.z = 0.0f;
-            if (j0 + 3 < lane) z.w = 0.0f;
-            if (lane >= j0) *reinterpret_cast<float4*>(rowp + j0) = z;
-        }
-        __syncwarp();
-        if (lane < d) {
-            if (lane >= j0 + 0) C[(j0 + 0) * ldc + lane] = e0;
-            if (lane >= j0 + 1 && j0 + 1 < d) C[(j0 + 1) * ldc + lane] = e1;
-            if (lane >= j0 + 2 && j0 + 2 < d) C[(j0 + 2) * ldc + lane] = e2;
-            if (lane >= j0 + 3 && j0 + 3 < d) C[(j0 + 3) * ldc + lane] = e3;
-        }
-        __syncwarp();
-    }
+    for (int p = 0; p < NG - 1; p++) icf_chol_panel_step<d, 4, false>(C, rowp, r, lane, p);
+    icf_chol_panel_step<d, d - 4 * (NG - 1), true>(C, rowp, r, lane, NG - 1);
 }
 
 // Cholesky of the d x d covariance by the WHOLE CTA (3 warps), left-looking by panels of four columns, same per-entry operation order as icf_chol_panel (so the
