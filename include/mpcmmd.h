@@ -141,6 +141,20 @@ int mpcmmd_validate_seeded_host(int device, int n_ep, int n_roll, int num_prime,
                                 const double *state0, const double *x_obs_traj, const double *y_obs_traj, int32_t *count,
                                 int32_t *count_lane, double *acc_out, double *steer_out, uint32_t *state_out);
 
+/* The same validation with COUNTER-BASED noise drawn by each rollout itself (k_validate_jax, DESIGN.md section 3 item 7): trajectory i's
+ * noise is the JAX 0.3.23 protocol's random.beta / random.normal of (k_acc, k_steer, k_z) = split(PRNGKey(seed[i]), 3) over an
+ * (n_roll, num_prime) array (csrc/drng.cuh), so a rollout's draws depend on n_roll.  Not NumPy's stream: the counts are a Monte-Carlo
+ * estimate of the same quantity, not the reference's numbers.  The arguments as mpcmmd_validate_seeded_host; no shape parameter check
+ * (a Beta shape of 0 gives what the sampler gives: NaN where both shapes are 0).  Fails on n_roll < 1 and n_roll * num_prime >= 2^31
+ * (JAX's uint32 element counters).  Optional outputs (NULL to skip): acc_out, steer_out (n_ep, n_roll, num_prime) the perturbed
+ * controls (both or neither).  All pointers are HOST pointers.  Synchronous. */
+int mpcmmd_validate_threefry_host(int device, int n_ep, int n_roll, int num_prime, int num_obs, int obs_cost_f32, int noise_kind,
+                                  double noise_level, double k_steer, double beta_a, double beta_b, double acc_const_noise,
+                                  double steer_const_noise, double dt, double wheel_base, double a_obs, double b_obs, double y_lb,
+                                  double y_ub, const uint32_t *seed, const double *acc_plan, const double *steer_plan,
+                                  const double *state0, const double *x_obs_traj, const double *y_obs_traj, int32_t *count,
+                                  int32_t *count_lane, double *acc_out, double *steer_out);
+
 /* Measured FP32 FMA throughput of the device (TFLOP/s, FMA = 2 flops): the roofline denominator of the FP32-bound kernels. */
 int mpcmmd_fp32_peak(int device, float *tflops, int *sm_count);
 /* Measured special-function-unit peaks (thread-level operations per second / 1e9): gops[0] = ex2.approx (MUFU.EX2), gops[1] = IEEE

@@ -164,6 +164,15 @@ __device__ __noinline__ float beta_elem(Key key, uint32_t n, uint32_t e, float a
     float ga = dm::exp_(lga - m), gb = dm::exp_(lgb - m);
     return ga / (ga + gb);
 }
+// beta_elem with (ka, kb) = split(key) made by the caller: a stream drawn element by element splits its key once, not per element
+__device__ __noinline__ float beta_elem_split(Key ka, Key kb, uint32_t n, uint32_t e, float a, float b) {
+    float lga = loggamma_one(split_row(ka, n, e), a);
+    float lgb = loggamma_one(split_row(kb, n, e), b);
+    float m = lga > lgb ? lga : lgb;
+    if (lga != lga || lgb != lgb) m = DM_NAN;
+    float ga = dm::exp_(lga - m), gb = dm::exp_(lgb - m);
+    return ga / (ga + gb);
+}
 
 // ---------------------------------------------------------------------------------------------
 // Replay form of the Beta sampler.  Every random number _gamma_one consumes is a pure function of (element key, round r,

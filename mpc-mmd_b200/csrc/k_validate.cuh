@@ -19,8 +19,57 @@ struct ValCfg {
     double dt, wheel_base, a2, b2, y_lb, y_ub;
 };
 
-// grid = episodes; thread r handles rollouts r, r + VAL_THREADS, ...; shared counters cnt[(O + 2)][np]:
-// rows 0..O-1 obstacle intersections per (obstacle, timestep), row O lower-lane, row O+1 upper-lane violations per timestep.
+// Shared counters cnt[(O + 2)][np]: rows 0..O-1 obstacle intersections per (obstacle, timestep), row O lower-lane, row O+1 upper-lane
+// violations per timestep.  val_count adds one rollout state per lane at timestep t; every lane of the warp must call it (ballots).
+// xo, yo: the trajectory's obstacle trajectories (O, np).
+__device__ __forceinline__ void val_count(const ValCfg& c, const double* __restrict__ xo, const double* __restrict__ yo, int t, double x,
+                                          double y, bool live, int lane, int* cnt) {
+    const int np = c.np, O = c.O;
+    const float a2f = (float)c.a2, b2f = (float)c.b2;
+    for (int o = 0; o < O; o++) {
+        bool nz;
+        if (c.obs_f32) {
+            const float wc = (float)x - (float)xo[o * np + t], ws = (float)y - (float)yo[o * np + t];
+            const float cost = ((-(wc * wc)) / a2f - (ws * ws) / b2f) + 1.0f;          // S/validation.py:112
+            nz = (cost > 0.0f) || (cost != cost);                                       // np.maximum(0, cost) != 0 (NaN counts)
+        } else {
+            const double wc = x - xo[o * np + t], ws = y - yo[o * np + t];
+            const double cost = ((-(wc * wc)) / c.a2 - (ws * ws) / c.b2) + 1.0;
+            nz = (cost > 0.0) || (cost != cost);
+        }
+        const unsigned m = __ballot_sync(0xffffffffu, live && nz);
+        if (lane == 0 && m) atomicAdd(&cnt[o * np + t], __popc(m));
+    }
+    const double lb = -y + c.y_lb, ub = y - c.y_ub;                                     // S/validation.py:118-119
+    const unsigned ml = __ballot_sync(0xffffffffu, live && ((lb > 0.0) || (lb != lb)));
+    const unsigned mu = __ballot_sync(0xffffffffu, live && ((ub > 0.0) || (ub != ub)));
+    if (lane == 0 && ml) atomicAdd(&cnt[O * np + t], __popc(ml));
+    if (lane == 0 && mu) atomicAdd(&cnt[(O + 1) * np + t], __popc(mu));
+}
+
+// one bicycle-model step with controls (a, st) (S/validation.py:21-38)
+__device__ __forceinline__ void val_step(const ValCfg& c, double a, double st, double& x, double& y, double& vx, double& vy, double& psi) {
+    double v = sqrt(vx * vx + vy * vy);
+    v = v + a * c.dt;
+    const double psidot = v * tan(st) / c.wheel_base;
+    const double psi_next = psi + psidot * c.dt;
+    const double vx_next = v * cos(psi_next), vy_next = v * sin(psi_next);
+    x = x + vx_next * c.dt; y = y + vy_next * c.dt;
+    vx = vx_next; vy = vy_next; psi = psi_next;
+}
+
+// one warp: count = max over (obstacle, timestep) of the intersection counts; count_lane = max_t lb + max_t ub (S/validation.py:156-169)
+__device__ __forceinline__ void val_reduce(const int* cnt, int O, int np, int lane, int32_t* count, int32_t* count_lane) {
+    int m = 0, l = 0, u = 0;
+    for (int i = lane; i < O * np; i += 32) m = max(m, cnt[i]);
+    for (int t = lane; t < np; t += 32) { l = max(l, cnt[O * np + t]); u = max(u, cnt[(O + 1) * np + t]); }
+    for (int off = 16; off >= 1; off >>= 1) {
+        m = max(m, __shfl_xor_sync(0xffffffffu, m, off)); l = max(l, __shfl_xor_sync(0xffffffffu, l, off)); u = max(u, __shfl_xor_sync(0xffffffffu, u, off));
+    }
+    if (lane == 0) { *count = m; *count_lane = l + u; }
+}
+
+// grid = episodes; thread r handles rollouts r, r + VAL_THREADS, ...
 __global__ void __launch_bounds__(VAL_THREADS) k_validate(ValCfg c, const double* __restrict__ acc, const double* __restrict__ steer,
                                                           const double* __restrict__ state0, const double* __restrict__ x_obs,
                                                           const double* __restrict__ y_obs, int32_t* __restrict__ count,
@@ -33,7 +82,6 @@ __global__ void __launch_bounds__(VAL_THREADS) k_validate(ValCfg c, const double
     const double* xo = x_obs + (size_t)e * O * np;
     const double* yo = y_obs + (size_t)e * O * np;
     const double* s0 = state0 + (size_t)e * 5;
-    const float a2f = (float)c.a2, b2f = (float)c.b2;
     for (int base = 0; base < c.n_roll; base += VAL_THREADS) {
         const int r = base + tid;
         const bool live = r < c.n_roll;
@@ -42,47 +90,10 @@ __global__ void __launch_bounds__(VAL_THREADS) k_validate(ValCfg c, const double
         for (int t = 0; t < np; t++) {
             // ---- record the state before the step (S/validation.py:98-100) and count on it
             if (live && x_roll) { x_roll[row + t] = x; y_roll[row + t] = y; }
-            for (int o = 0; o < O; o++) {
-                bool nz;
-                if (c.obs_f32) {
-                    const float wc = (float)x - (float)xo[o * np + t], ws = (float)y - (float)yo[o * np + t];
-                    const float cost = ((-(wc * wc)) / a2f - (ws * ws) / b2f) + 1.0f;          // S/validation.py:112
-                    nz = (cost > 0.0f) || (cost != cost);                                       // np.maximum(0, cost) != 0 (NaN counts)
-                } else {
-                    const double wc = x - xo[o * np + t], ws = y - yo[o * np + t];
-                    const double cost = ((-(wc * wc)) / c.a2 - (ws * ws) / c.b2) + 1.0;
-                    nz = (cost > 0.0) || (cost != cost);
-                }
-                const unsigned m = __ballot_sync(0xffffffffu, live && nz);
-                if (lane == 0 && m) atomicAdd(&cnt[o * np + t], __popc(m));
-            }
-            {
-                const double lb = -y + c.y_lb, ub = y - c.y_ub;                                 // S/validation.py:118-119
-                const unsigned ml = __ballot_sync(0xffffffffu, live && ((lb > 0.0) || (lb != lb)));
-                const unsigned mu = __ballot_sync(0xffffffffu, live && ((ub > 0.0) || (ub != ub)));
-                if (lane == 0 && ml) atomicAdd(&cnt[O * np + t], __popc(ml));
-                if (lane == 0 && mu) atomicAdd(&cnt[(O + 1) * np + t], __popc(mu));
-            }
-            // ---- one bicycle-model step (S/validation.py:21-38)
-            const double a = live ? acc[row + t] : 0.0, st = live ? steer[row + t] : 0.0;
-            double v = sqrt(vx * vx + vy * vy);
-            v = v + a * c.dt;
-            const double psidot = v * tan(st) / c.wheel_base;
-            const double psi_next = psi + psidot * c.dt;
-            const double vx_next = v * cos(psi_next), vy_next = v * sin(psi_next);
-            x = x + vx_next * c.dt; y = y + vy_next * c.dt;
-            vx = vx_next; vy = vy_next; psi = psi_next;
+            val_count(c, xo, yo, t, x, y, live, lane, cnt);
+            val_step(c, live ? acc[row + t] : 0.0, live ? steer[row + t] : 0.0, x, y, vx, vy, psi);
         }
     }
     __syncthreads();
-    // count = max over (obstacle, timestep) of the intersection counts; count_lane = max_t lb + max_t ub (S/validation.py:156-169)
-    if (tid < 32) {
-        int m = 0, l = 0, u = 0;
-        for (int i = tid; i < O * np; i += 32) m = max(m, cnt[i]);
-        for (int t = tid; t < np; t += 32) { l = max(l, cnt[O * np + t]); u = max(u, cnt[(O + 1) * np + t]); }
-        for (int off = 16; off >= 1; off >>= 1) {
-            m = max(m, __shfl_xor_sync(0xffffffffu, m, off)); l = max(l, __shfl_xor_sync(0xffffffffu, l, off)); u = max(u, __shfl_xor_sync(0xffffffffu, u, off));
-        }
-        if (tid == 0) { count[e] = m; count_lane[e] = l + u; }
-    }
+    if (tid < 32) val_reduce(cnt, O, np, lane, count + e, count_lane + e);
 }

@@ -22,6 +22,7 @@
 #include "k_select.cuh"
 #include "k_validate.cuh"
 #include "k_validate_noise.cuh"
+#include "k_validate_jax.cuh"
 
 static thread_local std::string g_err;
 static int fail(const std::string& m) { g_err = m; return -1; }
@@ -1050,6 +1051,68 @@ extern "C" int mpcmmd_validate_seeded_host(int device, int n_ep, int n_roll, int
     const int rc = body();
     cudaFree(d_seed); cudaFree(d_ap); cudaFree(d_sp); cudaFree(d_acc); cudaFree(d_steer); cudaFree(d_s0); cudaFree(d_xo); cudaFree(d_yo);
     cudaFree(d_cnt); cudaFree(d_lane); cudaFree(d_state);
+    return rc;
+}
+
+// The same with counter-based noise (k_validate_jax, DESIGN.md section 3 item 7): each rollout draws its JAX-protocol noise while it
+// rolls out, so n_roll is bounded only by JAX's uint32 element counters.
+extern "C" int mpcmmd_validate_threefry_host(int device, int n_ep, int n_roll, int num_prime, int num_obs, int obs_cost_f32, int noise_kind,
+                                             double noise_level, double k_steer, double beta_a, double beta_b, double acc_const_noise,
+                                             double steer_const_noise, double dt, double wheel_base, double a_obs, double b_obs, double y_lb,
+                                             double y_ub, const uint32_t* seed, const double* acc_plan, const double* steer_plan,
+                                             const double* state0, const double* x_obs_traj, const double* y_obs_traj, int32_t* count,
+                                             int32_t* count_lane, double* acc_out, double* steer_out) {
+    int ndev = 0;
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) return fail("mpcmmd_validate_threefry_host: no CUDA device (this library has no CPU fallback)");
+    if (device < 0 || device >= ndev) return fail("mpcmmd_validate_threefry_host: bad device index");
+    if (n_roll < 1) return fail("mpcmmd_validate_threefry_host: n_roll must be >= 1");
+    if (n_ep < 1 || num_prime < 1 || num_prime > MPCMMD_T || num_obs < 1) return fail("mpcmmd_validate_threefry_host: bad sizes");
+    if ((long long)n_roll * num_prime >= (1LL << 31))
+        return fail("mpcmmd_validate_threefry_host: n_roll * num_prime must be below 2^31 (JAX's uint32 element counters)");
+    if (noise_kind != 0 && noise_kind != 1) return fail("mpcmmd_validate_threefry_host: noise_kind must be 0 (gaussian) or 1 (beta)");
+    if (!seed || !acc_plan || !steer_plan || !state0 || !x_obs_traj || !y_obs_traj || !count || !count_lane)
+        return fail("mpcmmd_validate_threefry_host: null pointer");
+    if ((acc_out == nullptr) != (steer_out == nullptr)) return fail("mpcmmd_validate_threefry_host: acc_out and steer_out must both be given or both be null");
+    const size_t smem = (size_t)(num_obs + 2) * num_prime * sizeof(int);
+    if (smem > 200 * 1024) return fail("mpcmmd_validate_threefry_host: (num_obs + 2) * num_prime counters do not fit in shared memory");
+    CK(cudaSetDevice(device));
+    const size_t nc = (size_t)n_ep * n_roll * num_prime, no = (size_t)n_ep * num_obs * num_prime, npl = (size_t)n_ep * num_prime;
+    const size_t ncnt = (size_t)n_ep * (num_obs + 2) * num_prime;
+    double *d_ap = nullptr, *d_sp = nullptr, *d_acc = nullptr, *d_steer = nullptr, *d_s0 = nullptr, *d_xo = nullptr, *d_yo = nullptr;
+    uint32_t* d_seed = nullptr;
+    int32_t *d_cg = nullptr, *d_cnt = nullptr, *d_lane = nullptr;
+    auto body = [&]() -> int {
+        CK(cudaMalloc(&d_seed, (size_t)n_ep * 4)); CK(cudaMalloc(&d_ap, npl * 8)); CK(cudaMalloc(&d_sp, npl * 8));
+        CK(cudaMalloc(&d_s0, (size_t)n_ep * 5 * 8)); CK(cudaMalloc(&d_xo, no * 8)); CK(cudaMalloc(&d_yo, no * 8));
+        CK(cudaMalloc(&d_cg, ncnt * 4)); CK(cudaMalloc(&d_cnt, (size_t)n_ep * 4)); CK(cudaMalloc(&d_lane, (size_t)n_ep * 4));
+        if (acc_out) { CK(cudaMalloc(&d_acc, nc * 8)); CK(cudaMalloc(&d_steer, nc * 8)); }
+        CK(cudaMemcpy(d_seed, seed, (size_t)n_ep * 4, cudaMemcpyHostToDevice));
+        CK(cudaMemcpy(d_ap, acc_plan, npl * 8, cudaMemcpyHostToDevice)); CK(cudaMemcpy(d_sp, steer_plan, npl * 8, cudaMemcpyHostToDevice));
+        CK(cudaMemcpy(d_s0, state0, (size_t)n_ep * 5 * 8, cudaMemcpyHostToDevice));
+        CK(cudaMemcpy(d_xo, x_obs_traj, no * 8, cudaMemcpyHostToDevice)); CK(cudaMemcpy(d_yo, y_obs_traj, no * 8, cudaMemcpyHostToDevice));
+        CK(cudaMemset(d_cg, 0, ncnt * 4));
+        if (smem > 48 * 1024) CK(cudaFuncSetAttribute(k_validate_jax, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        ValCfg c;
+        c.n_roll = n_roll; c.np = num_prime; c.O = num_obs; c.obs_f32 = obs_cost_f32; c.dt = dt; c.wheel_base = wheel_base;
+        c.a2 = a_obs * a_obs; c.b2 = b_obs * b_obs; c.y_lb = y_lb; c.y_ub = y_ub;
+        ValJaxCfg j;
+        j.noise_kind = noise_kind; j.nl = noise_level; j.ks = k_steer * noise_level; j.beta_a = beta_a; j.beta_b = beta_b;
+        j.c_acc = acc_const_noise; j.c_steer = steer_const_noise;
+        const unsigned chunks = (unsigned)((n_roll + VALJ_THREADS - 1) / VALJ_THREADS);
+        for (int e0 = 0; e0 < n_ep; e0 += 65535) {                      // gridDim.y <= 65535 trajectories per launch
+            const dim3 grid(chunks, (unsigned)(n_ep - e0 < 65535 ? n_ep - e0 : 65535));
+            k_validate_jax<<<grid, VALJ_THREADS, smem>>>(c, j, e0, d_seed, d_ap, d_sp, d_s0, d_xo, d_yo, d_cg, d_acc, d_steer);
+            CK(cudaGetLastError());
+        }
+        k_validate_finish<<<n_ep, 32>>>(num_obs, num_prime, d_cg, d_cnt, d_lane);
+        CK(cudaGetLastError());
+        CK(cudaMemcpy(count, d_cnt, (size_t)n_ep * 4, cudaMemcpyDeviceToHost)); CK(cudaMemcpy(count_lane, d_lane, (size_t)n_ep * 4, cudaMemcpyDeviceToHost));
+        if (acc_out) { CK(cudaMemcpy(acc_out, d_acc, nc * 8, cudaMemcpyDeviceToHost)); CK(cudaMemcpy(steer_out, d_steer, nc * 8, cudaMemcpyDeviceToHost)); }
+        return 0;
+    };
+    const int rc = body();
+    cudaFree(d_seed); cudaFree(d_ap); cudaFree(d_sp); cudaFree(d_acc); cudaFree(d_steer); cudaFree(d_s0); cudaFree(d_xo); cudaFree(d_yo);
+    cudaFree(d_cg); cudaFree(d_cnt); cudaFree(d_lane);
     return rc;
 }
 

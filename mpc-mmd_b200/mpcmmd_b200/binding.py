@@ -35,7 +35,7 @@ class MpcmmdOut(C.Structure):
 EXPORTS = ("mpcmmd_last_error", "mpcmmd_version", "mpcmmd_create", "mpcmmd_destroy", "mpcmmd_solve", "mpcmmd_solve_host",
            "mpcmmd_last_launch_count", "mpcmmd_inner_cem_path", "mpcmmd_profile_solve", "mpcmmd_fp32_peak", "mpcmmd_xu_peaks", "mpcmmd_selfcheck_ieee", "mpcmmd_math_vec", "mpcmmd_rng_normal", "mpcmmd_rng_beta", "mpcmmd_get_tables",
            "mpcmmd_stage_project", "mpcmmd_stage_risk", "mpcmmd_stage_risk_injected", "mpcmmd_stage_init", "mpcmmd_stage_select", "mpcmmd_stage_noise", "mpcmmd_validate_host",
-           "mpcmmd_validate_seeded_host")
+           "mpcmmd_validate_seeded_host", "mpcmmd_validate_threefry_host")
 
 _lib = None
 
@@ -78,6 +78,7 @@ def load():
     lib.mpcmmd_stage_noise.argtypes = [V, C.c_int32, C.c_int32] + [V] * 5
     lib.mpcmmd_validate_host.argtypes = [C.c_int] * 6 + [C.c_double] * 6 + [V] * 9
     lib.mpcmmd_validate_seeded_host.argtypes = [C.c_int] * 7 + [C.c_double] * 12 + [V] * 11
+    lib.mpcmmd_validate_threefry_host.argtypes = [C.c_int] * 7 + [C.c_double] * 12 + [V] * 10
     _lib = lib
     return lib
 

@@ -8,10 +8,14 @@ controls go to `mpcmmd_validate_host` (csrc/k_validate.cuh), which rolls the 100
 Opt-in (`--rng device`, `compute_stats_batch(..., rng="device")`): the same legacy stream restated on the GPU (csrc/dnprng.cuh,
 k_validate_noise.cuh), one stream per trajectory.  Its stream consumption is NumPy's exactly; its values differ from NumPy's only where
 CUDA's double pow / log / exp round differently from glibc's (DESIGN.md section 3 item 6).  The host draws stay the default and the reference.
+Opt-in (`--rng jax`, `compute_stats_batch(..., rng="jax")`): counter-based noise from the JAX protocol the reference's solver draws with
+(csrc/drng.cuh, k_validate_jax.cuh, DESIGN.md section 3 item 7), drawn by each rollout on the GPU as it rolls out.  Same distributions,
+different random numbers: its counts estimate what the reference's estimate, for any number of rollouts (`--num_rollouts`).
 
 Same command line as the reference, same input files (`./data/{noise}_noise/noise_{L}/ts_{np}/{cost}_{nr}_samples_{O}_obs.npz`), same output
 (`./stats/{noise}_noise/noise_{L}/ts_{np}/{nr}_samples_{O}_obs.npz` with coll_cvar, coll_cvar_lane, coll_mmd_opt, coll_mmd_opt_lane,
-coll_mmd_random, coll_mmd_random_lane).  Trajectory pairs are enumerated exactly like the reference does -- `set(cvar rows) & set(mmd_opt rows)`
+coll_mmd_random, coll_mmd_random_lane; with `--rng jax` or a non-default `--num_rollouts` also rng and num_rollouts, so those counts are
+not taken for the reference's).  Trajectory pairs are enumerated exactly like the reference does -- `set(cvar rows) & set(mmd_opt rows)`
 in Python set-iteration order, position k in that order is the RNG seed of the pair (SURVEY.md Q21) -- so the per-pair draws are the same.
 """
 from __future__ import annotations
@@ -91,14 +95,16 @@ def compute_stats_batch(prob, items, num_prime, noise_level, noise, num_obs, wan
     x_obs_traj, y_obs_traj (num_obs, 100) (dynamic variant).  Returns count (n,), count_lane (n,) int arrays [, x_roll, y_roll].
 
     rng="host" (default) draws the noise from NumPy's legacy stream here, exactly as the reference does.  rng="device" draws the same
-    stream on the GPU (`seeded_stats_batch`): identical stream consumption, values within CUDA's libm rounding of NumPy's; it returns
-    no rollouts."""
-    if rng == "device":
+    stream on the GPU (`seeded_stats_batch`): identical stream consumption, values within CUDA's libm rounding of NumPy's.  rng="jax"
+    draws counter-based JAX-protocol noise in the rollout kernel (`threefry_stats_batch`): not NumPy's numbers, same distributions.
+    Neither returns rollouts."""
+    if rng in ("device", "jax"):
         if want_rollouts:
             raise ValueError("compute_stats_batch: want_rollouts needs rng='host'")
-        return seeded_stats_batch(prob, items, num_prime, noise_level, noise, num_obs, device=device, n_roll=n_roll)[:2]
+        f = seeded_stats_batch if rng == "device" else threefry_stats_batch
+        return f(prob, items, num_prime, noise_level, noise, num_obs, device=device, n_roll=n_roll)[:2]
     if rng != "host":
-        raise ValueError("compute_stats_batch: rng must be 'host' or 'device', not %r" % (rng,))
+        raise ValueError("compute_stats_batch: rng must be 'host', 'device' or 'jax', not %r" % (rng,))
     n = len(items)
     if n == 0:
         z = np.zeros(0, np.int64)
@@ -142,6 +148,17 @@ def check_beta_params(prob, acc, steer):
             raise ValueError("b <= 0")
 
 
+def _seeds(items):
+    """the per-trajectory seeds as uint32, refused outside np.random.seed's range"""
+    seeds = np.empty(len(items), np.uint32)
+    for i, it in enumerate(items):
+        k = int(it["key"])
+        if not 0 <= k <= 0xffffffff:
+            raise ValueError("Seed must be between 0 and 2**32 - 1")                  # np.random.seed's range
+        seeds[i] = k
+    return seeds
+
+
 def seeded_stats_batch(prob, items, num_prime, noise_level, noise, num_obs, want_draws=False, device=None, n_roll=NUM_ROLLOUTS):
     """`compute_stats_batch` with the legacy-stream noise drawn on the GPU (mpcmmd_validate_seeded_host, csrc/k_validate_noise.cuh):
     the planned controls are computed here, each trajectory's stream is np.random.seed(item["key"]) restated on the device.
@@ -153,12 +170,7 @@ def seeded_stats_batch(prob, items, num_prime, noise_level, noise, num_obs, want
     if n == 0:
         z = np.zeros(0, np.int64)
         return (z, z, np.zeros((0, n_roll, num_prime)), np.zeros((0, n_roll, num_prime)), np.zeros((0, STATE_WORDS), np.uint32)) if want_draws else (z, z)
-    seeds = np.empty(n, np.uint32)
-    for i, it in enumerate(items):
-        k = int(it["key"])
-        if not 0 <= k <= 0xffffffff:
-            raise ValueError("Seed must be between 0 and 2**32 - 1")                  # np.random.seed's range
-        seeds[i] = k
+    seeds = _seeds(items)
     if not _mvn_identity_is_exact(num_prime):
         raise RuntimeError("multivariate_normal(0, eye(%d)) is not exactly standard_normal with this LAPACK: use rng='host'" % num_prime)
     acc_p, steer_p, state0, xo, yo, static = _inputs(prob, items, num_prime, num_obs)
@@ -177,6 +189,37 @@ def seeded_stats_batch(prob, items, num_prime, noise_level, noise, num_obs, want
         float(prob.a_obs), float(prob.b_obs), float(prob.y_lb), float(prob.y_ub), p(seeds), p(acc_p), p(steer_p), p(state0), p(xo), p(yo),
         p(count), p(lane), p(acc), p(steer), p(state)))
     return (count, lane, acc, steer, state) if want_draws else (count, lane)
+
+
+def threefry_stats_batch(prob, items, num_prime, noise_level, noise, num_obs, want_draws=False, device=None, n_roll=NUM_ROLLOUTS):
+    """`compute_stats_batch` with counter-based noise (mpcmmd_validate_threefry_host, csrc/k_validate_jax.cuh; DESIGN.md section 3
+    item 7): trajectory i's noise is JAX's random.beta / random.normal of split(PRNGKey(item["key"]), 3) over an (n_roll, num_prime)
+    array, drawn by each rollout as it rolls out.  No shape parameter check (JAX makes none: at num_prime = 100 the acceleration
+    draws of the last knot are NaN and reach only the discarded final state).  Returns count, count_lane (n,) [, acc, steer
+    (n, n_roll, num_prime) perturbed controls]."""
+    if noise not in B.NOISE_KINDS:
+        raise ValueError("noise must be one of %s, not %r" % (sorted(B.NOISE_KINDS), noise))
+    if isinstance(n_roll, bool) or not isinstance(n_roll, (int, np.integer)) or n_roll < 1:
+        raise ValueError("n_roll must be an integer >= 1, not %r" % (n_roll,))
+    if int(n_roll) * int(num_prime) >= 2 ** 31:
+        raise ValueError("n_roll * num_prime must be below 2**31 (JAX's uint32 element counters)")
+    n = len(items)
+    if n == 0:
+        z = np.zeros(0, np.int64)
+        return (z, z, np.zeros((0, n_roll, num_prime)), np.zeros((0, n_roll, num_prime))) if want_draws else (z, z)
+    seeds = _seeds(items)
+    acc_p, steer_p, state0, xo, yo, static = _inputs(prob, items, num_prime, num_obs)
+    count = np.zeros(n, np.int32); lane = np.zeros(n, np.int32)
+    acc = np.empty((n, n_roll, num_prime)) if want_draws else None
+    steer = np.empty((n, n_roll, num_prime)) if want_draws else None
+    dev = prob.device.index if device is None else int(device)
+    p = lambda a: None if a is None else a.ctypes.data_as(C.c_void_p)
+    B.check(B.load().mpcmmd_validate_threefry_host(
+        dev or 0, n, int(n_roll), num_prime, num_obs, 1 if static else 0, B.NOISE_KINDS[noise], float(noise_level), float(prob.cem_helper.K_steer),
+        float(prob.beta_a), float(prob.beta_b), float(prob.acc_const_noise), float(prob.steer_const_noise), float(prob.t), float(prob.wheel_base),
+        float(prob.a_obs), float(prob.b_obs), float(prob.y_lb), float(prob.y_ub), p(seeds), p(acc_p), p(steer_p), p(state0), p(xo), p(yo),
+        p(count), p(lane), p(acc), p(steer)))
+    return (count, lane, acc, steer) if want_draws else (count, lane)
 
 
 def _load(root, noise, noise_level, num_prime, cost, num_reduced, num_obs):
@@ -228,13 +271,15 @@ def run_validation(args, variant="static", device=0, log=print):
                         log((len(pairs), _matrix(data_cvar, num_obs).shape[1]))                     # the reference prints eset.shape
                         # both costs of a scene share the seed k (validation.py:315-336)
                         items = [_item(data_mmd_opt, im, k, dynamic) for k, _, im in pairs] + [_item(data_cvar, ic, k, dynamic) for k, ic, _ in pairs]
-                        count, lane = compute_stats_batch(prob, items, num_prime, noise_level, noise, num_obs, rng=args.rng)
+                        count, lane = compute_stats_batch(prob, items, num_prime, noise_level, noise, num_obs, n_roll=args.num_rollouts, rng=args.rng)
                         m = len(pairs)
                         f = lambda a: np.asarray(a, np.float64)                                   # np.append([], int) yields float64 arrays
                         path = "{}/{}_noise/noise_{}/ts_{}/{}_samples_{}_obs".format(args.stats_root, noise, int(noise_level * 100), num_prime, num_reduced, num_obs)
                         os.makedirs(os.path.dirname(path), exist_ok=True)
+                        # counts that are not the reference's estimator (other noise or other rollout count) say so in the file
+                        tag = dict(rng=args.rng, num_rollouts=args.num_rollouts) if args.rng == "jax" or args.num_rollouts != NUM_ROLLOUTS else {}
                         np.savez(path, coll_cvar=f(count[m:]), coll_cvar_lane=f(lane[m:]), coll_mmd_opt=f(count[:m]), coll_mmd_opt_lane=f(lane[:m]),
-                                 coll_mmd_random=[], coll_mmd_random_lane=[])
+                                 coll_mmd_random=[], coll_mmd_random_lane=[], **tag)
                         written.append(path + ".npz")
                         del prob
     return written
@@ -252,10 +297,20 @@ def build_parser():
     p.add_argument("--root", type=str, default="./data")
     p.add_argument("--stats_root", type=str, default="./stats")
     p.add_argument("--variant", type=str, default="static", choices=["static", "dynamic"])
-    p.add_argument("--rng", type=str, default="host", choices=["host", "device"],
+    p.add_argument("--rng", type=str, default="host", choices=["host", "device", "jax"],
                    help="host (default): NumPy's legacy stream, as the reference; device: the same stream drawn on the GPU (identical "
-                        "consumption, values within CUDA's pow / log / exp rounding)")
+                        "consumption, values within CUDA's pow / log / exp rounding); jax: counter-based JAX-protocol noise drawn by each "
+                        "rollout on the GPU (same distributions, not the reference's numbers)")
+    p.add_argument("--num_rollouts", type=_positive_int, default=NUM_ROLLOUTS,
+                   help="noisy rollouts per planned trajectory (default %d, the reference's _num_batch)" % NUM_ROLLOUTS)
     return p
+
+
+def _positive_int(s):
+    v = int(s)
+    if v < 1:
+        raise argparse.ArgumentTypeError("must be >= 1, not %d" % v)
+    return v
 
 
 def main(argv=None, variant=None):
