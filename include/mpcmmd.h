@@ -33,6 +33,9 @@ extern "C" {
 
 enum { MPCMMD_COST_MMD_OPT = 0, MPCMMD_COST_MMD_RANDOM = 1, MPCMMD_COST_CVAR = 2, MPCMMD_COST_SAA = 3 };
 enum { MPCMMD_NOISE_GAUSSIAN = 0, MPCMMD_NOISE_BETA = 1 };
+/* kernel of the MMD risk costs (mmd_opt, mmd_random): Laplace exp(-|d|_1 / sigma) as the reference, or Gaussian exp(-|d|_2^2 / (2 sigma^2)).
+ * DESIGN.md section 3 items 4 and 8 fix the float32 arithmetic of both. */
+enum { MPCMMD_KERNEL_LAPLACE = 0, MPCMMD_KERNEL_GAUSSIAN = 1 };
 
 /* Every constant of CEM.__init__ (cem.py:20-171) the hot path reads.  The matrices are HOST
  * pointers, copied to the device by mpcmmd_create; the host shim computes them once in float64
@@ -89,6 +92,10 @@ int mpcmmd_version(void);
 /* Environment read here: MPCMMD_PROJ = tc | tc-always selects the tensor-core projection kernel (k_project_tc: tcgen05 kind::tf32 products,
  * 1e-4 stage parity) for throughput-sized / all launches; unset = the bit-exact FP32 kernel.  See INTEGRATION.md. */
 int mpcmmd_create(const mpcmmd_config *cfg, int device, mpcmmd_handle *out);
+/* mpcmmd_create with the MMD kernel chosen (MPCMMD_KERNEL_*; mpcmmd_create = MPCMMD_KERNEL_LAPLACE).  The kernel is fixed for the handle's
+ * lifetime: every solve and stage entry point of the handle uses it.  Unknown kinds are refused.  A Gaussian handle is refused when
+ * MPCMMD_INNER_CEM = warp | pipe | split or MPCMMD_CHOL = la | cta select an experimental inner-CEM kernel: those exist for Laplace only. */
+int mpcmmd_create_with_kernel(const mpcmmd_config *cfg, int mmd_kernel, int device, mpcmmd_handle *out);
 int mpcmmd_destroy(mpcmmd_handle h);
 
 /* n_ep solves, all pointers DEVICE pointers; asynchronous on `stream` (a cudaStream_t, 0 = default).
@@ -168,7 +175,8 @@ int mpcmmd_selfcheck_ieee(int device, unsigned long long *mismatches /* [3], hos
 /* ---- stage entry points (teacher-forced parity tests; all DEVICE pointers, synchronous) ---- */
 
 /* deterministic math / RNG primitives: fn 0 exp,1 log,2 log1p,3 sin,4 cos,5 tan,6 atan,7 atan2(y,x),8 erfinv, 9 exp on x <= 0, 10/11 sincos,
- * 12 Laplace kernel entry k(d = x; sigma = y) = 2^(-(d s2)) of the reduced-set inner CEM (kernel_computation.py:31-37; DESIGN.md 3.4) */
+ * 12 Laplace kernel entry k(d = x; sigma = y) = 2^(-(d s2)) of the reduced-set inner CEM (kernel_computation.py:31-37; DESIGN.md 3.4),
+ * 13 Gaussian kernel entry k(q = x; sigma = y) = 2^(-(q g2)), q a squared distance (DESIGN.md 3.8) */
 int mpcmmd_math_vec(int fn, const float *x, const float *y, float *out, int n, int device);
 int mpcmmd_rng_normal(uint32_t k0, uint32_t k1, int n, float *out, int device);
 int mpcmmd_rng_beta(uint32_t k0, uint32_t k1, const float *a, const float *b, int n, float *out, int device);

@@ -21,6 +21,8 @@ struct DCfg {
     float lam_inv, one_m_alpha_mean, alpha_mean, one_m_alpha_cov, alpha_cov;
     float sigma_clip, inv_nm, m2_inv_nm, beta_del, sigma_random;
     float obs_win;                                           // half-width of the x window outside of which the obstacle indicator is exactly 0: sqrt(a2_obs) + 0.01
+    int kernel;                                              // MMD kernel form (dm::KER_*) of the scalar-cost MMD (the inner-CEM kernels take it as a template argument); fills the
+                                                             // alignment gap before the pointers, so no other member moves
     const float *P, *Pd, *Pdd, *Gx, *Gy, *Kx, *Ky, *Wfit;   // device copies of the host constants
     const float* proj_const;                                 // P | Pd | Pdd | Gx | Gy | Kx | Ky as ONE 16-byte-aligned block (bulk-copied into shared memory by k_project)
     const float* proj_tc_const;                              // tf32 (hi, lo) images of P / Pd / Pdd + Gx | Gy | Kx | Ky for k_project_tc

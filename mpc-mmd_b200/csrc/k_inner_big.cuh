@@ -48,10 +48,11 @@ __device__ __forceinline__ void big_topk(const float* __restrict__ row, int nm, 
     }
 }
 // the (nr+1) KKT solve and the cost of one beta sample; same operation order as beta_finish<NR> (k_risk.cuh), arrays in memory
+template <int KER>
 __device__ __forceinline__ float big_finish(const DCfg& c, int nr, int nm, const int* __restrict__ ti, float sigma, const float* __restrict__ rowsum,
                                             const float* __restrict__ D, float* __restrict__ beta, float* __restrict__ K, float* __restrict__ Lm,
                                             float* __restrict__ rd, float* __restrict__ u, float* __restrict__ w) {
-    const dm::LapScale ls = dm::lap_scale(sigma);
+    const dm::LapScale ls = dm::kern_scale<KER>(sigma);
     for (int i = 0; i < nr; i++) {
         K[i * nr + i] = 1.0f;
         for (int j = 0; j < i; j++) { const float k = dm::lap_(D[(size_t)ti[i] * nm + ti[j]], ls); K[i * nr + j] = k; K[j * nr + i] = k; }
@@ -91,8 +92,8 @@ __device__ __forceinline__ float big_finish(const DCfg& c, int nr, int nm, const
     return s1 + s2;
 }
 
-// one CTA per chain; chain g of this launch uses state block (g - g_base) (the host launches chain ranges that fit the scratch budget)
-template <int NT>
+// one CTA per chain; chain g of this launch uses state block (g - g_base) (the host launches chain ranges that fit the scratch budget); KER: MMD kernel form
+template <int NT, int KER = dm::KER_LAPLACE>
 __global__ void __launch_bounds__(NT) k_inner_cem_big(DCfg c, RollArgs ra, float* __restrict__ state, int g_base, int n_chains) {
     __shared__ float blk[16];
     __shared__ float red[3 * MPCMMD_MAX_NR_DEV * (NT / 32)];
@@ -114,7 +115,7 @@ __global__ void __launch_bounds__(NT) k_inner_cem_big(DCfg c, RollArgs ra, float
         const float* Fa = F + (i / nm) * 2 * NV; const float* Fb = F + (i % nm) * 2 * NV;
         float dist = 0.0f;
 #pragma unroll
-        for (int f = 0; f < 2 * NV; f++) dist = dist + fabsf(Fa[f] - Fb[f]);
+        for (int f = 0; f < 2 * NV; f++) dist = dm::kern_dist_acc<KER>(dist, Fa[f], Fb[f]);
         D[i] = dist;
     }
     for (size_t i = tid; i < (size_t)S * d; i += nt) th[i] = __ldg(c.theta0 + i);
@@ -127,12 +128,12 @@ __global__ void __launch_bounds__(NT) k_inner_cem_big(DCfg c, RollArgs ra, float
         __syncthreads();
         for (int task = tid; task < (S - s0) * nr; task += nt) {
             const int s = s0 + task / nr, i = task % nr;
-            rs[s * nr + i] = beta_rowsum(D, nm, idxs[s * nr + i], th[(size_t)s * d + nm]);
+            rs[s * nr + i] = beta_rowsum<KER>(D, nm, idxs[s * nr + i], th[(size_t)s * d + nm]);
         }
         __syncthreads();
         for (int s = s0 + tid; s < S; s += nt) {
             float* ks = st + L.kscr + (size_t)s * L.kstride;
-            cost[s] = big_finish(c, nr, nm, idxs + s * nr, th[(size_t)s * d + nm], rs + s * nr, D, betas + s * nr, ks, ks + nr * nr, ks + 2 * nr * nr,
+            cost[s] = big_finish<KER>(c, nr, nm, idxs + s * nr, th[(size_t)s * d + nm], rs + s * nr, D, betas + s * nr, ks, ks + nr * nr, ks + 2 * nr * nr,
                                  ks + 2 * nr * nr + nr, ks + 2 * nr * nr + 2 * nr);
         }
         __syncthreads();
@@ -336,7 +337,7 @@ __global__ void __launch_bounds__(NT) k_inner_cem_big(DCfg c, RollArgs ra, float
         }
         const float sigma = small[200];
         a.sigma[g] = sigma;
-        a.risk[g] = mmd_cost(c, beta, cs, sigma);
-        a.lane[g] = mmd_cost(c, beta, lbv, sigma) + mmd_cost(c, beta, ubv, sigma);
+        a.risk[g] = mmd_cost<KER>(c, beta, cs, sigma);
+        a.lane[g] = mmd_cost<KER>(c, beta, lbv, sigma) + mmd_cost<KER>(c, beta, ubv, sigma);
     }
 }

@@ -35,13 +35,14 @@ __device__ __forceinline__ float ex2_approx(float x) { float y; asm("ex2.approx.
 }  // namespace pk
 
 // Laplace kernel entries k(d; sigma) two at a time (dm::lap_ per lane, operation for operation).  LapK carries the per-bandwidth constants: exact contract
-// (FM = false): sc2 = (-s2, -s2) and the distance cap; fast math (FM = true): sc2 = -(1/sigma) * log2(e) in both lanes, the exponentials run on the XU pipe (MUFU.EX2).
+// (FM = false): sc2 = (-s2, -s2) and the distance cap; fast math (FM = true): sc2 = -s2 in both lanes, the exponentials run on the XU pipe (MUFU.EX2).
+// KER = kernel form (dm::KER_*): the Gaussian entry is the same function of a stored squared distance with its own scale g2 in place of s2 (dm::kern_scale).
 struct LapK { pk::f2 sc2; float dcap; };
-template <bool FM>
+template <bool FM, int KER = dm::KER_LAPLACE>
 __device__ __forceinline__ LapK lap_k(float sigma) {
     LapK k;
-    if constexpr (FM) { const float rinv = 1.0f / sigma; k.sc2 = pk::dup(-rinv * 1.44269504088896341f); k.dcap = 0.0f; }
-    else { const dm::LapScale L = dm::lap_scale(sigma); k.sc2 = pk::dup(L.ns2); k.dcap = L.dcap; }
+    if constexpr (FM) { k.sc2 = pk::dup(dm::kern_ns2<KER>(sigma)); k.dcap = 0.0f; }
+    else { const dm::LapScale L = dm::kern_scale<KER>(sigma); k.sc2 = pk::dup(L.ns2); k.dcap = L.dcap; }
     return k;
 }
 namespace pk {
@@ -132,13 +133,13 @@ __device__ __noinline__ int top_abs_exact(const float* __restrict__ row) {     /
 // the QP + MMD cost of one beta sample given its reduced set (indices ti, ascending |theta|) and bandwidth sigma
 // [compute_beta.py:70-91, 120-129]; bit-identical to the second half of beta_sample<NR> of k_risk.cuh
 // LDD = row stride of D in floats; a multiple of four selects the vectorised row-sum loop (four columns per 16-byte load, same operations in the same order)
-template <int NR, bool FM = false, int LDD = NR * NR>
+template <int NR, bool FM = false, int LDD = NR * NR, int KER = dm::KER_LAPLACE>
 __device__ __forceinline__ float beta_eval(const DCfg& c, const int (&ti)[NR], float sigma, const float* __restrict__ D,
                                            float* __restrict__ beta_out, int* __restrict__ idx_out /* one packed word */) {
     constexpr int nm = NR * NR;
     constexpr bool VEC = (LDD % 4 == 0) && nm >= 4;
     constexpr int MV = VEC ? (nm & ~3) : 0;          // columns handled by the vectorised loop
-    const LapK rinv2 = lap_k<FM>(sigma);
+    const LapK rinv2 = lap_k<FM, KER>(sigma);
     // ---- ker_mixed row sums: rowsum_i = sum_m k(D[idx_i][m]; sigma), ascending m  [kernel_computation.py:31-37, compute_beta.py:77]
     constexpr int NP = NR / 2;                       // pairs of reduced rows handled together
     pk::f2 rs2[NP > 0 ? NP : 1];
@@ -275,7 +276,7 @@ __device__ __forceinline__ float beta_eval(const DCfg& c, const int (&ti)[NR], f
 }
 
 // one beta sample of the inner CEM [compute_beta.py:113-129, 70-91]; bit-identical to beta_sample<NR> of k_risk.cuh
-template <int NR, bool FM = false, int LDD = NR * NR>
+template <int NR, bool FM = false, int LDD = NR * NR, int KER = dm::KER_LAPLACE>
 __device__ __forceinline__ float beta_sample_fast(const DCfg& c, const float* __restrict__ row, const float* __restrict__ D,
                                                   float* __restrict__ beta_out, int* __restrict__ idx_out /* one packed word */) {
     constexpr int nm = NR * NR;
@@ -322,7 +323,7 @@ __device__ __forceinline__ float beta_sample_fast(const DCfg& c, const float* __
 #pragma unroll
         for (int p = 0; p < NR; p++) ti[p] = (pkd >> (5 * p)) & 31;
     }
-    return beta_eval<NR, FM, LDD>(c, ti, row[nm], D, beta_out, idx_out);
+    return beta_eval<NR, FM, LDD, KER>(c, ti, row[nm], D, beta_out, idx_out);
 }
 
 // float -> uint32 whose unsigned order is "ascending float, -0 == +0, NaN last" (jnp.argsort order of the costs)
@@ -689,7 +690,8 @@ template <int d> __device__ __forceinline__ void icl_chol_regs(float* __restrict
 // whole shared-memory layout folds into immediate offsets, which takes the address arithmetic the 56-register cap otherwise re-derives in every phase out of the kernel
 // CH = Cholesky of the covariance: 0 one-warp panel factorisation (icf_chol_panel), 1 two-warp look-ahead (icl_chol_lookahead), 2 CTA-wide panels (icf_chol_cta);
 // MPCMMD_CHOL=panel|la|cta selects the build of the specialised throughput kernel
-template <int NR, bool LAT, bool FM = false, int SC = 0, int NEC = 0, int CH = 0>
+// KER = MMD kernel form (dm::KER_*): changes only the distance table and the per-bandwidth scale
+template <int NR, bool LAT, bool FM = false, int SC = 0, int NEC = 0, int CH = 0, int KER = dm::KER_LAPLACE>
 __global__ void __launch_bounds__(ICF_THREADS, LAT ? 3 : 12) k_inner_cem_fast(DCfg c, RollArgs ra) {
     extern __shared__ __align__(128) float sm[];
     const RiskArgs& a = ra.r;
@@ -719,7 +721,7 @@ __global__ void __launch_bounds__(ICF_THREADS, LAT ? 3 : 12) k_inner_cem_fast(DC
             const float* Fa = F + (i / nm) * 2 * NV; const float* Fb = F + (i % nm) * 2 * NV;
             float dist = 0.0f;
 #pragma unroll 2
-            for (int f = 0; f < 2 * NV; f++) dist = dist + fabsf(Fa[f] - Fb[f]);
+            for (int f = 0; f < 2 * NV; f++) dist = dm::kern_dist_acc<KER>(dist, Fa[f], Fb[f]);
             D[(i / nm) * LDD + i % nm] = dist;
         }
         __syncthreads();
@@ -753,7 +755,7 @@ __global__ void __launch_bounds__(ICF_THREADS, LAT ? 3 : 12) k_inner_cem_fast(DC
         const int nrow = S - ne;
         // -- evaluate the new rows (the elites keep last iteration's cost: same row => same arithmetic => same bits)
 #pragma unroll 1
-        for (int s = tid; s < n_new; s += nt) cost[s] = beta_sample_fast<NR, FM, LDD>(c, s < nrow ? th + s * ldt : eth + (s - nrow) * ldt, D, betas + s * NR, idxs + s);
+        for (int s = tid; s < n_new; s += nt) cost[s] = beta_sample_fast<NR, FM, LDD, KER>(c, s < nrow ? th + s * ldt : eth + (s - nrow) * ldt, D, betas + s * NR, idxs + s);
         __syncthreads();
         // -- stable argsort, first ne entries: candidate j < n_old is elite j, else new row j - n_old  [compute_beta.py:56]
         if (warp == 0) icf_select(lane, S, n_old, ne, ecost, cost, perm, ecost);
@@ -877,19 +879,19 @@ __global__ void __launch_bounds__(OPT_RISK_THREADS) k_opt_risk(DCfg c, RollArgs 
         vals[tid] = m; vals[OPT_RISK_THREADS + tid] = l; vals[2 * OPT_RISK_THREADS + tid] = u;
     }
     __syncthreads();
-    // the three Laplace-kernel MMD values of the sample [kernel_computation.py:67-87]: thread r evaluates kernel row r of each (ascending-j fma chains, 3 (nr + 1)
+    // the three MMD values of the sample [kernel_computation.py:67-87]: thread r evaluates kernel row r of each (ascending-j fma chains, 3 (nr + 1)
     // exponentials instead of 3 nr (nr + 1) on one thread), thread 0 of the sample folds the rows in ascending i -- the operations of mmd_cost in the same order
     __shared__ float rows_t[3 * OPT_RISK_THREADS], rows_u[3 * OPT_RISK_THREADS];
     if (live) {
-        const float sigma = a.sigma[g];
+        const float v = dm::kern_cost_v(c.kernel, a.sigma[g]);
         const int base = tid - r;
 #pragma unroll
         for (int q = 0; q < 3; q++) {
             const float* cst = vals + q * OPT_RISK_THREADS + base;
             const float ci = cst[r];
             float t = 0.0f;
-            for (int j = 0; j < nr; j++) t = fmaf(dm::exp_(-fabsf(ci - cst[j]) / sigma), a.beta[(size_t)g * nr + j], t);
-            const float e = dm::exp_(-fabsf(ci - 0.0f) / sigma);
+            for (int j = 0; j < nr; j++) t = fmaf(dm::kern_cost(c.kernel, ci - cst[j], v), a.beta[(size_t)g * nr + j], t);
+            const float e = dm::kern_cost(c.kernel, ci - 0.0f, v);
             float u = 0.0f;
             for (int j = 0; j < nr; j++) u = fmaf(e, c.beta_del, u);
             rows_t[q * OPT_RISK_THREADS + tid] = t; rows_u[q * OPT_RISK_THREADS + tid] = u;
@@ -958,10 +960,10 @@ __device__ __forceinline__ int icl_topk(const float* __restrict__ row) {
     return packed;
 }
 // sum_m k(D[row][m]; sigma), m ascending, two kernel entries per packed evaluation: one lane of beta_eval's row-sum loop
-template <int NR>
+template <int NR, int KER>
 __device__ __forceinline__ float icl_rowsum(const float* __restrict__ Drow, float sigma) {
     constexpr int nm = NR * NR;
-    const LapK rinv2 = lap_k<false>(sigma);
+    const LapK rinv2 = lap_k<false, KER>(sigma);
     float rs = 0.0f;
 #pragma unroll 4
     for (int m = 0; m + 1 < nm; m += 2) {
@@ -972,11 +974,11 @@ __device__ __forceinline__ float icl_rowsum(const float* __restrict__ Drow, floa
     return rs;
 }
 // reduced kernel, KKT solve and cost of one beta sample from its row sums: second half of beta_eval, operation for operation
-template <int NR, int LDD = NR * NR>
+template <int NR, int LDD, int KER>
 __device__ __forceinline__ float icl_finish(const DCfg& c, int packed, float sigma, const float* __restrict__ rowsum, const float* __restrict__ D,
                                             float* __restrict__ beta_out) {
     constexpr int nm = NR * NR;
-    const LapK rinv2 = lap_k<false>(sigma);
+    const LapK rinv2 = lap_k<false, KER>(sigma);
     int ti[NR];
 #pragma unroll
     for (int i = 0; i < NR; i++) ti[i] = (packed >> (5 * i)) & 31;
@@ -1204,7 +1206,7 @@ __device__ __forceinline__ void icl_chol_regs(float* __restrict__ C, int lane) {
     __syncwarp();
 }
 
-template <int NR, int SC = 0, int NEC = 0>          // SC / NEC: compile-time sample / elite counts, see k_inner_cem_fast
+template <int NR, int SC = 0, int NEC = 0, int KER = dm::KER_LAPLACE>          // SC / NEC: compile-time sample / elite counts, KER: kernel form, see k_inner_cem_fast
 __global__ void __launch_bounds__(ICL_THREADS, 1) k_inner_cem_lat(DCfg c, RollArgs ra) {
     extern __shared__ __align__(128) float sm[];
     const RiskArgs& a = ra.r;
@@ -1234,7 +1236,7 @@ __global__ void __launch_bounds__(ICL_THREADS, 1) k_inner_cem_lat(DCfg c, RollAr
             const float* Fa = F + (i / nm) * 2 * NV; const float* Fb = F + (i % nm) * 2 * NV;
             float dist = 0.0f;
 #pragma unroll 2
-            for (int f = 0; f < 2 * NV; f++) dist = dist + fabsf(Fa[f] - Fb[f]);
+            for (int f = 0; f < 2 * NV; f++) dist = dm::kern_dist_acc<KER>(dist, Fa[f], Fb[f]);
             D[(i / nm) * LDD + i % nm] = dist;
         }
         __syncthreads();
@@ -1260,12 +1262,12 @@ __global__ void __launch_bounds__(ICL_THREADS, 1) k_inner_cem_lat(DCfg c, RollAr
 #pragma unroll 1
         for (int task = tid; task < n_new * NR; task += nt) {
             const int s = task / NR, i = task - s * NR;
-            rsum[task] = icl_rowsum<NR>(D + ((tis[s] >> (5 * i)) & 31) * LDD, rows[s * rstride + nm]);
+            rsum[task] = icl_rowsum<NR, KER>(D + ((tis[s] >> (5 * i)) & 31) * LDD, rows[s * rstride + nm]);
         }
         __syncthreads();
 #pragma unroll 1
         for (int s = tid; s < n_new; s += nt) {
-            cost[s] = icl_finish<NR, LDD>(c, tis[s], rows[s * rstride + nm], rsum + s * NR, D, betas + s * NR);
+            cost[s] = icl_finish<NR, LDD, KER>(c, tis[s], rows[s * rstride + nm], rsum + s * NR, D, betas + s * NR);
             idxs[s] = tis[s];
         }
         __syncthreads();

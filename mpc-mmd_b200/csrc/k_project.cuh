@@ -72,6 +72,7 @@ __global__ void k_math_vec(int fn, const float* x, const float* y, float* out, i
             case 10: { float s, cc; dm::sincos_(x[i], s, cc); v = s; } break;
             case 11: { float s, cc; dm::sincos_(x[i], s, cc); v = cc; } break;
             case 12: v = dm::lap_(x[i], dm::lap_scale(y[i])); break;          // Laplace kernel entry k(d = x; sigma = y) of the reduced-set inner CEM
+            case 13: v = dm::lap_(x[i], dm::kern_scale<dm::KER_GAUSSIAN>(y[i])); break;      // Gaussian kernel entry k(q = x; sigma = y), q a squared distance
             default: v = DM_NAN;
         }
         out[i] = v;

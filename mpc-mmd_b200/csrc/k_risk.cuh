@@ -77,32 +77,35 @@ __device__ __forceinline__ void rollout_fit(const DCfg& c, const float* a, const
 #pragma unroll
     for (int k = 0; k < NV; k++) { feat[k] = fx[k]; feat[NV + k] = fy[k]; }
 }
-// Laplace-kernel MMD of nr scalar costs against the zero cost  [kernel_computation.py:67-87]
+// MMD of nr scalar costs against the zero cost, kernel form KER (dm::KER_*)  [kernel_computation.py:67-87]
+template <int KER = dm::KER_LAPLACE>
 __device__ __noinline__ float mmd_cost(const DCfg& c, const float* beta, const float* cost, float sigma) {
     const int nr = c.nr;
+    const float v = dm::kern_cost_v(KER, sigma);
     float s1 = 0.0f, s2 = 0.0f;
     for (int i = 0; i < nr; i++) {
         float t = 0.0f;
-        for (int j = 0; j < nr; j++) t = fmaf(dm::exp_(-fabsf(cost[i] - cost[j]) / sigma), beta[j], t);
+        for (int j = 0; j < nr; j++) t = fmaf(dm::kern_cost(KER, cost[i] - cost[j], v), beta[j], t);
         s1 = fmaf(beta[i], t, s1);
-        float e = dm::exp_(-fabsf(cost[i] - 0.0f) / sigma), u = 0.0f;
+        float e = dm::kern_cost(KER, cost[i] - 0.0f, v), u = 0.0f;
         for (int j = 0; j < nr; j++) u = fmaf(e, c.beta_del, u);
         s2 = fmaf(beta[i], u, s2);
     }
     return c.ker_wt * (s1 - 2.0f * s2);
 }
 // the same value computed by a whole warp (num_reduced <= 64): lane l evaluates the kernel rows i = l, l + 32 as the same ascending-j
-// fma chains, then every lane folds them in ascending i -- bit-identical to mmd_cost, nr^2 / 32 exps per lane instead of nr^2 on one
+// fma chains, then every lane folds them in ascending i -- bit-identical to mmd_cost, nr^2 / 32 exps per lane instead of nr^2 on one.  Kernel form: c.kernel
 __device__ __forceinline__ float mmd_cost_warp(const DCfg& c, const float* beta, const float* cost, float sigma, int lane) {
     const int nr = c.nr;
+    const float v = dm::kern_cost_v(c.kernel, sigma);
     float tv[2] = {0.0f, 0.0f}, uv[2] = {0.0f, 0.0f};
 #pragma unroll
     for (int h = 0; h < 2; h++) {
         const int i = lane + 32 * h;
         if (i < nr) {
             float t = 0.0f;
-            for (int j = 0; j < nr; j++) t = fmaf(dm::exp_(-fabsf(cost[i] - cost[j]) / sigma), beta[j], t);
-            const float e = dm::exp_(-fabsf(cost[i] - 0.0f) / sigma);
+            for (int j = 0; j < nr; j++) t = fmaf(dm::kern_cost(c.kernel, cost[i] - cost[j], v), beta[j], t);
+            const float e = dm::kern_cost(c.kernel, cost[i] - 0.0f, v);
             float u = 0.0f;
             for (int j = 0; j < nr; j++) u = fmaf(e, c.beta_del, u);
             tv[h] = t; uv[h] = u;
@@ -502,19 +505,20 @@ __device__ __forceinline__ void beta_topk(const float* __restrict__ row, int* __
 #pragma unroll
     for (int i = 0; i < NR; i++) ti_out[i] = ti[i];
 }
-// sum_m exp(-(D[m][ti] / sigma)), ascending m  [kernel_computation.py:31-37, compute_beta.py:77]; D is symmetric bit for bit
+// sum_m k(D[m][ti]; sigma), ascending m  [kernel_computation.py:31-37, compute_beta.py:77]; D is symmetric bit for bit
+template <int KER = dm::KER_LAPLACE>
 __device__ __forceinline__ float beta_rowsum(const float* __restrict__ D, int nm, int ti, float sigma) {
-    const dm::LapScale ls = dm::lap_scale(sigma);
+    const dm::LapScale ls = dm::kern_scale<KER>(sigma);
     float acc = 0.0f;
 #pragma unroll 4
     for (int m = 0; m < nm; m++) acc = acc + dm::lap_(D[m * nm + ti], ls);
     return acc;
 }
-template <int NR>
+template <int NR, int KER = dm::KER_LAPLACE>
 __device__ __forceinline__ float beta_finish(const DCfg& c, const int* __restrict__ ti, float sigma, const float* __restrict__ rowsum,
                                              const float* __restrict__ D, float* __restrict__ beta_out) {
     constexpr int nm = NR * NR;
-    const dm::LapScale ls = dm::lap_scale(sigma);
+    const dm::LapScale ls = dm::kern_scale<KER>(sigma);
     float K[NR][NR];                               // ker_red (symmetric bit for bit); diagonal: k(0) = 1
 #pragma unroll
     for (int i = 0; i < NR; i++) {
@@ -574,14 +578,14 @@ __device__ __forceinline__ float beta_finish(const DCfg& c, const int* __restric
     return s1 + s2;
 }
 
-template <int NR>
+template <int NR, int KER = dm::KER_LAPLACE>
 __device__ __forceinline__ float beta_sample(const DCfg& c, const float* __restrict__ row, const float* __restrict__ D,
                                              float* __restrict__ beta_out, int* __restrict__ idx_out) {
     constexpr int nm = NR * NR;
     int ti[NR];
     beta_topk<NR>(row, ti);
     const float sigma = row[nm];
-    const dm::LapScale ls = dm::lap_scale(sigma);
+    const dm::LapScale ls = dm::kern_scale<KER>(sigma);
     float rowsum[NR];
 #pragma unroll
     for (int i = 0; i < NR; i++) rowsum[i] = 0.0f;
@@ -593,7 +597,7 @@ __device__ __forceinline__ float beta_sample(const DCfg& c, const float* __restr
     }
 #pragma unroll
     for (int i = 0; i < NR; i++) idx_out[i] = ti[i];
-    return beta_finish<NR>(c, ti, sigma, rowsum, D, beta_out);
+    return beta_finish<NR, KER>(c, ti, sigma, rowsum, D, beta_out);
 }
 
 // float -> int64 key whose signed order is "ascending float, -0 == +0, NaN last", tie-broken by the index in the low bits
@@ -606,7 +610,8 @@ __device__ __forceinline__ long long sort_key64(float x, int idx) {
 }
 
 // SC / NEC: compile-time copies of the inner CEM's sample / elite counts (0 = from the configuration), as in k_inner_cem_fast: the shared-memory layout folds
-template <int NR, int SC = 0, int NEC = 0>
+// KER: MMD kernel form (dm::KER_*)
+template <int NR, int SC = 0, int NEC = 0, int KER = dm::KER_LAPLACE>
 __global__ void __launch_bounds__(risko_threads(NR), (NR <= 5) ? 7 : 1) k_inner_cem(DCfg c, RollArgs ra) {
     extern __shared__ __align__(128) float sm[];
     const RiskArgs& a = ra.r;
@@ -632,7 +637,7 @@ __global__ void __launch_bounds__(risko_threads(NR), (NR <= 5) ? 7 : 1) k_inner_
         const float* Fa = F + (i / nm) * 2 * NV; const float* Fb = F + (i % nm) * 2 * NV;
         float dist = 0.0f;
 #pragma unroll
-        for (int f = 0; f < 2 * NV; f++) dist = dist + fabsf(Fa[f] - Fb[f]);
+        for (int f = 0; f < 2 * NV; f++) dist = dm::kern_dist_acc<KER>(dist, Fa[f], Fb[f]);
         D[i] = dist;
     }
     // ---- inner CEM  [compute_beta.py:93-157]
@@ -649,7 +654,7 @@ __global__ void __launch_bounds__(risko_threads(NR), (NR <= 5) ? 7 : 1) k_inner_
         // -- evaluate the new samples (all of them in iteration 0; afterwards rows 0..ne-1 are last iteration's elites)
         if constexpr (SMALL) {
 #pragma unroll 1
-            for (int s = (it == 0 ? 0 : ne) + tid; s < S; s += nt) cost[s] = beta_sample<NR>(c, th + s * d, D, betas + s * NR, idxs + s * NR);
+            for (int s = (it == 0 ? 0 : ne) + tid; s < S; s += nt) cost[s] = beta_sample<NR, KER>(c, th + s * d, D, betas + s * NR, idxs + s * NR);
         } else {
             // phased evaluation: (A) top-NR per sample, (B) one task per (sample, reduced index): the nm-term kernel row sum -- 97 % of the
             // exponentials, spread over all threads instead of one thread per sample --, (C) the (nr+1) KKT solve and the cost per sample
@@ -661,11 +666,11 @@ __global__ void __launch_bounds__(risko_threads(NR), (NR <= 5) ? 7 : 1) k_inner_
 #pragma unroll 1
             for (int task = tid; task < (S - s0) * NR; task += nt) {
                 const int s = s0 + task / NR, i = task % NR;
-                rs[s * NR + i] = beta_rowsum(D, nm, idxs[s * NR + i], th[s * d + nm]);
+                rs[s * NR + i] = beta_rowsum<KER>(D, nm, idxs[s * NR + i], th[s * d + nm]);
             }
             __syncthreads();
 #pragma unroll 1
-            for (int s = s0 + tid; s < S; s += nt) cost[s] = beta_finish<NR>(c, idxs + s * NR, th[s * d + nm], rs + s * NR, D, betas + s * NR);
+            for (int s = s0 + tid; s < S; s += nt) cost[s] = beta_finish<NR, KER>(c, idxs + s * NR, th[s * d + nm], rs + s * NR, D, betas + s * NR);
         }
         __syncthreads();
 #pragma unroll 1
@@ -892,7 +897,7 @@ __global__ void __launch_bounds__(risko_threads(NR), (NR <= 5) ? 7 : 1) k_inner_
         }
         const float sigma = small[48];
         a.sigma[g] = sigma;
-        a.risk[g] = mmd_cost(c, beta, cs, sigma);
-        a.lane[g] = mmd_cost(c, beta, lbv, sigma) + mmd_cost(c, beta, ubv, sigma);
+        a.risk[g] = mmd_cost<KER>(c, beta, cs, sigma);
+        a.lane[g] = mmd_cost<KER>(c, beta, lbv, sigma) + mmd_cost<KER>(c, beta, ubv, sigma);
     }
 }

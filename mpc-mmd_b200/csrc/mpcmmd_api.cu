@@ -214,46 +214,58 @@ static SplitKernels split_kernels(int nr) {
 static size_t split_eval_smem(const DCfg& d) { const int dd = d.nm + 1; return (size_t)(al4(d.nm * d.nm) + (dd + 1) * al4(dd)) * sizeof(float); }
 static size_t split_update_smem(const DCfg& d) { return (size_t)ICU_WARPS * upd_layout(d.nr).total * sizeof(float); }
 static int g_chol = 0;       // MPCMMD_CHOL=panel|la|cta (read at create): Cholesky build of the specialised throughput kernel (0 one-warp panels, 1 two-warp look-ahead, 2 CTA-wide panels)
-static inner_cem_fn inner_cem_kernel(const DCfg& d, int kind) {
-    if (kind == INNER_WARP) switch (d.nr) {
-        case 2: return k_inner_cem_warp<2>; case 3: return k_inner_cem_warp<3>; case 4: return k_inner_cem_warp<4>; case 5: return k_inner_cem_warp<5>;
-    }
+// KER = MMD kernel form (dm::KER_*).  The experimental warp-per-chain kernel and the Cholesky variants exist for Laplace only (a Gaussian handle refuses them at create)
+template <int KER>
+static inner_cem_fn inner_cem_kernel_k(const DCfg& d, int kind) {
+    if constexpr (KER == dm::KER_LAPLACE) {
+        if (kind == INNER_WARP) switch (d.nr) {
+            case 2: return k_inner_cem_warp<2>; case 3: return k_inner_cem_warp<3>; case 4: return k_inner_cem_warp<4>; case 5: return k_inner_cem_warp<5>;
+        }
+        if (d.nr == 5 && d.S_in == 100 && d.n_el_in == 11) {
+            if (kind == INNER_CTA && g_chol == 1) return k_inner_cem_fast<5, false, false, 100, 11, 1>;
+            if (kind == INNER_CTA && g_chol == 2) return k_inner_cem_fast<5, false, false, 100, 11, 2>;
+        }
+    } else if (kind == INNER_WARP) return nullptr;
     if (d.nr == 5 && d.S_in == 100 && d.n_el_in == 11) {          // the reference's sizes as compile-time constants
-        if (kind == INNER_CTA && g_chol == 1) return k_inner_cem_fast<5, false, false, 100, 11, 1>;
-        if (kind == INNER_CTA && g_chol == 2) return k_inner_cem_fast<5, false, false, 100, 11, 2>;
-        if (kind == INNER_CTA) return k_inner_cem_fast<5, false, false, 100, 11>;
-        if (kind == INNER_CTA_LAT) return k_inner_cem_fast<5, true, false, 100, 11>;
-        if (kind == INNER_CTA_FASTMATH) return k_inner_cem_fast<5, false, true, 100, 11>;
-        if (kind == INNER_LAT512) return k_inner_cem_lat<5, 100, 11>;
+        if (kind == INNER_CTA) return k_inner_cem_fast<5, false, false, 100, 11, 0, KER>;
+        if (kind == INNER_CTA_LAT) return k_inner_cem_fast<5, true, false, 100, 11, 0, KER>;
+        if (kind == INNER_CTA_FASTMATH) return k_inner_cem_fast<5, false, true, 100, 11, 0, KER>;
+        if (kind == INNER_LAT512) return k_inner_cem_lat<5, 100, 11, KER>;
     }
     if (kind == INNER_CTA) switch (d.nr) {
-        case 2: return k_inner_cem_fast<2, false>; case 3: return k_inner_cem_fast<3, false>; case 4: return k_inner_cem_fast<4, false>; case 5: return k_inner_cem_fast<5, false>;
+        case 2: return k_inner_cem_fast<2, false, false, 0, 0, 0, KER>; case 3: return k_inner_cem_fast<3, false, false, 0, 0, 0, KER>;
+        case 4: return k_inner_cem_fast<4, false, false, 0, 0, 0, KER>; case 5: return k_inner_cem_fast<5, false, false, 0, 0, 0, KER>;
     }
     if (kind == INNER_LAT512) switch (d.nr) {
-        case 2: return k_inner_cem_lat<2>; case 3: return k_inner_cem_lat<3>; case 4: return k_inner_cem_lat<4>; case 5: return k_inner_cem_lat<5>;
+        case 2: return k_inner_cem_lat<2, 0, 0, KER>; case 3: return k_inner_cem_lat<3, 0, 0, KER>; case 4: return k_inner_cem_lat<4, 0, 0, KER>; case 5: return k_inner_cem_lat<5, 0, 0, KER>;
     }
     if (kind == INNER_CTA_FASTMATH) switch (d.nr) {
-        case 2: return k_inner_cem_fast<2, false, true>; case 3: return k_inner_cem_fast<3, false, true>; case 4: return k_inner_cem_fast<4, false, true>; case 5: return k_inner_cem_fast<5, false, true>;
+        case 2: return k_inner_cem_fast<2, false, true, 0, 0, 0, KER>; case 3: return k_inner_cem_fast<3, false, true, 0, 0, 0, KER>;
+        case 4: return k_inner_cem_fast<4, false, true, 0, 0, 0, KER>; case 5: return k_inner_cem_fast<5, false, true, 0, 0, 0, KER>;
     }
     if (kind == INNER_CTA_LAT) switch (d.nr) {
-        case 2: return k_inner_cem_fast<2, true>; case 3: return k_inner_cem_fast<3, true>; case 4: return k_inner_cem_fast<4, true>; case 5: return k_inner_cem_fast<5, true>;
+        case 2: return k_inner_cem_fast<2, true, false, 0, 0, 0, KER>; case 3: return k_inner_cem_fast<3, true, false, 0, 0, 0, KER>;
+        case 4: return k_inner_cem_fast<4, true, false, 0, 0, 0, KER>; case 5: return k_inner_cem_fast<5, true, false, 0, 0, 0, KER>;
     }
     if (d.S_in == 100 && d.n_el_in == 11) switch (d.nr) {       // the reference's sizes as compile-time constants (generic kernel, num_reduced 6..10)
-        case 6: return k_inner_cem<6, 100, 11>; case 7: return k_inner_cem<7, 100, 11>; case 8: return k_inner_cem<8, 100, 11>;
-        case 9: return k_inner_cem<9, 100, 11>; case 10: return k_inner_cem<10, 100, 11>;
+        case 6: return k_inner_cem<6, 100, 11, KER>; case 7: return k_inner_cem<7, 100, 11, KER>; case 8: return k_inner_cem<8, 100, 11, KER>;
+        case 9: return k_inner_cem<9, 100, 11, KER>; case 10: return k_inner_cem<10, 100, 11, KER>;
     }
     switch (d.nr) {
-        case 2: return k_inner_cem<2>;
-        case 3: return k_inner_cem<3>;
-        case 4: return k_inner_cem<4>;
-        case 5: return k_inner_cem<5>;
-        case 6: return k_inner_cem<6>;
-        case 7: return k_inner_cem<7>;
-        case 8: return k_inner_cem<8>;
-        case 9: return k_inner_cem<9>;
-        case 10: return k_inner_cem<10>;
+        case 2: return k_inner_cem<2, 0, 0, KER>;
+        case 3: return k_inner_cem<3, 0, 0, KER>;
+        case 4: return k_inner_cem<4, 0, 0, KER>;
+        case 5: return k_inner_cem<5, 0, 0, KER>;
+        case 6: return k_inner_cem<6, 0, 0, KER>;
+        case 7: return k_inner_cem<7, 0, 0, KER>;
+        case 8: return k_inner_cem<8, 0, 0, KER>;
+        case 9: return k_inner_cem<9, 0, 0, KER>;
+        case 10: return k_inner_cem<10, 0, 0, KER>;
         default: return nullptr;
     }
+}
+static inner_cem_fn inner_cem_kernel(const DCfg& d, int kind) {
+    return d.kernel == dm::KER_GAUSSIAN ? inner_cem_kernel_k<dm::KER_GAUSSIAN>(d, kind) : inner_cem_kernel_k<dm::KER_LAPLACE>(d, kind);
 }
 static size_t inner_cem_smem_kind(const DCfg& d, int kind) {
     if (kind == INNER_WARP) return (size_t)warp_layout(d.nr, d.S_in, d.n_el_in).total * sizeof(float);
@@ -264,7 +276,18 @@ static size_t inner_cem_smem_kind(const DCfg& d, int kind) {
 
 static int create_body(mpcmmd_handle_s* h, const mpcmmd_config* cfg, int device);
 extern "C" int mpcmmd_create(const mpcmmd_config* cfg, int device, mpcmmd_handle* out) {
+    return mpcmmd_create_with_kernel(cfg, MPCMMD_KERNEL_LAPLACE, device, out);
+}
+extern "C" int mpcmmd_create_with_kernel(const mpcmmd_config* cfg, int mmd_kernel, int device, mpcmmd_handle* out) {
     if (!cfg || !out) return fail("mpcmmd_create: null argument");
+    if (mmd_kernel != MPCMMD_KERNEL_LAPLACE && mmd_kernel != MPCMMD_KERNEL_GAUSSIAN) return fail("mpcmmd_create: mmd_kernel must be 0 (laplace) or 1 (gaussian)");
+    if (mmd_kernel == MPCMMD_KERNEL_GAUSSIAN) {
+        const char* mode = getenv("MPCMMD_INNER_CEM"); const char* cl = getenv("MPCMMD_CHOL");
+        if (mode && (!strcmp(mode, "warp") || !strcmp(mode, "pipe") || !strcmp(mode, "split")))
+            return fail("mpcmmd_create: the Gaussian MMD kernel has no MPCMMD_INNER_CEM=warp|pipe|split build (experimental inner-CEM kernels are Laplace only)");
+        if (cl && (!strcmp(cl, "la") || !strcmp(cl, "cta")))
+            return fail("mpcmmd_create: the Gaussian MMD kernel has no MPCMMD_CHOL=la|cta build (experimental inner-CEM kernels are Laplace only)");
+    }
     int ndev = 0;
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) return fail("mpcmmd_create: no CUDA device (this library has no CPU fallback)");
     if (device < 0 || device >= ndev) return fail("mpcmmd_create: bad device index");
@@ -284,7 +307,7 @@ extern "C" int mpcmmd_create(const mpcmmd_config* cfg, int device, mpcmmd_handle
     if (cfg->noise_kind != 0 && cfg->noise_kind != 1) return fail("mpcmmd_create: noise_kind must be 0 (gaussian) or 1 (beta)");
     if (B < 1 || B > (1 << 20)) return fail("mpcmmd_create: num_batch must be in [1, 2^20]");
     mpcmmd_handle_s* h = new mpcmmd_handle_s();
-    h->device = device; h->cfg = *cfg; h->E = E;
+    h->device = device; h->cfg = *cfg; h->E = E; h->d.kernel = mmd_kernel;
     if (create_body(h, cfg, device)) { mpcmmd_destroy(h); return -1; }      // one cleanup path: every failure after the allocation frees the handle and its device memory
     *out = h;
     return 0;
@@ -578,8 +601,9 @@ static int launch_risk(mpcmmd_handle_s* h, const RiskArgs& r, cudaStream_t s, in
         int nl = 1;
         for (int g0 = 0; g0 < r.n_samples; g0 += h->big_chunk) {       // chain ranges share the scratch: launches on one stream run in order
             const int nc = r.n_samples - g0 < h->big_chunk ? r.n_samples - g0 : h->big_chunk;
-            if (r.n_samples <= h->sm_count) k_inner_cem_big<BIG_THREADS><<<nc, BIG_THREADS, 0, s>>>(d, ra, h->big_state, g0, nc);
-            else k_inner_cem_big<BIG_THREADS_SMALL><<<nc, BIG_THREADS_SMALL, 0, s>>>(d, ra, h->big_state, g0, nc);
+            const bool gauss = d.kernel == dm::KER_GAUSSIAN;
+            if (r.n_samples <= h->sm_count) (gauss ? k_inner_cem_big<BIG_THREADS, dm::KER_GAUSSIAN> : k_inner_cem_big<BIG_THREADS>)<<<nc, BIG_THREADS, 0, s>>>(d, ra, h->big_state, g0, nc);
+            else (gauss ? k_inner_cem_big<BIG_THREADS_SMALL, dm::KER_GAUSSIAN> : k_inner_cem_big<BIG_THREADS_SMALL>)<<<nc, BIG_THREADS_SMALL, 0, s>>>(d, ra, h->big_state, g0, nc);
             nl++;
         }
         if (n_launch) *n_launch = nl;

@@ -14,6 +14,7 @@ UP = C.POINTER(C.c_uint32)
 
 COST_KINDS = {"mmd_opt": 0, "mmd_random": 1, "cvar": 2, "saa": 3}
 NOISE_KINDS = {"gaussian": 0, "beta": 1}
+MMD_KERNELS = {"laplace": 0, "gaussian": 1}      # MPCMMD_KERNEL_*
 
 
 class MpcmmdConfig(C.Structure):
@@ -32,7 +33,7 @@ class MpcmmdOut(C.Structure):
     _fields_ = [(n, C.c_void_p) for n in ("cx", "cy", "cost_lane", "cost_obs", "beta", "sigma", "res_beta")]
 
 
-EXPORTS = ("mpcmmd_last_error", "mpcmmd_version", "mpcmmd_create", "mpcmmd_destroy", "mpcmmd_solve", "mpcmmd_solve_host",
+EXPORTS = ("mpcmmd_last_error", "mpcmmd_version", "mpcmmd_create", "mpcmmd_create_with_kernel", "mpcmmd_destroy", "mpcmmd_solve", "mpcmmd_solve_host",
            "mpcmmd_last_launch_count", "mpcmmd_inner_cem_path", "mpcmmd_profile_solve", "mpcmmd_fp32_peak", "mpcmmd_xu_peaks", "mpcmmd_selfcheck_ieee", "mpcmmd_math_vec", "mpcmmd_rng_normal", "mpcmmd_rng_beta", "mpcmmd_get_tables",
            "mpcmmd_stage_project", "mpcmmd_stage_risk", "mpcmmd_stage_risk_injected", "mpcmmd_stage_init", "mpcmmd_stage_select", "mpcmmd_stage_noise", "mpcmmd_validate_host",
            "mpcmmd_validate_seeded_host", "mpcmmd_validate_threefry_host")
@@ -56,6 +57,7 @@ def load():
     lib.mpcmmd_last_error.restype = C.c_char_p
     V = C.c_void_p
     lib.mpcmmd_create.argtypes = [C.POINTER(MpcmmdConfig), C.c_int, C.POINTER(V)]
+    lib.mpcmmd_create_with_kernel.argtypes = [C.POINTER(MpcmmdConfig), C.c_int, C.c_int, C.POINTER(V)]
     lib.mpcmmd_destroy.argtypes = [V]
     lib.mpcmmd_solve.argtypes = [V, C.c_int, C.c_int] + [V] * 7 + [C.POINTER(MpcmmdOut), V]
     lib.mpcmmd_solve_host.argtypes = [V, C.c_int, C.c_int] + [V] * 7 + [C.POINTER(MpcmmdOut)]

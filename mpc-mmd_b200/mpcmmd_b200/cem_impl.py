@@ -42,11 +42,16 @@ class CEM:
     """`CEM(num_reduced, num_obs, noise_level, num_prime, noise, acc_const_noise, steer_const_noise)`
     (cem.py:17-18).  Keyword-only extras: `variant` ("static" | "dynamic": which of the reference's two
     optimizer/ copies to mirror), `max_episodes` (workspace capacity of `solve_batch`), `device`,
-    `num_batch` / `maxiter_cem` overrides for scaled or reduced runs."""
+    `num_batch` / `maxiter_cem` overrides for scaled or reduced runs, `kernel` ("laplace" as the reference, or
+    "gaussian"): the kernel of the MMD risk costs of mmd_opt and mmd_random, fixed for the object's lifetime
+    (DESIGN.md section 3 items 4 and 8)."""
 
     def __init__(self, num_reduced, num_obs, noise_level, num_prime, noise, acc_const_noise, steer_const_noise, *,
                  variant="static", max_episodes=1, device=0, num_batch=100, maxiter_cem=20,
-                 num_samples_cem=100, maxiter_beta_cem=20):
+                 num_samples_cem=100, maxiter_beta_cem=20, kernel="laplace"):
+        if kernel not in B.MMD_KERNELS:
+            raise ValueError(f"kernel must be one of {sorted(B.MMD_KERNELS)}, got {kernel!r}")
+        self.kernel = kernel
         if noise not in B.NOISE_KINDS:
             noise_kind = B.NOISE_KINDS["beta"]               # reference: anything but "gaussian" takes the beta branch (cem_helper.py:405,416)
         else:
@@ -116,7 +121,7 @@ class CEM:
         self._cfg = cfg
         self._lib = B.load()
         self._h = C.c_void_p()
-        B.check(self._lib.mpcmmd_create(C.byref(cfg), int(device), C.byref(self._h)))
+        B.check(self._lib.mpcmmd_create_with_kernel(C.byref(cfg), B.MMD_KERNELS[kernel], int(device), C.byref(self._h)))
 
     def __del__(self):
         h = getattr(self, "_h", None)

@@ -13,6 +13,9 @@ What differs from the reference: the 200 episodes of a sweep point are solved in
 independent: every input depends only on (k, num_obs)), optionally sharded over ranks (`episodes k = rank, rank+W, ...`;
 the per-episode records are gathered and written by rank 0 in episode order, SURVEY.md section 8e).
 
+`--kernel gaussian` (default `laplace`, the reference's) plans mmd_opt / mmd_random with the Gaussian-kernel MMD; their files then
+also hold `kernel="gaussian"`.  The cvar / saa files do not depend on the kernel and are written as always.
+
     python -m mpcmmd_b200.driver --costs mmd_opt cvar --noises beta --noise_levels 0.3 --num_reduced_sets 5 \\
         --num_obs 4 --num_prime 50 --acc_const_noise 0.0 --steer_const_noise 0.0 [--num_configs 200] [--root ./data]
 """
@@ -84,6 +87,11 @@ def assemble(records, num_obs, threshold_obs, variant="static"):
     return out
 
 
+def kernel_tag(kernel, cost):
+    """extra arrays of a data file: an MMD plan made with a non-reference kernel says so"""
+    return dict(kernel=kernel) if kernel != "laplace" and cost in ("mmd_opt", "mmd_random") else {}
+
+
 def data_path(root, noise, noise_level, num_prime, cost, num_reduced, num_obs):
     return os.path.join(root, "{}_noise".format(noise), "noise_{}".format(int(noise_level * 100)), "ts_{}".format(num_prime),
                         "{}_{}_samples_{}_obs".format(cost, num_reduced, num_obs))
@@ -92,6 +100,7 @@ def data_path(root, noise, noise_level, num_prime, cost, num_reduced, num_obs):
 def run_sweep(args, rank=0, world=1, gather=None, device=0, log=print):
     """`gather(records) -> all records on rank 0` is the only cross-rank exchange (torch.distributed all_gather in __main__)."""
     written = []
+    kernel = getattr(args, "kernel", "laplace")
     for noise in args.noises:
         for noise_level in args.noise_levels:
             for num_prime in args.num_prime:
@@ -99,7 +108,7 @@ def run_sweep(args, rank=0, world=1, gather=None, device=0, log=print):
                     for num_reduced in args.num_reduced_sets:
                         mine = shard(args.num_configs, rank, world)
                         prob = CEM(num_reduced, num_obs, noise_level, num_prime, noise, args.acc_const_noise, args.steer_const_noise,
-                                   variant=args.variant, max_episodes=max(len(mine), 1), device=device)
+                                   variant=args.variant, max_episodes=max(len(mine), 1), device=device, kernel=kernel)
                         batch = scenes.static_batch(prob, mine, args.variant)
                         for cost in args.costs:
                             _, threshold_obs = thresholds(prob, cost)
@@ -110,6 +119,7 @@ def run_sweep(args, rank=0, world=1, gather=None, device=0, log=print):
                                 rec = gather(rec)
                             if rank == 0:
                                 arrays = assemble(rec, num_obs, threshold_obs, args.variant)
+                                arrays.update(kernel_tag(kernel, cost))
                                 path = data_path(args.root, noise, noise_level, num_prime, cost, num_reduced, num_obs)
                                 os.makedirs(os.path.dirname(path), exist_ok=True)
                                 np.savez(path, **arrays)
@@ -146,6 +156,8 @@ def build_parser():
     p.add_argument("--num_configs", type=int, default=200, help="episodes per sweep point (main_mpc.py:76)")
     p.add_argument("--root", type=str, default="./data")
     p.add_argument("--variant", type=str, default="static", choices=["static", "dynamic"])
+    p.add_argument("--kernel", type=str, default="laplace", choices=["laplace", "gaussian"],
+                   help="kernel of the mmd_opt / mmd_random risk cost (default: laplace, the reference's)")
     return p
 
 

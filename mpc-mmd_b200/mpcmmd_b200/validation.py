@@ -15,7 +15,7 @@ different random numbers: its counts estimate what the reference's estimate, for
 Same command line as the reference, same input files (`./data/{noise}_noise/noise_{L}/ts_{np}/{cost}_{nr}_samples_{O}_obs.npz`), same output
 (`./stats/{noise}_noise/noise_{L}/ts_{np}/{nr}_samples_{O}_obs.npz` with coll_cvar, coll_cvar_lane, coll_mmd_opt, coll_mmd_opt_lane,
 coll_mmd_random, coll_mmd_random_lane; with `--rng jax` or a non-default `--num_rollouts` also rng and num_rollouts, so those counts are
-not taken for the reference's).  Trajectory pairs are enumerated exactly like the reference does -- `set(cvar rows) & set(mmd_opt rows)`
+not taken for the reference's; when the mmd_opt plans carry `kernel` (driver `--kernel gaussian`), so does the stats file).  Trajectory pairs are enumerated exactly like the reference does -- `set(cvar rows) & set(mmd_opt rows)`
 in Python set-iteration order, position k in that order is the RNG seed of the pair (SURVEY.md Q21) -- so the per-pair draws are the same.
 """
 from __future__ import annotations
@@ -278,6 +278,8 @@ def run_validation(args, variant="static", device=0, log=print):
                         os.makedirs(os.path.dirname(path), exist_ok=True)
                         # counts that are not the reference's estimator (other noise or other rollout count) say so in the file
                         tag = dict(rng=args.rng, num_rollouts=args.num_rollouts) if args.rng == "jax" or args.num_rollouts != NUM_ROLLOUTS else {}
+                        if "kernel" in data_mmd_opt.files:                                        # plans made with a non-reference MMD kernel
+                            tag["kernel"] = str(data_mmd_opt["kernel"])
                         np.savez(path, coll_cvar=f(count[m:]), coll_cvar_lane=f(lane[m:]), coll_mmd_opt=f(count[:m]), coll_mmd_opt_lane=f(lane[:m]),
                                  coll_mmd_random=[], coll_mmd_random_lane=[], **tag)
                         written.append(path + ".npz")
