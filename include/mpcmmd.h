@@ -93,8 +93,8 @@ int mpcmmd_version(void);
  * 1e-4 stage parity) for throughput-sized / all launches; unset = the bit-exact FP32 kernel.  See INTEGRATION.md. */
 int mpcmmd_create(const mpcmmd_config *cfg, int device, mpcmmd_handle *out);
 /* mpcmmd_create with the MMD kernel chosen (MPCMMD_KERNEL_*; mpcmmd_create = MPCMMD_KERNEL_LAPLACE).  The kernel is fixed for the handle's
- * lifetime: every solve and stage entry point of the handle uses it.  Unknown kinds are refused.  A Gaussian handle is refused when
- * MPCMMD_INNER_CEM = warp | pipe | split or MPCMMD_CHOL = la | cta select an experimental inner-CEM kernel: those exist for Laplace only. */
+ * lifetime: every solve and stage entry point of the handle uses it.  Unknown kinds are refused.  Both create functions refuse an
+ * MPCMMD_INNER_CEM value other than auto | cta | lat | lat512 | generic (see INTEGRATION.md). */
 int mpcmmd_create_with_kernel(const mpcmmd_config *cfg, int mmd_kernel, int device, mpcmmd_handle *out);
 int mpcmmd_destroy(mpcmmd_handle h);
 

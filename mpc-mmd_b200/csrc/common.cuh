@@ -27,7 +27,7 @@ struct DCfg {
     const float* proj_const;                                 // P | Pd | Pdd | Gx | Gy | Kx | Ky as ONE 16-byte-aligned block (bulk-copied into shared memory by k_project)
     const float* proj_tc_const;                              // tf32 (hi, lo) images of P / Pd / Pdd + Gx | Gy | Kx | Ky for k_project_tc
     const float *z_init, *theta0, *zb_iter;                  // constant normal tables (generated at create)
-    const float *theta0T;                                    // theta0 transposed to [column][row]
+    const float *unused_slot;                                // read by no kernel (null); keeps zb_iterT, and with it every kernel's parameter loads, where they were
     const float *zb_iterT;                                   // zb_iter transposed to [iter][column][row] for coalesced row-per-thread reads
 };
 

@@ -371,38 +371,6 @@ __device__ __forceinline__ void icf_select(int lane, int S, int n_old, int ne, c
     if (lane < ne) { perm[lane] = mine; ecost_n[lane] = won; }
 }
 
-// Cholesky of the d x d covariance by ONE warp, right-looking, in place: lane i owns row i of the lower triangle; step j turns column j
-// into row j of LT (LT[j][q] = L[q][j] for q >= j, zeros for q < j) and subtracts l_ij * LT[j][q] from A[i][q], j < q <= i.  Entry (i,q)
-// therefore accumulates fma(-L_ik, L_qk, .) for k ascending: the contract's order.  Rolled on purpose (instruction cache).
-template <int d>
-__device__ __forceinline__ void icf_chol(float* __restrict__ C, int ldc, int lane) {
-    float* LT = C;
-    float* rowp = C + (lane < d ? lane : d - 1) * ldc;
-#pragma unroll 1
-    for (int j = 0; j < d; j++) {
-        const float aj = rowp[j];
-        const float ajj = __shfl_sync(FULL, aj, j);
-        const float dd = sqrtf(ajj);
-        const float rdj = 1.0f / dd;
-        const float lij = lane == j ? dd : aj * rdj;
-        if (lane < d) LT[j * ldc + lane] = lane < j ? 0.0f : lij;
-        __syncwarp();
-        if (lane > j && lane < d) {
-            const pk::f2 nl = pk::dup(-lij);
-            const float* lrow = LT + j * ldc;
-#pragma unroll 1
-            for (int g4 = (j + 1) >> 2; g4 <= (lane >> 2); g4++) {
-                const float4 l = *reinterpret_cast<const float4*>(lrow + 4 * g4);
-                float4 v = *reinterpret_cast<float4*>(rowp + 4 * g4);
-                pk::unpack(pk::fma2(nl, pk::pack(l.x, l.y), pk::pack(v.x, v.y)), v.x, v.y);
-                pk::unpack(pk::fma2(nl, pk::pack(l.z, l.w), pk::pack(v.z, v.w)), v.z, v.w);
-                *reinterpret_cast<float4*>(rowp + 4 * g4) = v;
-            }
-        }
-    }
-    __syncwarp();
-}
-
 // Cholesky of the d x d covariance by ONE warp, left-looking by PANELS of four columns: lane r owns row r.  For panel j0 = 4p each lane first
 // accumulates its four entries (r, j0..j0+3) over the finished columns k < j0 -- four independent fma chains per lane, two FFMA2, that share one load
 // of L[r][k] and the broadcast L[j0..j0+3][k] (the factor is kept TRANSPOSED: LT[k][q] = L[q][k], so both are conflict-free) -- then the
@@ -411,7 +379,7 @@ __device__ __forceinline__ void icf_chol(float* __restrict__ C, int ldc, int lan
 // panel factors only the columns that exist (d = 26: two).  Entry (r, j) accumulates fma(-L_rk, L_jk, .) for k = 0 .. j-1 ascending, then
 // the pivot's square root / reciprocal scaling: the contract's order, bit for bit the same as the column-by-column versions.  In place: LT lives in
 // the upper triangle (and diagonal) of C while the untouched part of C's lower triangle still holds the covariance.  The resampling loops read
-// whole float4 groups from the diagonal's group on (icf_mvn_row_unrolled, icu_row_elem), so the only zero fill they need is the strict lower
+// whole float4 groups from the diagonal's group on (icf_mvn_row_unrolled, icf_mvn_row_regs), so the only zero fill they need is the strict lower
 // triangle of each 4 x 4 diagonal block (LT[k][q] = 0 for 4 (k / 4) <= q < k); the rest of the lower triangle is never read again.
 // One panel of W <= 4 live columns j0 .. j0 + W - 1 (W < 4 only for the last panel of a d that is not a multiple of four).
 template <int d, int W, bool LAST>
@@ -514,83 +482,6 @@ __device__ __forceinline__ void icf_chol_panel(float* __restrict__ C, int ldc_, 
     icf_chol_panel_step<d, d - 4 * (NG - 1), true>(C, rowp, r, lane, NG - 1);
 }
 
-// Cholesky of the d x d covariance by the WHOLE CTA (3 warps), left-looking by panels of four columns, same per-entry operation order as icf_chol_panel (so the
-// same bits): entry (r, j) accumulates fma(-L_rk, L_jk, .) for k ascending, then the pivot's square root / reciprocal scaling.  The one-warp version leaves two of the
-// three warps parked behind a barrier for a third of the kernel's time; here
-//   A. every thread owns ONE entry (row r >= j0, column j0 + u) of the panel and runs its k < j0 chain (2 shared loads + 1 fma per k), result to a scratch S[r][u];
-//   B. warp 0 factors the 4 x 4 diagonal block from S (the serial sqrt -> reciprocal chain, once per CTA) and publishes pivots, reciprocals and the six
-//      sub-diagonal entries in F;
-//   C. every thread finishes its entry with the block's columns, stores it into the transposed factor (LT[k][q] = L[q][k], upper triangle of C) and zeroes the
-//      consumed covariance entry below the diagonal (the zero fill the resampling relies on).
-// Three block barriers per panel.  S (d x 4 floats) and F (16 floats) live in a region that is dead during the factorisation.
-template <int d>
-__device__ __forceinline__ void icf_chol_cta(float* __restrict__ C, float* __restrict__ scratch, int tid) {
-    constexpr int NG = (d + 3) / 4, ldc = (d + 3) & ~3, RPP = ICF_THREADS / 4;       // rows per pass
-    float* S = scratch; float* F = scratch + 4 * ((d + 3) & ~3);
-    const int u = tid & 3, ro = tid >> 2, warp = tid >> 5, lane = tid & 31;
-#pragma unroll 1
-    for (int p = 0; p < NG; p++) {
-        const int j0 = 4 * p;
-        // ---- A: k < j0 part of every panel entry (rows below j0 are final already)
-#pragma unroll 1
-        for (int r = j0 + ro; r < d; r += RPP) {
-            float acc = C[r * ldc + j0 + u];
-            const float* pr = C + r; const float* pj = C + j0 + u;
-#pragma unroll 1
-            for (int k4 = 0; k4 < p; k4++) {
-#pragma unroll
-                for (int q = 0; q < 4; q++) acc = fmaf(-pr[q * ldc], pj[q * ldc], acc);
-                pr += 4 * ldc; pj += 4 * ldc;
-            }
-            S[r * 4 + u] = acc;
-        }
-        __syncthreads();
-        // ---- B: the diagonal block (rows beyond the matrix shadow the last row, as the lanes of icf_chol_panel do; their results are never stored)
-        if (warp == 0) {
-            const float4 b0 = *reinterpret_cast<const float4*>(S + 4 * j0);
-            const float4 b1 = *reinterpret_cast<const float4*>(S + 4 * (j0 + 1 < d ? j0 + 1 : d - 1));
-            const float4 b2 = *reinterpret_cast<const float4*>(S + 4 * (j0 + 2 < d ? j0 + 2 : d - 1));
-            const float4 b3 = *reinterpret_cast<const float4*>(S + 4 * (j0 + 3 < d ? j0 + 3 : d - 1));
-            float d0, r0, d1, r1, d2, r2, d3, r3;
-            dm::sqrt_rcp(b0.x, d0, r0);
-            const float l10 = b1.x * r0, l20 = b2.x * r0, l30 = b3.x * r0;
-            dm::sqrt_rcp(fmaf(-l10, l10, b1.y), d1, r1);
-            const float l21 = fmaf(-l20, l10, b2.y) * r1, l31 = fmaf(-l30, l10, b3.y) * r1;
-            dm::sqrt_rcp(fmaf(-l21, l21, fmaf(-l20, l20, b2.z)), d2, r2);
-            const float l32 = fmaf(-l31, l21, fmaf(-l30, l20, b3.z)) * r2;
-            dm::sqrt_rcp(fmaf(-l32, l32, fmaf(-l31, l31, fmaf(-l30, l30, b3.w))), d3, r3);
-            if (lane == 0) {
-                *reinterpret_cast<float4*>(F) = make_float4(d0, d1, d2, d3);
-                *reinterpret_cast<float4*>(F + 4) = make_float4(r0, r1, r2, r3);
-                *reinterpret_cast<float4*>(F + 8) = make_float4(l10, l20, l30, l21);
-                *reinterpret_cast<float4*>(F + 12) = make_float4(l31, l32, 0.0f, 0.0f);
-            }
-        }
-        __syncthreads();
-        // ---- C: own entry L[r][j0 + u] (on the diagonal the pivot itself), transposed store, zero fill
-        {
-            const float4 dg = *reinterpret_cast<const float4*>(F), rc = *reinterpret_cast<const float4*>(F + 4);
-            const float4 la = *reinterpret_cast<const float4*>(F + 8), lb = *reinterpret_cast<const float4*>(F + 12);
-            const float l10 = la.x, l20 = la.y, l30 = la.z, l21 = la.w, l31 = lb.x, l32 = lb.y;
-            const int col = j0 + u;
-#pragma unroll 1
-            for (int r = j0 + ro; r < d; r += RPP) {
-                const float4 a = *reinterpret_cast<const float4*>(S + 4 * r);
-                const float e0 = a.x * rc.x;
-                const float e1 = fmaf(-e0, l10, a.y) * rc.y;
-                const float e2 = fmaf(-e1, l21, fmaf(-e0, l20, a.z)) * rc.z;
-                const float e3 = fmaf(-e2, l32, fmaf(-e1, l31, fmaf(-e0, l30, a.w))) * rc.w;
-                float val = u == 0 ? e0 : u == 1 ? e1 : u == 2 ? e2 : e3;
-                const float dv = u == 0 ? dg.x : u == 1 ? dg.y : u == 2 ? dg.z : dg.w;
-                if (r == col) val = dv;
-                if (col < d && r >= col) C[col * ldc + r] = val;
-                if (col < d && r > col) C[r * ldc + col] = 0.0f;
-            }
-        }
-        __syncthreads();
-    }
-}
-
 // one covariance task: C[r][4*q4 .. 4*q4+3] = (sum_el xc[el][r] * xc[el][q]) / (ne - 1) (+ 0.05 on the diagonal), el ascending  [compute_beta.py:61]
 __device__ __forceinline__ void icf_cov_task(const float* __restrict__ xc, float* __restrict__ C, int ldc, int ne, int r, int q4) {
     const float nm1 = (float)(ne - 1);
@@ -611,40 +502,8 @@ __device__ __forceinline__ void icf_cov_task(const float* __restrict__ xc, float
 }
 
 // one resampled row: acc[p] = (sum_k L[2p][k] z[k], sum_k L[2p+1][k] z[k]), k ascending  [compute_beta.py:63].  LT[k][q] = 0 for q < k, so a
-// term with k > q adds an exact zero and whole float4 groups can be used; the k loop is rolled in two ranges whose (static) column-group
-// sets skip most of the zero triangle.
-template <int d>
-__device__ __forceinline__ void icf_mvn_row(const float* __restrict__ LT, int ldc, const float* __restrict__ zT, int nrow, int r, pk::f2 (&acc)[2 * ((d + 3) / 4)]) {
-    constexpr int NG = (d + 3) / 4, GH = NG / 2, KH = 4 * GH;      // row k needs columns q >= k only: k >= KH touches groups >= GH
-#pragma unroll
-    for (int p = 0; p < 2 * NG; p++) acc[p] = pk::dup(0.0f);
-    const float* zp = zT + r;
-    float z0 = __ldg(zp), z1 = __ldg(zp + (d > 1 ? nrow : 0));   // the normals are fetched two steps ahead (L2 latency)
-#pragma unroll 1
-    for (int k = 0; k < KH; k++) {
-        const pk::f2 z2 = pk::dup(z0);
-        z0 = z1; z1 = __ldg(zp + (k + 2 < d ? k + 2 : d - 1) * nrow);
-#pragma unroll
-        for (int g4 = 0; g4 < NG; g4++) {
-            const float4 l = *reinterpret_cast<const float4*>(LT + k * ldc + 4 * g4);
-            acc[2 * g4] = pk::fma2(pk::pack(l.x, l.y), z2, acc[2 * g4]);
-            acc[2 * g4 + 1] = pk::fma2(pk::pack(l.z, l.w), z2, acc[2 * g4 + 1]);
-        }
-    }
-#pragma unroll 1
-    for (int k = KH; k < d; k++) {
-        const pk::f2 z2 = pk::dup(z0);
-        z0 = z1; z1 = __ldg(zp + (k + 2 < d ? k + 2 : d - 1) * nrow);
-#pragma unroll
-        for (int g4 = GH; g4 < NG; g4++) {
-            const float4 l = *reinterpret_cast<const float4*>(LT + k * ldc + 4 * g4);
-            acc[2 * g4] = pk::fma2(pk::pack(l.x, l.y), z2, acc[2 * g4]);
-            acc[2 * g4 + 1] = pk::fma2(pk::pack(l.z, l.w), z2, acc[2 * g4 + 1]);
-        }
-    }
-}
-// the same row, fully unrolled over k with the exact triangular group sets: ~40 % fewer executed instructions for ~450 more of code
-// (used by the CTA-per-chain kernel, whose warps run in near lockstep and share the instruction cache)
+// term with k > q adds an exact zero and whole float4 groups can be used.  Fully unrolled over k with the exact triangular group sets: ~40 % fewer
+// executed instructions than a rolled k loop for ~450 more of code (the CTA-per-chain kernel's warps run in near lockstep and share the instruction cache)
 template <int d>
 __device__ __forceinline__ void icf_mvn_row_unrolled(const float* __restrict__ LT, int ldc, const float* __restrict__ zT, int nrow, int r, pk::f2 (&acc)[2 * ((d + 3) / 4)]) {
     constexpr int NG = (d + 3) / 4;
@@ -681,17 +540,14 @@ __device__ __forceinline__ void icf_mvn_row_regs(const float* __restrict__ LT, i
     }
 }
 
-template <int d> __device__ __forceinline__ void icl_chol_lookahead(float* __restrict__ C, float* __restrict__ ps, int warp, int lane);
 template <int d> __device__ __forceinline__ void icl_chol_regs(float* __restrict__ C, int lane);
 // LAT = the build for launches that fit in a single wave of CTAs (one episode = 100 chains): no register cap (156 instead of the 56 registers
 // that let 12 chains share an SM) and the resampling normals prefetched behind the Cholesky (mmd_opt p50 at batch 1: 8.3 -> 7.4 ms)
 // FM = opt-in fast-math build (MPCMMD_MATH=fast): the Laplace-kernel exponentials on MUFU.EX2 instead of the contract's polynomial; tolerance parity only
 // SC / NEC = compile-time copies of the inner CEM's sample / elite counts (0 = read them from the configuration): with the reference's sizes (100 / 11) baked in, the
 // whole shared-memory layout folds into immediate offsets, which takes the address arithmetic the 56-register cap otherwise re-derives in every phase out of the kernel
-// CH = Cholesky of the covariance: 0 one-warp panel factorisation (icf_chol_panel), 1 two-warp look-ahead (icl_chol_lookahead), 2 CTA-wide panels (icf_chol_cta);
-// MPCMMD_CHOL=panel|la|cta selects the build of the specialised throughput kernel
 // KER = MMD kernel form (dm::KER_*): changes only the distance table and the per-bandwidth scale
-template <int NR, bool LAT, bool FM = false, int SC = 0, int NEC = 0, int CH = 0, int KER = dm::KER_LAPLACE>
+template <int NR, bool LAT, bool FM = false, int SC = 0, int NEC = 0, int KER = dm::KER_LAPLACE>
 __global__ void __launch_bounds__(ICF_THREADS, LAT ? 3 : 12) k_inner_cem_fast(DCfg c, RollArgs ra) {
     extern __shared__ __align__(128) float sm[];
     const RiskArgs& a = ra.r;
@@ -805,17 +661,13 @@ __global__ void __launch_bounds__(ICF_THREADS, LAT ? 3 : 12) k_inner_cem_fast(DC
                 for (int k = 0; k < d; k++) zpre[k] = __ldg(zp + k * (S - ne));
             }
         }
-        // -- Cholesky by warp 0, left-looking by panels of four columns, factor transposed in place (icf_chol_panel).  The two-warp look-ahead variant of the
-        //    latency kernel (icl_chol_lookahead, partial sums in the dead row region) was measured here too (-DICF_CHOL_LOOKAHEAD): 155.7 vs 153.6 ms per 200-episode
-        //    solve -- under the 56-register cap it spills, and with 12 chains per SM the phase is bound by issued instructions, not by warp 0's critical path.
+        // -- Cholesky by warp 0, left-looking by panels of four columns, factor transposed in place (icf_chol_panel).  A two-warp look-ahead and a CTA-wide
+        //    panel factorisation were measured here too and lost (DESIGN.md 5.4): under the 56-register cap the look-ahead spills, and with 12 chains per SM
+        //    the phase is bound by issued instructions, not by warp 0's critical path.
         if constexpr (LAT) { if (warp == 0) icl_chol_regs<d>(C, lane); }       // latency build: register-resident right-looking factorisation (see icl_chol_regs)
-        else if constexpr (CH == 1) { if (warp < 2) icl_chol_lookahead<d>(C, xc, warp, lane); }
-        else if constexpr (CH == 2) icf_chol_cta<d>(C, xc, tid);
         else if (warp == 0) icf_chol_panel<d>(C, ldc, lane);
         __syncthreads();
-        // -- resample: one thread per new row, two columns per packed accumulator, k ascending  [compute_beta.py:63-66].
-        //    LT[k][q] = 0 for q < k, so a term with k > q adds an exact zero and whole float4 groups can be used; the k loop is rolled in
-        //    two ranges whose (static) column-group sets skip most of the zero triangle.
+        // -- resample: one thread per new row, two columns per packed accumulator, k ascending  [compute_beta.py:63-66] (icf_mvn_row_unrolled).
         {
             constexpr int NG = (d + 3) / 4;
             const float* zT = c.zb_iterT + (size_t)it * d * nrow;
@@ -1058,105 +910,6 @@ __device__ __forceinline__ float icl_finish(const DCfg& c, int packed, float sig
     return s1 + s2;
 }
 
-// Two-warp panel Cholesky with LOOK-AHEAD (latency kernel only).  Entry (r, j) of panel p accumulates fma(-L_rk, L_jk, .) over k = 0 .. j0-1 ascending; the terms
-// k < j0 - 4 use columns that were final one panel earlier, so warp 1 computes them for panel p + 1 (all rows, partial sums into a double-buffered 26 x 4
-// shared array) while warp 0 gathers, factors and writes panel p.  Warp 0's critical path keeps only the four newest columns of the k loop, the 4 x 4 block chain and
-// the stores.  Same per-entry operation order as icf_chol_panel => same bits.  Named barriers 1/2 (partial sums of an even / odd panel ready: warp 1 arrives,
-// warp 0 waits) and 3/4 (columns of an even / odd panel written: warp 0 arrives, warp 1 waits), 64 participants each; immediates, see k_inner_pipe.cuh.
-template <int ID> __device__ __forceinline__ void icl_bar_sync64() { asm volatile("bar.sync %0, 64;" :: "n"(ID) : "memory"); }
-template <int ID> __device__ __forceinline__ void icl_bar_arrive64() { asm volatile("bar.arrive %0, 64;" :: "n"(ID) : "memory"); }
-template <int d>
-__device__ __forceinline__ void icl_chol_lookahead(float* __restrict__ C, float* __restrict__ ps /* [2][32][4] */, int warp, int lane) {
-    constexpr int NG = (d + 3) / 4, ldc = (d + 3) & ~3;
-    const int r = lane < d ? lane : d - 1;
-    float* rowp = C + r * ldc;
-    if (warp == 1) {
-        // partial sums of panel p (p >= 2) over the columns k < 4 (p - 1): needs panel p - 2 written
-#pragma unroll 1
-        for (int p = 2; p < NG; p++) {
-            if ((p & 1) == 0) icl_bar_sync64<3>(); else icl_bar_sync64<4>();          // panel p - 2 (same parity) is in place
-            const int j0 = 4 * p;
-            const float4 av = *reinterpret_cast<const float4*>(rowp + j0);
-            float a0 = av.x, a1 = av.y, a2 = av.z, a3 = av.w;
-            const float* pr = C + r; const float* pj = C + j0;
-#pragma unroll 1
-            for (int k4 = 0; k4 < p - 1; k4++) {
-#pragma unroll
-                for (int u = 0; u < 4; u++) {
-                    const float lr = pr[u * ldc];
-                    const float4 lj = *reinterpret_cast<const float4*>(pj + u * ldc);
-                    a0 = fmaf(-lr, lj.x, a0); a1 = fmaf(-lr, lj.y, a1); a2 = fmaf(-lr, lj.z, a2); a3 = fmaf(-lr, lj.w, a3);
-                }
-                pr += 4 * ldc; pj += 4 * ldc;
-            }
-            *reinterpret_cast<float4*>(ps + ((p & 1) * 32 + lane) * 4) = make_float4(a0, a1, a2, a3);
-            __threadfence_block();
-            __syncwarp();
-            if ((p & 1) == 0) icl_bar_arrive64<1>(); else icl_bar_arrive64<2>();
-        }
-        return;
-    }
-    // warp 0: the panels
-#pragma unroll 1
-    for (int p = 0; p < NG; p++) {
-        const int j0 = 4 * p;
-        const float4 av = *reinterpret_cast<const float4*>(rowp + j0);          // a(r, j0..j0+3): needed for the zero fill below even when the sums come from warp 1
-        float a0 = av.x, a1 = av.y, a2 = av.z, a3 = av.w;
-        if (p >= 2) {
-            if ((p & 1) == 0) icl_bar_sync64<1>(); else icl_bar_sync64<2>();
-            const float4 pv = *reinterpret_cast<const float4*>(ps + ((p & 1) * 32 + lane) * 4);
-            a0 = pv.x; a1 = pv.y; a2 = pv.z; a3 = pv.w;
-        }
-        if (p >= 1) {                                                             // the four newest columns k = j0 - 4 .. j0 - 1
-            const float* pr = C + (j0 - 4) * ldc + r; const float* pj = C + (j0 - 4) * ldc + j0;
-#pragma unroll
-            for (int u = 0; u < 4; u++) {
-                const float lr = pr[u * ldc];
-                const float4 lj = *reinterpret_cast<const float4*>(pj + u * ldc);
-                a0 = fmaf(-lr, lj.x, a0); a1 = fmaf(-lr, lj.y, a1); a2 = fmaf(-lr, lj.z, a2); a3 = fmaf(-lr, lj.w, a3);
-            }
-        }
-        const float b00 = __shfl_sync(FULL, a0, j0);
-        const float b10 = __shfl_sync(FULL, a0, j0 + 1), b11 = __shfl_sync(FULL, a1, j0 + 1);
-        const float b20 = __shfl_sync(FULL, a0, j0 + 2), b21 = __shfl_sync(FULL, a1, j0 + 2), b22 = __shfl_sync(FULL, a2, j0 + 2);
-        const float b30 = __shfl_sync(FULL, a0, j0 + 3), b31 = __shfl_sync(FULL, a1, j0 + 3), b32 = __shfl_sync(FULL, a2, j0 + 3), b33 = __shfl_sync(FULL, a3, j0 + 3);
-        float d0, r0, d1, r1, d2, r2, d3, r3;
-        dm::sqrt_rcp(b00, d0, r0);
-        const float l10 = b10 * r0, l20 = b20 * r0, l30 = b30 * r0;
-        dm::sqrt_rcp(fmaf(-l10, l10, b11), d1, r1);
-        const float l21 = fmaf(-l20, l10, b21) * r1, l31 = fmaf(-l30, l10, b31) * r1;
-        dm::sqrt_rcp(fmaf(-l21, l21, fmaf(-l20, l20, b22)), d2, r2);
-        const float l32 = fmaf(-l31, l21, fmaf(-l30, l20, b32)) * r2;
-        dm::sqrt_rcp(fmaf(-l32, l32, fmaf(-l31, l31, fmaf(-l30, l30, b33))), d3, r3);
-        float e0 = a0 * r0;
-        a1 = fmaf(-e0, l10, a1); float e1 = a1 * r1;
-        a2 = fmaf(-e1, l21, fmaf(-e0, l20, a2)); float e2 = a2 * r2;
-        a3 = fmaf(-e2, l32, fmaf(-e1, l31, fmaf(-e0, l30, a3))); float e3 = a3 * r3;
-        if (lane == j0) e0 = d0;
-        if (lane == j0 + 1) e1 = d1;
-        if (lane == j0 + 2) e2 = d2;
-        if (lane == j0 + 3) e3 = d3;
-        if (lane < d) {
-            float4 z = av;
-            if (j0 + 0 < lane) z.x = 0.0f;
-            if (j0 + 1 < lane) z.y = 0.0f;
-            if (j0 + 2 < lane) z.z = 0.0f;
-            if (j0 + 3 < lane) z.w = 0.0f;
-            if (lane >= j0) *reinterpret_cast<float4*>(rowp + j0) = z;
-        }
-        __syncwarp();
-        if (lane < d) {
-            if (lane >= j0 + 0) C[(j0 + 0) * ldc + lane] = e0;
-            if (lane >= j0 + 1 && j0 + 1 < d) C[(j0 + 1) * ldc + lane] = e1;
-            if (lane >= j0 + 2 && j0 + 2 < d) C[(j0 + 2) * ldc + lane] = e2;
-            if (lane >= j0 + 3 && j0 + 3 < d) C[(j0 + 3) * ldc + lane] = e3;
-        }
-        __threadfence_block();
-        __syncwarp();
-        if (p + 2 < NG) { if ((p & 1) == 0) icl_bar_arrive64<3>(); else icl_bar_arrive64<4>(); }     // panel p is in place: warp 1 may start the sums of panel p + 2
-    }
-}
-
 // Latency kernel only: Cholesky of the d x d covariance by ONE warp with the whole lower triangle in registers (lane r holds row r), right-looking and fully
 // unrolled: column j takes its pivot from lane j (one shuffle), every lane scales its entry, and the trailing entries (r, q), q > j, receive fma(-L_rj, L_qj, .)
 // with L_qj shuffled from lane q.  Entry (r, q) therefore accumulates its k terms in ascending k and is then scaled by the pivot's reciprocal: the contract's order,
@@ -1302,7 +1055,7 @@ __global__ void __launch_bounds__(ICL_THREADS, 1) k_inner_cem_lat(DCfg c, RollAr
         __syncthreads();
         if (cr >= 0) icf_cov_task(xc, C, ldc, ne, cr, cg);
         __syncthreads();
-        if (warp == 0) icl_chol_regs<d>(C, lane);          // (icl_chol_lookahead, two warps, was the previous version: 3.7 us per factorisation against ~1.7)
+        if (warp == 0) icl_chol_regs<d>(C, lane);          // (a two-warp look-ahead panel factorisation was the previous version: 3.7 us per factorisation against ~1.7)
         else if (warp >= 2) {                             // the other warps fetch the iteration's normals (first touch: L2 latency) behind the Cholesky
             // eight independent loads in flight per thread, then the stores: rolled one at a time, each thread paid the L2 / DRAM latency of a first touch six times in
             // a row (the ncu source page showed this phase waiting on these stores, not on the factorisation)

@@ -169,13 +169,12 @@ struct RollArgs {
     int spb;                 // samples per CTA
     int R;                   // rollouts per sample (nr or nr*nr)
     int stage_ctrl;          // cvar / saa / mmd_random: draw the noisy controls into shared memory with the whole CTA first (latency regime: few samples)
-    int write_rolls;         // mmd_opt: also write the mother rollouts (only the generic / warp-per-chain inner kernels read them back)
+    int write_rolls;         // mmd_opt: also write the mother rollouts (only the generic and large-set inner kernels read them back)
     int fold_risk;           // mmd_opt, small launches: the mother rollouts also fold their obstacle / lane maxima into mrisk, k_opt_risk does not re-roll
     float* mrisk;            // [n][nm][3]
     float *xroll, *yroll;    // [n][R][np]   (mmd_opt, write_rolls only)
     float* feat;             // [n][nm][22]  (mmd_opt only)
     float* ctrl;             // [n][2][nr*np]  noisy acceleration and tan(noisy steering) of the sample (mmd_opt): k_opt_risk re-rolls the chosen reduced set from them
-    float* stash;            // [persistent CTAs][S][32]  row stash of k_inner_cem_warp
     int* ridx;               // [n][nr]  reduced set chosen by k_inner_cem_fast, read by k_opt_risk
     float* bscratch;         // [n][S][nr + 1]  per-row beta vectors and packed reduced-set indices of k_inner_cem_fast's current iteration
 };
@@ -282,7 +281,7 @@ __device__ __forceinline__ void rollout_risk(const DCfg& c, const RiskArgs& A, i
 // MODE 0: mmd_opt; 1: num_reduced-rollout costs, throughput regime; 2: the same, latency regime.  Three instantiations keep each launch's code small.
 enum { ROLL_OPT = 0, ROLL_FLY = 1, ROLL_STAGED = 2 };
 // OV (ROLL_OPT only) = which of the three mmd_opt bodies the launch runs, fixed at compile time so that the throughput kernel does not carry the other two (the
-// combined kernel was 4500 SASS instructions, instruction-fetch stalls 2.5 per issue): 0 features only, 1 also the mother rollouts' positions (generic / warp-per-chain
+// combined kernel was 4500 SASS instructions, instruction-fetch stalls 2.5 per issue): 0 features only, 1 also the mother rollouts' positions (the generic and large-set
 // inner kernels read them back), 2 the latency regime (RollArgs::fold_risk)
 enum { OV_PLAIN = 0, OV_WRITE = 1, OV_FOLD = 2 };
 template <int MODE, bool SORTED = false, int NZ = NZ_ANY, int OV = OV_PLAIN>

@@ -15,9 +15,6 @@
 #include "k_project_tc.cuh"
 #include "k_risk.cuh"
 #include "k_inner_cem.cuh"
-#include "k_inner_cem_warp.cuh"
-#include "k_inner_split.cuh"
-#include "k_inner_pipe.cuh"
 #include "k_inner_big.cuh"
 #include "k_select.cuh"
 #include "k_validate.cuh"
@@ -54,20 +51,15 @@ struct mpcmmd_handle_s {
     DWork w;
     float *beq_x = nullptr, *beq_y = nullptr, *state0 = nullptr;   // [E][3], [E][4], [E][5]
     float *xroll = nullptr, *yroll = nullptr, *feat = nullptr;     // mmd_opt scratch (ensure_opt_scratch)
-    float *rolls_x = nullptr, *rolls_y = nullptr;                  // [E*B][nm][np] mother rollouts (generic / warp-per-chain inner kernels only)
+    float *rolls_x = nullptr, *rolls_y = nullptr;                  // [E*B][nm][np] mother rollouts (generic and large-set inner kernels only)
     int* ridx = nullptr;       // [E*B][nr] reduced sets (k_inner_cem_fast -> k_opt_risk)
     float* bscratch = nullptr; // [E*B][S][nr+1] row records of k_inner_cem_fast
     float* ctrl = nullptr;     // [E*B][2][nr*np] noisy controls (k_rollouts -> k_opt_risk)
     float* mrisk = nullptr;         // [E*B][nm][3] obstacle / lane maxima of the mother rollouts (small mmd_opt launches: RollArgs::fold_risk)
-    float* throws = nullptr;        // [E*B][nm+1][ICP_TH_LD] candidate-elite rows of the pipelined inner CEM (k_inner_pipe.cuh)
-    int pipe_minb = 8;              // CTAs per SM the pipelined kernel is compiled for (MPCMMD_PIPE_MINB=8|9|12)
     float* big_state = nullptr;     // [big_chunk][BigLayout::total] chain blocks of k_inner_cem_big (num_reduced > 10), reused by successive chain ranges
     int big_chunk = 0;
-    float* split_state = nullptr;   // [E*B][SplitLayout::total] chain blocks of the phase-split inner CEM (k_inner_split.cuh)
-    float* stash = nullptr;    // row stash of k_inner_cem_warp, [warp_grid][S][32]
-    int warp_grid = 0;         // persistent CTAs of k_inner_cem_warp (SMs x resident CTAs per SM)
     int sm_count = 148;
-    int inner_mode = 0;        // 0 auto, 1 warp-per-chain, 2 CTA-per-chain, 3 generic, 4 CTA-per-chain latency build, 5 phase-split (MPCMMD_INNER_CEM=auto|warp|cta|generic|lat|split)
+    int inner_mode = 0;        // INNER_AUTO or the inner-CEM kernel MPCMMD_INNER_CEM forces (see parse_inner_mode)
     int E = 0;
     bool fast_math = false;    // MPCMMD_MATH=fast: Laplace-kernel exponentials of the inner CEM on MUFU.EX2 (opt-in, tolerance parity only)
     bool proj_tc = false;      // MPCMMD_PROJ=tc: tensor-core projection kernel (k_project_tc)
@@ -80,14 +72,13 @@ struct mpcmmd_handle_s {
     cudaStream_t aux_stream[MAX_GROUPS - 1] = {};   // further branches of a solve graph whose episodes are split into groups (see solve_groups)
     cudaEvent_t ev_fork = nullptr, ev_join[MAX_GROUPS - 1] = {};
     int groups_override = 0;                 // MPCMMD_GROUPS=1..8: force the number of episode groups of a solve graph (0 = automatic)
-    int prio_mode = 0;                       // MPCMMD_PRIO=0|1|2 (experiment, default off): highest stream priority on the kernel nodes of mmd_opt graphs (1) / of the other cost functions' graphs (2)
 };
 
 // ---- episode-offset view of a handle's workspace: every per-episode array advanced by e0 episodes.  A solve graph can then enqueue disjoint episode
 // ranges on different streams with the unchanged launch code (episodes are independent; sample index g and episode index e stay relative to the view).
-struct ViewSave { DWork w; float *beq_x, *beq_y, *state0, *feat, *ctrl, *bscratch, *throws, *split_state, *rolls_x, *rolls_y, *xroll, *mrisk; int* ridx; };
+struct ViewSave { DWork w; float *beq_x, *beq_y, *state0, *feat, *ctrl, *bscratch, *rolls_x, *rolls_y, *xroll, *mrisk; int* ridx; };
 static ViewSave push_view(mpcmmd_handle_s* h, int e0) {
-    ViewSave sv = {h->w, h->beq_x, h->beq_y, h->state0, h->feat, h->ctrl, h->bscratch, h->throws, h->split_state, h->rolls_x, h->rolls_y, h->xroll, h->mrisk, h->ridx};
+    ViewSave sv = {h->w, h->beq_x, h->beq_y, h->state0, h->feat, h->ctrl, h->bscratch, h->rolls_x, h->rolls_y, h->xroll, h->mrisk, h->ridx};
     if (e0 == 0) return sv;
     const DCfg& d = h->d; DWork& w = h->w;
     const size_t e = (size_t)e0, B = d.B, n = (size_t)d.nr * d.np, ncem = (size_t)(d.B - d.n_el) * NPAR, it = d.iters;
@@ -101,7 +92,6 @@ static ViewSave push_view(mpcmmd_handle_s* h, int e0) {
     ADV(w.o_cx, NV); ADV(w.o_cy, NV); ADV(w.o_lane, 1); ADV(w.o_obs, 1); ADV(w.o_beta, d.nr); ADV(w.o_sigma, 1); ADV(w.o_res_beta, d.iters_in); ADV(w.o_sel, it);
     ADV(h->beq_x, 3); ADV(h->beq_y, 4); ADV(h->state0, 5);
     ADV(h->feat, B * d.nm * 2 * NV); ADV(h->ctrl, B * 2 * n); ADV(h->ridx, B * d.nr); ADV(h->bscratch, B * d.S_in * (d.nr + 1));
-    ADV(h->throws, B * (d.nm + 1) * ICP_TH_LD); ADV(h->split_state, B * (size_t)split_layout(d.nr, d.S_in, d.n_el_in).total);
     ADV(h->rolls_x, B * d.nm * d.np); ADV(h->rolls_y, B * d.nm * d.np); ADV(h->mrisk, B * d.nm * 3);
     if (h->xroll) h->xroll = h->feat;
 #undef ADV
@@ -109,7 +99,7 @@ static ViewSave push_view(mpcmmd_handle_s* h, int e0) {
 }
 static void pop_view(mpcmmd_handle_s* h, const ViewSave& sv) {
     h->w = sv.w; h->beq_x = sv.beq_x; h->beq_y = sv.beq_y; h->state0 = sv.state0; h->feat = sv.feat; h->ctrl = sv.ctrl; h->bscratch = sv.bscratch;
-    h->throws = sv.throws; h->split_state = sv.split_state; h->rolls_x = sv.rolls_x; h->rolls_y = sv.rolls_y; h->xroll = sv.xroll; h->mrisk = sv.mrisk; h->ridx = sv.ridx;
+    h->rolls_x = sv.rolls_x; h->rolls_y = sv.rolls_y; h->xroll = sv.xroll; h->mrisk = sv.mrisk; h->ridx = sv.ridx;
 }
 
 template <typename Tp>
@@ -188,64 +178,46 @@ static const void* rollouts_kernel(int mode, int nz, int sorted, int ov = OV_PLA
 #undef RK_NZ
 }
 typedef void (*inner_cem_fn)(DCfg, RollArgs);
-enum { INNER_WARP = 1, INNER_CTA = 2, INNER_GENERIC = 3, INNER_CTA_LAT = 4, INNER_SPLIT = 5, INNER_PIPE = 6, INNER_CTA_FASTMATH = 7, INNER_BIG = 8, INNER_LAT512 = 9 };
+// inner-CEM kernels of mmd_opt.  The k_inner_cem_fast family (one CTA per chain, num_reduced <= 5): CTA (throughput build), CTA_LAT (its latency build),
+// CTA_FASTMATH (MPCMMD_MATH=fast) and LAT512 (k_inner_cem_lat, 16 warps per chain); these leave the chosen reduced set to k_opt_risk.  GENERIC (k_inner_cem,
+// num_reduced <= 10) and BIG (k_inner_cem_big, larger sets) evaluate the risk themselves from the stored mother rollouts.
+enum { INNER_AUTO = 0, INNER_CTA, INNER_CTA_LAT, INNER_CTA_FASTMATH, INNER_LAT512, INNER_GENERIC, INNER_BIG };
 #define MPCMMD_BIG_SCRATCH_BYTES ((size_t)8 << 30)      // global chain state of k_inner_cem_big held at a time (num_reduced 40: 23 MB per chain)
-#define INNER_DEFAULT_THROUGHPUT INNER_CTA
-typedef void (*pipe_fn)(DCfg, RollArgs, float*);
-// the pipelined kernel stages the mother features through its row buffer: (S - ne) rows of nm + 1 (odd stride) must hold nm x 22 floats
-static bool pipe_ok(const DCfg& d) { return inner_cem_is_fast(d) && (d.S_in - d.n_el_in) * ((d.nm + 1) | 1) >= d.nm * 2 * NV; }
-static pipe_fn pipe_kernel(int nr, int minb) {
-#define PK(N) (minb >= 12 ? k_inner_cem_pipe<N, 12> : minb == 9 ? k_inner_cem_pipe<N, 9> : k_inner_cem_pipe<N, 8>)
-    switch (nr) { case 2: return PK(2); case 3: return PK(3); case 4: return PK(4); case 5: return PK(5); default: return nullptr; }
-#undef PK
+static bool inner_is_cta_family(int kind) { return kind == INNER_CTA || kind == INNER_CTA_LAT || kind == INNER_CTA_FASTMATH || kind == INNER_LAT512; }
+// MPCMMD_INNER_CEM: test / profiling override of the inner-CEM kernel choice, read once at create.  Unset or "auto": chosen per launch from its size
+// (launch_risk).  Returns -1 for any other value, which create refuses: a misspelt override must not silently measure the default.
+#define INNER_CEM_VALUES "auto, cta, lat, lat512, generic"
+static int parse_inner_mode(const char* v) {
+    if (!v || !strcmp(v, "auto")) return INNER_AUTO;
+    if (!strcmp(v, "cta")) return INNER_CTA;
+    if (!strcmp(v, "lat")) return INNER_CTA_LAT;
+    if (!strcmp(v, "lat512")) return INNER_LAT512;
+    if (!strcmp(v, "generic")) return INNER_GENERIC;
+    return -1;
 }
-typedef void (*split_dist_fn)(DCfg, SplitArgs);
-typedef void (*split_it_fn)(DCfg, SplitArgs, int);
-struct SplitKernels { split_dist_fn dist; split_it_fn eval, update; };
-static SplitKernels split_kernels(int nr) {
-    switch (nr) {
-        case 2: return {k_icem_dist<2>, k_icem_eval<2>, k_icem_update<2>};
-        case 3: return {k_icem_dist<3>, k_icem_eval<3>, k_icem_update<3>};
-        case 4: return {k_icem_dist<4>, k_icem_eval<4>, k_icem_update<4>};
-        case 5: return {k_icem_dist<5>, k_icem_eval<5>, k_icem_update<5>};
-        default: return {nullptr, nullptr, nullptr};
-    }
-}
-static size_t split_eval_smem(const DCfg& d) { const int dd = d.nm + 1; return (size_t)(al4(d.nm * d.nm) + (dd + 1) * al4(dd)) * sizeof(float); }
-static size_t split_update_smem(const DCfg& d) { return (size_t)ICU_WARPS * upd_layout(d.nr).total * sizeof(float); }
-static int g_chol = 0;       // MPCMMD_CHOL=panel|la|cta (read at create): Cholesky build of the specialised throughput kernel (0 one-warp panels, 1 two-warp look-ahead, 2 CTA-wide panels)
-// KER = MMD kernel form (dm::KER_*).  The experimental warp-per-chain kernel and the Cholesky variants exist for Laplace only (a Gaussian handle refuses them at create)
+// KER = MMD kernel form (dm::KER_*)
 template <int KER>
 static inner_cem_fn inner_cem_kernel_k(const DCfg& d, int kind) {
-    if constexpr (KER == dm::KER_LAPLACE) {
-        if (kind == INNER_WARP) switch (d.nr) {
-            case 2: return k_inner_cem_warp<2>; case 3: return k_inner_cem_warp<3>; case 4: return k_inner_cem_warp<4>; case 5: return k_inner_cem_warp<5>;
-        }
-        if (d.nr == 5 && d.S_in == 100 && d.n_el_in == 11) {
-            if (kind == INNER_CTA && g_chol == 1) return k_inner_cem_fast<5, false, false, 100, 11, 1>;
-            if (kind == INNER_CTA && g_chol == 2) return k_inner_cem_fast<5, false, false, 100, 11, 2>;
-        }
-    } else if (kind == INNER_WARP) return nullptr;
     if (d.nr == 5 && d.S_in == 100 && d.n_el_in == 11) {          // the reference's sizes as compile-time constants
-        if (kind == INNER_CTA) return k_inner_cem_fast<5, false, false, 100, 11, 0, KER>;
-        if (kind == INNER_CTA_LAT) return k_inner_cem_fast<5, true, false, 100, 11, 0, KER>;
-        if (kind == INNER_CTA_FASTMATH) return k_inner_cem_fast<5, false, true, 100, 11, 0, KER>;
+        if (kind == INNER_CTA) return k_inner_cem_fast<5, false, false, 100, 11, KER>;
+        if (kind == INNER_CTA_LAT) return k_inner_cem_fast<5, true, false, 100, 11, KER>;
+        if (kind == INNER_CTA_FASTMATH) return k_inner_cem_fast<5, false, true, 100, 11, KER>;
         if (kind == INNER_LAT512) return k_inner_cem_lat<5, 100, 11, KER>;
     }
     if (kind == INNER_CTA) switch (d.nr) {
-        case 2: return k_inner_cem_fast<2, false, false, 0, 0, 0, KER>; case 3: return k_inner_cem_fast<3, false, false, 0, 0, 0, KER>;
-        case 4: return k_inner_cem_fast<4, false, false, 0, 0, 0, KER>; case 5: return k_inner_cem_fast<5, false, false, 0, 0, 0, KER>;
+        case 2: return k_inner_cem_fast<2, false, false, 0, 0, KER>; case 3: return k_inner_cem_fast<3, false, false, 0, 0, KER>;
+        case 4: return k_inner_cem_fast<4, false, false, 0, 0, KER>; case 5: return k_inner_cem_fast<5, false, false, 0, 0, KER>;
     }
     if (kind == INNER_LAT512) switch (d.nr) {
         case 2: return k_inner_cem_lat<2, 0, 0, KER>; case 3: return k_inner_cem_lat<3, 0, 0, KER>; case 4: return k_inner_cem_lat<4, 0, 0, KER>; case 5: return k_inner_cem_lat<5, 0, 0, KER>;
     }
     if (kind == INNER_CTA_FASTMATH) switch (d.nr) {
-        case 2: return k_inner_cem_fast<2, false, true, 0, 0, 0, KER>; case 3: return k_inner_cem_fast<3, false, true, 0, 0, 0, KER>;
-        case 4: return k_inner_cem_fast<4, false, true, 0, 0, 0, KER>; case 5: return k_inner_cem_fast<5, false, true, 0, 0, 0, KER>;
+        case 2: return k_inner_cem_fast<2, false, true, 0, 0, KER>; case 3: return k_inner_cem_fast<3, false, true, 0, 0, KER>;
+        case 4: return k_inner_cem_fast<4, false, true, 0, 0, KER>; case 5: return k_inner_cem_fast<5, false, true, 0, 0, KER>;
     }
     if (kind == INNER_CTA_LAT) switch (d.nr) {
-        case 2: return k_inner_cem_fast<2, true, false, 0, 0, 0, KER>; case 3: return k_inner_cem_fast<3, true, false, 0, 0, 0, KER>;
-        case 4: return k_inner_cem_fast<4, true, false, 0, 0, 0, KER>; case 5: return k_inner_cem_fast<5, true, false, 0, 0, 0, KER>;
+        case 2: return k_inner_cem_fast<2, true, false, 0, 0, KER>; case 3: return k_inner_cem_fast<3, true, false, 0, 0, KER>;
+        case 4: return k_inner_cem_fast<4, true, false, 0, 0, KER>; case 5: return k_inner_cem_fast<5, true, false, 0, 0, KER>;
     }
     if (d.S_in == 100 && d.n_el_in == 11) switch (d.nr) {       // the reference's sizes as compile-time constants (generic kernel, num_reduced 6..10)
         case 6: return k_inner_cem<6, 100, 11, KER>; case 7: return k_inner_cem<7, 100, 11, KER>; case 8: return k_inner_cem<8, 100, 11, KER>;
@@ -268,7 +240,6 @@ static inner_cem_fn inner_cem_kernel(const DCfg& d, int kind) {
     return d.kernel == dm::KER_GAUSSIAN ? inner_cem_kernel_k<dm::KER_GAUSSIAN>(d, kind) : inner_cem_kernel_k<dm::KER_LAPLACE>(d, kind);
 }
 static size_t inner_cem_smem_kind(const DCfg& d, int kind) {
-    if (kind == INNER_WARP) return (size_t)warp_layout(d.nr, d.S_in, d.n_el_in).total * sizeof(float);
     if (kind == INNER_CTA || kind == INNER_CTA_LAT || kind == INNER_CTA_FASTMATH) return (size_t)fast_layout(d.nr, d.S_in, d.n_el_in).total * sizeof(float);
     if (kind == INNER_LAT512) return (size_t)(fast_layout(d.nr, d.S_in, d.n_el_in).total + al4(d.S_in) + al4(d.S_in * d.nr) + al4((d.nm + 1) * (d.S_in - d.n_el_in)) + 256) * sizeof(float);
     return (size_t)opt_layout(d.nr, d.np, d.S_in, d.n_el_in).total * sizeof(float);
@@ -281,13 +252,9 @@ extern "C" int mpcmmd_create(const mpcmmd_config* cfg, int device, mpcmmd_handle
 extern "C" int mpcmmd_create_with_kernel(const mpcmmd_config* cfg, int mmd_kernel, int device, mpcmmd_handle* out) {
     if (!cfg || !out) return fail("mpcmmd_create: null argument");
     if (mmd_kernel != MPCMMD_KERNEL_LAPLACE && mmd_kernel != MPCMMD_KERNEL_GAUSSIAN) return fail("mpcmmd_create: mmd_kernel must be 0 (laplace) or 1 (gaussian)");
-    if (mmd_kernel == MPCMMD_KERNEL_GAUSSIAN) {
-        const char* mode = getenv("MPCMMD_INNER_CEM"); const char* cl = getenv("MPCMMD_CHOL");
-        if (mode && (!strcmp(mode, "warp") || !strcmp(mode, "pipe") || !strcmp(mode, "split")))
-            return fail("mpcmmd_create: the Gaussian MMD kernel has no MPCMMD_INNER_CEM=warp|pipe|split build (experimental inner-CEM kernels are Laplace only)");
-        if (cl && (!strcmp(cl, "la") || !strcmp(cl, "cta")))
-            return fail("mpcmmd_create: the Gaussian MMD kernel has no MPCMMD_CHOL=la|cta build (experimental inner-CEM kernels are Laplace only)");
-    }
+    const char* inner_env = getenv("MPCMMD_INNER_CEM");
+    const int inner_mode = parse_inner_mode(inner_env);
+    if (inner_mode < 0) return fail(std::string("mpcmmd_create: MPCMMD_INNER_CEM=") + inner_env + " is not one of " INNER_CEM_VALUES);
     int ndev = 0;
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) return fail("mpcmmd_create: no CUDA device (this library has no CPU fallback)");
     if (device < 0 || device >= ndev) return fail("mpcmmd_create: bad device index");
@@ -307,7 +274,7 @@ extern "C" int mpcmmd_create_with_kernel(const mpcmmd_config* cfg, int mmd_kerne
     if (cfg->noise_kind != 0 && cfg->noise_kind != 1) return fail("mpcmmd_create: noise_kind must be 0 (gaussian) or 1 (beta)");
     if (B < 1 || B > (1 << 20)) return fail("mpcmmd_create: num_batch must be in [1, 2^20]");
     mpcmmd_handle_s* h = new mpcmmd_handle_s();
-    h->device = device; h->cfg = *cfg; h->E = E; h->d.kernel = mmd_kernel;
+    h->device = device; h->cfg = *cfg; h->E = E; h->d.kernel = mmd_kernel; h->inner_mode = inner_mode;
     if (create_body(h, cfg, device)) { mpcmmd_destroy(h); return -1; }      // one cleanup path: every failure after the allocation frees the handle and its device memory
     *out = h;
     return 0;
@@ -419,10 +386,7 @@ static int create_body(mpcmmd_handle_s* h, const mpcmmd_config* cfg, int device)
         float* zbT;
         if (dalloc(h, &zbT, (size_t)d.iters_in * (S - ne) * dd)) return -1;
         k_transpose_tables<<<64, 256>>>(zb, zbT, d.iters_in, S - ne, dd);
-        float* th0T;
-        if (dalloc(h, &th0T, (size_t)S * dd)) return -1;
-        k_transpose_tables<<<64, 256>>>(theta0, th0T, 1, S, dd);
-        d.z_init = z_init; d.theta0 = theta0; d.theta0T = th0T; d.zb_iter = zb; d.zb_iterT = zbT;
+        d.z_init = z_init; d.theta0 = theta0; d.zb_iter = zb; d.zb_iterT = zbT;
     }
     // opt-in shared memory sizes (raise-only per (device, kernel): see raise_smem)
     cudaDeviceGetAttribute(&h->sm_count, cudaDevAttrMultiProcessorCount, device);
@@ -438,34 +402,15 @@ static int create_body(mpcmmd_handle_s* h, const mpcmmd_config* cfg, int device)
         }
     }
     {
-        const char* mode = getenv("MPCMMD_INNER_CEM");       // test / profiling override of the kernel choice
-        h->inner_mode = !mode ? 0 : !strcmp(mode, "warp") ? INNER_WARP : !strcmp(mode, "cta") ? INNER_CTA : !strcmp(mode, "generic") ? INNER_GENERIC :
-                        !strcmp(mode, "lat") ? INNER_CTA_LAT : !strcmp(mode, "split") ? INNER_SPLIT : !strcmp(mode, "pipe") ? INNER_PIPE : !strcmp(mode, "lat512") ? INNER_LAT512 : 0;
-        if (!inner_cem_is_fast(d) && h->inner_mode != 0) h->inner_mode = INNER_GENERIC;
-        if (inner_cem_is_fast(d)) {
-            const SplitKernels sk = split_kernels(d.nr);
-            if (raise_smem(device, (const void*)sk.eval, split_eval_smem(d)) || raise_smem(device, (const void*)sk.update, split_update_smem(d), true))
-                return fail("k_icem smem opt-in failed");
-            cudaFuncSetAttribute(sk.eval, cudaFuncAttributePreferredSharedMemoryCarveout, 50);     // 12 CTAs x 5.5 KB of operands, the rest stays L1
-            const char* mb = getenv("MPCMMD_PIPE_MINB");
-            if (mb) h->pipe_minb = atoi(mb);
-            if (raise_smem(device, (const void*)pipe_kernel(d.nr, h->pipe_minb), pipe_smem_bytes(d.nr, d.S_in, d.n_el_in), true)) return fail("k_inner_cem_pipe smem opt-in failed");
-        }
+        if (!inner_cem_is_fast(d) && h->inner_mode != INNER_AUTO) h->inner_mode = INNER_GENERIC;
         { const char* mm = getenv("MPCMMD_MATH"); h->fast_math = mm && !strcmp(mm, "fast"); }
-        { const char* cl = getenv("MPCMMD_CHOL"); g_chol = !cl ? 0 : !strcmp(cl, "la") ? 1 : !strcmp(cl, "cta") ? 2 : 0; }
-        for (int kind = INNER_WARP; kind <= INNER_LAT512; kind++) {
-            if (kind == INNER_SPLIT || kind == INNER_PIPE || kind == INNER_BIG) continue;
+        for (int kind : {INNER_CTA, INNER_CTA_LAT, INNER_CTA_FASTMATH, INNER_LAT512, INNER_GENERIC}) {
             if (kind != INNER_GENERIC && !inner_cem_is_fast(d)) continue;
             inner_cem_fn f = inner_cem_kernel(d, kind);
             if (!f) continue;
             const size_t sm = inner_cem_smem_kind(d, kind);
             if (sm > 227 * 1024) return fail("mpcmmd_create: reduced-set state does not fit in shared memory");
-            if (raise_smem(device, (const void*)f, sm, kind != INNER_GENERIC)) return fail("k_inner_cem smem opt-in failed");
-            if (kind == INNER_WARP) {
-                int per_sm = 0;
-                if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, f, 32, sm) != cudaSuccess || per_sm < 1) per_sm = 1;
-                h->warp_grid = per_sm * h->sm_count;
-            }
+            if (raise_smem(device, (const void*)f, sm, inner_is_cta_family(kind))) return fail("k_inner_cem smem opt-in failed");
         }
     }
     CK(cudaStreamCreateWithFlags(&h->own_stream, cudaStreamNonBlocking));
@@ -475,16 +420,6 @@ static int create_body(mpcmmd_handle_s* h, const mpcmmd_config* cfg, int device)
         CK(cudaEventCreateWithFlags(&h->ev_join[i], cudaEventDisableTiming));
     }
     { const char* gv = getenv("MPCMMD_GROUPS"); h->groups_override = gv ? atoi(gv) : 0; }
-    { const char* pv = getenv("MPCMMD_PRIO"); h->prio_mode = pv ? atoi(pv) : 0; }
-    {   // MPCMMD_CARVE=1 (experiment): every kernel of a solve prefers the maximum shared-memory carve-out, so that kernels of concurrent branches / handles
-        // never wait for an SM to drain before its L1 / shared split can change
-        const char* cv = getenv("MPCMMD_CARVE");
-        if (cv) {
-            const void* fns[] = {(const void*)k_project, rollouts_kernel(ROLL_OPT, NZ_BETA_TABLE, 0), rollouts_kernel(ROLL_FLY, NZ_BETA_TABLE, 0), rollouts_kernel(ROLL_STAGED, NZ_BETA_TABLE, 0),
-                                 (const void*)k_opt_risk<false>, (const void*)k_select, (const void*)k_noise, (const void*)k_init, (const void*)k_boundary};
-            for (const void* f : fns) cudaFuncSetAttribute(f, cudaFuncAttributePreferredSharedMemoryCarveout, atoi(cv) == 1 ? cudaSharedmemCarveoutMaxShared : cudaSharedmemCarveoutDefault);
-        }
-    }
     CK(cudaDeviceSynchronize());
     CK(cudaGetLastError());
     return 0;
@@ -535,18 +470,14 @@ static int ensure_opt_scratch(mpcmmd_handle_s* h) {
         if (dalloc(h, &h->big_state, chunk * (per / sizeof(float)))) return -1;
     }
     if (dalloc(h, &h->feat, EB * d.nm * 2 * NV) || dalloc(h, &h->ctrl, EB * 2 * d.nr * d.np)) return -1;
-    // the mother rollouts are stored only for the kernels that read them back (generic / warp-per-chain); allocated on first such launch
+    // the mother rollouts are stored only for the kernels that read them back (generic and large-set)
     h->xroll = h->feat;     // non-null marker: scratch is ready
-    if (!inner_cem_is_fast(d) || h->inner_mode == INNER_WARP || h->inner_mode == INNER_GENERIC) {
+    if (!inner_cem_is_fast(d) || h->inner_mode == INNER_GENERIC) {
         if (dalloc(h, &h->rolls_x, EB * d.nm * d.np) || dalloc(h, &h->rolls_y, EB * d.nm * d.np)) return -1;
     }
     if (dalloc(h, &h->ridx, EB * d.nr)) return -1;
     if (inner_cem_is_fast(d) && dalloc(h, &h->bscratch, EB * d.S_in * (d.nr + 1))) return -1;
     if (inner_cem_is_fast(d) && dalloc(h, &h->mrisk, EB * d.nm * 3)) return -1;
-    // scratch of the opt-in variants only when they are selected (0.35 GB at 200 episodes)
-    if (inner_cem_is_fast(d) && h->inner_mode == INNER_PIPE && dalloc(h, &h->throws, EB * (d.nm + 1) * ICP_TH_LD)) return -1;
-    if (inner_cem_is_fast(d) && h->inner_mode == INNER_SPLIT && dalloc(h, &h->split_state, EB * split_layout(d.nr, d.S_in, d.n_el_in).total)) return -1;
-    if (inner_cem_is_fast(d) && h->warp_grid > 0 && dalloc(h, &h->stash, (size_t)h->warp_grid * d.S_in * ICW_STASH_LD)) return -1;
     CK(cudaDeviceSynchronize());     // dalloc's memsets run on the legacy default stream; solves run on non-blocking streams that do not wait for it
     return 0;
 }
@@ -556,32 +487,26 @@ static int launch_risk(mpcmmd_handle_s* h, const RiskArgs& r, cudaStream_t s, in
     const bool opt = r.cost_kind == MPCMMD_COST_MMD_OPT;
     if (r.n_samples > h->E * d.B) return fail("risk stage: more samples than the workspace holds (max_episodes * num_batch)");
     RollArgs ra;
-    ra.r = r; ra.spb = roll_spb(h, r.cost_kind, r.n_samples); ra.R = opt ? d.nm : d.nr; ra.xroll = h->xroll; ra.yroll = h->yroll; ra.feat = h->feat; ra.stash = nullptr; ra.ridx = h->ridx; ra.bscratch = h->bscratch; ra.ctrl = h->ctrl; ra.write_rolls = 0; ra.fold_risk = 0; ra.mrisk = h->mrisk; ra.stage_ctrl = roll_stage_ctrl(h, r.cost_kind, r.n_samples);
+    ra.r = r; ra.spb = roll_spb(h, r.cost_kind, r.n_samples); ra.R = opt ? d.nm : d.nr; ra.xroll = h->xroll; ra.yroll = h->yroll; ra.feat = h->feat; ra.ridx = h->ridx; ra.bscratch = h->bscratch; ra.ctrl = h->ctrl; ra.write_rolls = 0; ra.fold_risk = 0; ra.mrisk = h->mrisk; ra.stage_ctrl = roll_stage_ctrl(h, r.cost_kind, r.n_samples);
     inner_cem_fn f = nullptr;
     int kind = INNER_GENERIC;
     if (opt) {
-        // default: one 3-warp CTA per chain (k_inner_cem_fast).  The warp-per-chain persistent kernel is kept as an opt-in
-        // (MPCMMD_INNER_CEM=warp): measured 233 ms vs 209 ms per 200-episode mmd_opt solve on B200 (profiles/r01_v7_summary.md) --
-        // 19 independent instruction streams per SM thrash the 32 KB instruction cache.
-        // a launch that fits in one wave of resident CTAs (e.g. a single episode) is latency-bound: take the build with the 96-register budget
-        // a launch of at most 3 chains per SM (one episode = 100 chains) is pure dependency latency: the latency build of the fused kernel
-        // (at most one chain per SM: the 16-warp latency kernel k_inner_cem_lat; up to 3 per SM: the 3-warp latency build of the fused kernel)
-        if (inner_cem_is_fast(d)) kind = h->inner_mode ? h->inner_mode : (r.n_samples <= h->sm_count ? INNER_LAT512 : r.n_samples <= 3 * h->sm_count ? INNER_CTA_LAT : INNER_DEFAULT_THROUGHPUT);
+        // default (num_reduced <= 5): k_inner_cem_fast, one 3-warp CTA per chain.  A launch of at most 3 chains per SM (one episode = 100 chains) is pure
+        // dependency latency: up to 3 chains per SM take the 3-warp latency build of the fused kernel, at most one the 16-warp latency kernel k_inner_cem_lat
+        if (inner_cem_is_fast(d)) kind = h->inner_mode ? h->inner_mode : (r.n_samples <= h->sm_count ? INNER_LAT512 : r.n_samples <= 3 * h->sm_count ? INNER_CTA_LAT : INNER_CTA);
         if (d.nr > MPCMMD_MAX_NR) kind = INNER_BIG;
-        if (kind == INNER_PIPE && !pipe_ok(d)) kind = INNER_CTA;
         if (kind == INNER_CTA && h->fast_math) kind = INNER_CTA_FASTMATH;
-        if (kind == INNER_WARP && !h->stash) return fail("internal: row stash of k_inner_cem_warp not allocated");
-        if (kind != INNER_SPLIT && kind != INNER_PIPE && kind != INNER_BIG) {
+        if (kind != INNER_BIG) {
             f = inner_cem_kernel(d, kind);
             if (!f) return fail("mmd_opt: num_reduced must be in [2, 10]");
         }
         if (!h->xroll) return fail("internal: mmd_opt scratch not allocated");
-        ra.stash = h->stash;
-        // latency regime (at most 3 chains per SM): the serial rollout recurrence is the cost of every kernel, so k_opt_risk's re-roll of the chosen reduced set is
-        // replaced by maxima the mother rollouts fold in themselves (mmd_opt p50 at batch 1: 6.79 -> 6.57 ms).  Larger launches keep the re-roll: the extra
-        // obstacle work in k_rollouts (+20 %) costs more than the short k_opt_risk it removes (measured at 13 / 25 / 50 episodes: 14.4 / 22.9 / 41.8 ms vs 14.7 / 24.0 / 42.4)
-        if (kind != INNER_GENERIC && kind != INNER_WARP && kind != INNER_BIG && h->mrisk && d.O <= OBS_SORT_MIN && r.n_samples <= 3 * h->sm_count) ra.fold_risk = 1;
-        if (kind != INNER_CTA && kind != INNER_CTA_LAT && kind != INNER_CTA_FASTMATH && kind != INNER_LAT512 && kind != INNER_SPLIT && kind != INNER_PIPE) {          // these kernels evaluate the risk themselves from the stored mother rollouts
+        if (inner_is_cta_family(kind)) {
+            // latency regime (at most 3 chains per SM): the serial rollout recurrence is the cost of every kernel, so k_opt_risk's re-roll of the chosen reduced set is
+            // replaced by maxima the mother rollouts fold in themselves (mmd_opt p50 at batch 1: 6.79 -> 6.57 ms).  Larger launches keep the re-roll: the extra
+            // obstacle work in k_rollouts (+20 %) costs more than the short k_opt_risk it removes (measured at 13 / 25 / 50 episodes: 14.4 / 22.9 / 41.8 ms vs 14.7 / 24.0 / 42.4)
+            if (h->mrisk && d.O <= OBS_SORT_MIN && r.n_samples <= 3 * h->sm_count) ra.fold_risk = 1;
+        } else {            // GENERIC and BIG evaluate the risk themselves from the stored mother rollouts
             if (!h->rolls_x) return fail("internal: mother-rollout scratch not allocated");
             ra.write_rolls = 1; ra.xroll = h->rolls_x; ra.yroll = h->rolls_y;
         }
@@ -596,7 +521,16 @@ static int launch_risk(mpcmmd_handle_s* h, const RiskArgs& r, cudaStream_t s, in
         CK(cudaLaunchKernel(fk, dim3(grid), dim3(ROLL_THREADS), kargs, rsm, s));
     }
     if (n_launch) *n_launch = 1;
-    if (opt && kind == INNER_BIG) {
+    if (!opt) return 0;
+    if (inner_is_cta_family(kind)) {           // the k_inner_cem_fast family, then k_opt_risk on the reduced set it chose
+        f<<<r.n_samples, kind == INNER_LAT512 ? ICL_THREADS : ICF_THREADS, inner_cem_smem_kind(d, kind), s>>>(d, ra);
+        const int ospb = OPT_RISK_THREADS / d.nr, grid = (r.n_samples + ospb - 1) / ospb;
+        if (r.sx_obs) k_opt_risk<true><<<grid, OPT_RISK_THREADS, 0, s>>>(d, ra); else k_opt_risk<false><<<grid, OPT_RISK_THREADS, 0, s>>>(d, ra);
+        if (n_launch) *n_launch = 3;
+    } else if (kind == INNER_GENERIC) {
+        f<<<r.n_samples, risko_threads(d.nr), inner_cem_smem_kind(d, kind), s>>>(d, ra);
+        if (n_launch) *n_launch = 2;
+    } else {                                   // INNER_BIG
         if (!h->big_state) return fail("internal: large-reduced-set scratch not allocated");
         int nl = 1;
         for (int g0 = 0; g0 < r.n_samples; g0 += h->big_chunk) {       // chain ranges share the scratch: launches on one stream run in order
@@ -607,33 +541,6 @@ static int launch_risk(mpcmmd_handle_s* h, const RiskArgs& r, cudaStream_t s, in
             nl++;
         }
         if (n_launch) *n_launch = nl;
-    } else if (opt && kind == INNER_PIPE) {
-        pipe_kernel(d.nr, h->pipe_minb)<<<(r.n_samples + 1) / 2, ICP_THREADS, pipe_smem_bytes(d.nr, d.S_in, d.n_el_in), s>>>(d, ra, h->throws);
-        { const int ospb = OPT_RISK_THREADS / d.nr; if (r.sx_obs) k_opt_risk<true><<<(r.n_samples + ospb - 1) / ospb, OPT_RISK_THREADS, 0, s>>>(d, ra); else k_opt_risk<false><<<(r.n_samples + ospb - 1) / ospb, OPT_RISK_THREADS, 0, s>>>(d, ra); }
-        if (n_launch) *n_launch = 3;
-    } else if (opt && kind == INNER_SPLIT) {
-        const SplitKernels sk = split_kernels(d.nr);
-        SplitArgs sa;
-        sa.n_chains = r.n_samples; sa.g0 = 0; sa.state = h->split_state; sa.feat = h->feat; sa.bscratch = h->bscratch;
-        sa.beta = r.beta; sa.sigma = r.sigma; sa.res_beta = r.res_beta; sa.ridx = h->ridx;
-        const long long nd = (long long)r.n_samples * d.nm * d.nm;
-        sk.dist<<<(unsigned)((nd + 255) / 256), 256, 0, s>>>(d, sa);
-        const size_t se = split_eval_smem(d), su = split_update_smem(d);
-        for (int it = 0; it < d.iters_in; it++) {
-            sk.eval<<<r.n_samples, (it == 0 && d.S_in > ICE_THREADS) ? 128 : ICE_THREADS, se, s>>>(d, sa, it);
-            sk.update<<<(r.n_samples + ICU_WARPS - 1) / ICU_WARPS, ICU_WARPS * 32, su, s>>>(d, sa, it);
-        }
-        { const int ospb = OPT_RISK_THREADS / d.nr; if (r.sx_obs) k_opt_risk<true><<<(r.n_samples + ospb - 1) / ospb, OPT_RISK_THREADS, 0, s>>>(d, ra); else k_opt_risk<false><<<(r.n_samples + ospb - 1) / ospb, OPT_RISK_THREADS, 0, s>>>(d, ra); }
-        if (n_launch) *n_launch = 3 + 2 * d.iters_in;
-    } else if (opt) {
-        const size_t sm = inner_cem_smem_kind(d, kind);
-        if (kind == INNER_WARP) f<<<r.n_samples < h->warp_grid ? r.n_samples : h->warp_grid, 32, sm, s>>>(d, ra);
-        else f<<<r.n_samples, kind == INNER_LAT512 ? ICL_THREADS : (kind == INNER_CTA || kind == INNER_CTA_LAT || kind == INNER_CTA_FASTMATH) ? ICF_THREADS : risko_threads(d.nr), sm, s>>>(d, ra);
-        if (n_launch) *n_launch = 2;
-        if (kind == INNER_CTA || kind == INNER_CTA_LAT || kind == INNER_CTA_FASTMATH || kind == INNER_LAT512) {
-            { const int ospb = OPT_RISK_THREADS / d.nr; if (r.sx_obs) k_opt_risk<true><<<(r.n_samples + ospb - 1) / ospb, OPT_RISK_THREADS, 0, s>>>(d, ra); else k_opt_risk<false><<<(r.n_samples + ospb - 1) / ospb, OPT_RISK_THREADS, 0, s>>>(d, ra); }
-            if (n_launch) *n_launch = 3;
-        }
     }
     return 0;
 }
@@ -679,7 +586,7 @@ static int enqueue_solve(mpcmmd_handle_s* h, int kind, int n_ep, cudaStream_t s,
 // (tools/overlap_probe.py, mmd_opt solve of 25 / 50 / 100 episodes): 1 group 24.2 / 41.9 / 78.8 ms, 2 groups 22.6 / 41.1 / 79.5, 3 groups 21.6 / 39.9 / 78.2,
 // 4 groups 22.5 / 42.9 / 78.4.
 static int solve_groups(const mpcmmd_handle_s* h, int kind, int n_ep) {
-    if (n_ep < 2 || h->inner_mode == INNER_WARP) return 1;         // the warp-per-chain kernel's row stash is per persistent CTA, not per chain
+    if (n_ep < 2) return 1;
     if (h->groups_override >= 1 && h->groups_override <= MAX_GROUPS) return h->groups_override < n_ep ? h->groups_override : n_ep;
     const long long chains = (long long)n_ep * h->d.B;
     if (kind != MPCMMD_COST_MMD_OPT || !inner_cem_is_fast(h->d) || chains <= 6LL * h->sm_count || chains > 36LL * h->sm_count) return 1;
@@ -713,27 +620,6 @@ static int get_graph(mpcmmd_handle_s* h, int kind, int n_ep, cudaGraphExec_t* ou
     cudaError_t ce = cudaStreamEndCapture(h->own_stream, &g);
     if (rc) { if (ce == cudaSuccess && g) cudaGraphDestroy(g); return -1; }
     CK(ce);
-    if ((h->prio_mode == 1 && kind == MPCMMD_COST_MMD_OPT) || (h->prio_mode == 2 && kind != MPCMMD_COST_MMD_OPT)) {
-        // Experiment (default off; measured, no effect): when the sweep's cost functions solve concurrently on one device, MPCMMD_PRIO=1 gives the kernel nodes
-        // of mmd_opt graphs (the long pole) the device's highest priority, MPCMMD_PRIO=2 those of the short latency-bound cost functions.  The attribute is accepted
-        // on every node, and the cvar + mmd_opt step of 25 / 50 / 100 episodes takes the same time in all three modes (profiles/r02_overlap_probe.md).
-        int lo = 0, hi = 0;
-        if (cudaDeviceGetStreamPriorityRange(&lo, &hi) == cudaSuccess && hi != lo) {
-            size_t nn = 0; int nset = 0, nfail = 0;
-            if (cudaGraphGetNodes(g, nullptr, &nn) == cudaSuccess && nn) {
-                std::vector<cudaGraphNode_t> nodes(nn);
-                cudaGraphGetNodes(g, nodes.data(), &nn);
-                for (auto nd : nodes) {
-                    cudaGraphNodeType ty;
-                    if (cudaGraphNodeGetType(nd, &ty) != cudaSuccess || ty != cudaGraphNodeTypeKernel) continue;
-                    cudaKernelNodeAttrValue v; memset(&v, 0, sizeof(v)); v.priority = hi;
-                    if (cudaGraphKernelNodeSetAttribute(nd, cudaKernelNodeAttributePriority, &v) == cudaSuccess) nset++; else nfail++;
-                }
-            }
-            cudaGetLastError();
-            if (getenv("MPCMMD_DEBUG")) fprintf(stderr, "[mpcmmd] graph kind %d n_ep %d: priority %d (range %d..%d) set on %d kernel nodes, %d failures\n", kind, n_ep, hi, lo, hi, nset, nfail);
-        }
-    }
     cudaGraphExec_t ge;
     ce = cudaGraphInstantiate(&ge, g, 0);
     cudaGraphDestroy(g);
@@ -798,15 +684,10 @@ extern "C" const char* mpcmmd_inner_cem_path(mpcmmd_handle h) {
     if (!h) return "";
     if (!inner_cem_is_fast(h->d)) return "k_inner_cem (generic, one CTA per chain)";
     switch (h->inner_mode) {
-        case INNER_WARP: return "k_inner_cem_warp (one warp per chain, persistent)";
         case INNER_CTA: return "k_inner_cem_fast (one CTA per chain)";
-        case INNER_PIPE: return "k_inner_cem_pipe (two chains per CTA: 3 evaluation warps + 1 serial warp, pipelined)";
-        case INNER_SPLIT: return "phase-split: k_icem_dist + 20 x (k_icem_eval + k_icem_update)";
         case INNER_CTA_LAT: return "k_inner_cem_fast<LAT> (one CTA per chain, latency build)";
         case INNER_GENERIC: return "k_inner_cem (generic, one CTA per chain)";
-        default: return INNER_DEFAULT_THROUGHPUT == INNER_PIPE
-                            ? "k_inner_cem_pipe (two chains per CTA: 3 evaluation warps + 1 serial warp); launches of <= 3 chains per SM: k_inner_cem_fast<LAT>"
-                            : "k_inner_cem_fast (one CTA per chain); launches of <= 3 chains per SM: its latency build; <= 1 chain per SM: k_inner_cem_lat (16 warps per chain)";
+        default: return "k_inner_cem_fast (one CTA per chain); launches of <= 3 chains per SM: its latency build; <= 1 chain per SM: k_inner_cem_lat (16 warps per chain)";
     }
 }
 

@@ -516,11 +516,13 @@ def test_fast_math_gaussian_within_tolerance(mods, KO, monkeypatch):
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("var,val", [("MPCMMD_INNER_CEM", "warp"), ("MPCMMD_INNER_CEM", "pipe"), ("MPCMMD_INNER_CEM", "split"),
-                                     ("MPCMMD_CHOL", "la"), ("MPCMMD_CHOL", "cta")])
-def test_experimental_variants_refuse_gaussian(mods, monkeypatch, var, val):
+@pytest.mark.parametrize("kernel", ["laplace", "gaussian"])
+@pytest.mark.parametrize("val", ["warp", "pipe", "split", "lat12", ""])
+def test_unknown_inner_cem_override_refused(mods, monkeypatch, kernel, val):
+    """MPCMMD_INNER_CEM outside auto | cta | lat | lat512 | generic (retired kernels, a misspelling, an empty value) is refused at create for
+    both MMD kernel forms, naming the valid values, instead of silently running the default choice"""
     cem_impl, _ = mods
     from mpcmmd_b200 import binding as B
-    monkeypatch.setenv(var, val)
-    with pytest.raises(B.MpcmmdError, match="Laplace only"):
-        cem_impl.CEM(5, 2, 0.1, 30, "gaussian", 0.0, 0.0, max_episodes=1, num_batch=24, kernel="gaussian")
+    monkeypatch.setenv("MPCMMD_INNER_CEM", val)
+    with pytest.raises(B.MpcmmdError, match="MPCMMD_INNER_CEM=.* is not one of auto, cta, lat, lat512, generic"):
+        cem_impl.CEM(5, 2, 0.1, 30, "gaussian", 0.0, 0.0, max_episodes=1, num_batch=24, kernel=kernel)

@@ -1,10 +1,7 @@
 #!/usr/bin/env python
 """Strong-scaled shard of the sweep on ONE GPU (E = 25 / 50 / 100 episodes = the per-rank share at 8 / 4 / 2 GPUs): the cvar + mmd_opt step of bench.py
-(one handle + stream per cost function, concurrent) under the graph-level switches of mpcmmd_create:
-  MPCMMD_GROUPS = episode groups (branches) of a solve graph, MPCMMD_PRIO = highest stream priority on the kernel nodes of mmd_opt graphs,
-  MPCMMD_CARVE  = maximum shared-memory carve-out preference on every kernel of a solve.
-usage: [PROBE_GROUPS=1,2,3,4] [PROBE_PRIOS=0,1,2] [PROBE_CARVES=0,1] overlap_probe.py [E ...]      (writes gpurun_out/overlap_probe.json)"""
-import itertools
+(one handle + stream per cost function, concurrent) for each number of episode groups (branches) of the mmd_opt solve graph (MPCMMD_GROUPS).
+usage: [PROBE_GROUPS=1,2,3,4] overlap_probe.py [E ...]      (writes overlap_probe.json to the output directory at the end of the script)"""
 import json
 import os
 import sys
@@ -42,22 +39,17 @@ def timed(fn, n=9):
 out = {}
 Es = [int(a) for a in sys.argv[1:]] or [25, 50, 100]
 GROUPS = os.environ.get("PROBE_GROUPS", "1,2,3,4").split(",")
-PRIOS = os.environ.get("PROBE_PRIOS", "0").split(",")
-CARVES = os.environ.get("PROBE_CARVES", "0").split(",")
-combos = [dict(MPCMMD_GROUPS=g, MPCMMD_PRIO=p, MPCMMD_CARVE=c) for c, p, g in itertools.product(CARVES, PRIOS, GROUPS)]
 for E in Es:
     host = None
-    for env in combos:
-        os.environ.update(env)
+    for groups in GROUPS:
         hs = {}
         for c in ("cvar", "mmd_opt"):
-            os.environ["MPCMMD_GROUPS"] = env["MPCMMD_GROUPS"] if c == "mmd_opt" else "1"
+            os.environ["MPCMMD_GROUPS"] = groups if c == "mmd_opt" else "1"
             hs[c] = CEM(*args, variant="static", max_episodes=E, device=0)
         if host is None:
             host = scenes.static_batch(hs["cvar"], list(range(E)), "static")
             dev_in = {k: torch.as_tensor(host[k], device=dev) for k in keys}
-        hi = {"0": None, "1": "mmd_opt", "2": "cvar"}[env["MPCMMD_PRIO"]]        # the launching stream's priority follows the node priority
-        streams = {c: torch.cuda.Stream(dev, priority=-1 if c == hi else 0) for c in hs}
+        streams = {c: torch.cuda.Stream(dev) for c in hs}
 
         def serial():
             for c in ("cvar", "mmd_opt"):
@@ -74,7 +66,7 @@ for E in Es:
         t_both = timed(step)
         t_opt = timed(lambda: step(("mmd_opt",)))
         t_cvar = timed(lambda: step(("cvar",)))
-        tag = "E%d_g%s_p%s_c%s" % (E, env["MPCMMD_GROUPS"], env["MPCMMD_PRIO"], env["MPCMMD_CARVE"])
+        tag = "E%d_g%s" % (E, groups)
         t_serial = timed(serial)
         out[tag] = {"both_ms": t_both, "mmd_opt_ms": t_opt, "cvar_ms": t_cvar, "serial_ms": t_serial}
         print(tag, "both %.3f  mmd_opt %.3f  cvar %.3f  serial (one stream) %.3f" % (t_both, t_opt, t_cvar, t_serial), flush=True)

@@ -1,6 +1,6 @@
 #!/bin/bash
-# compute-sanitizer over the kernels that alias shared-memory regions across barriers (k_inner_cem_fast), hand-roll mbarrier / named-barrier
-# protocols (k_project, k_project_tc, k_inner_cem_pipe) or exchange data through L2 (k_icem_*).  Logs -> gpurun_out/sanitize_*.log
+# compute-sanitizer over the kernels that alias shared-memory regions across barriers (k_inner_cem_fast) or hand-roll mbarrier protocols
+# (k_project, k_project_tc).  One log per tool, sanitize_<tool>.log, in the output directory created below.
 set -u
 mkdir -p gpurun_out
 SEL_MEM='inner_cem_kernel_variants or stage_project_bit_exact or solve_small or tensor_core_within or stage_risk_bit_exact or injected'

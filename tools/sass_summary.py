@@ -20,8 +20,8 @@ print("| kernel | SASS instructions | " + " | ".join(keys) + " |"); print("|---|
 for k, c in cnt.items():
     name = subprocess.run(["c++filt", k], capture_output=True, text=True).stdout.strip()
     name = re.sub(r"\(DCfg.*|\(ValCfg.*|\(float const\*.*|\(unsigned.*", "", name).replace("void ", "").replace("(int)", "").replace("(bool)", "")
-    if not re.match(r"k_(project|inner_cem|icem|rollouts|opt_risk|select|noise|obs_sort|validate|init)", name):
+    if not re.match(r"k_(project|inner_cem|rollouts|opt_risk|select|noise|obs_sort|validate|init)", name):
         continue
-    if re.search(r"<[234],|<[234]>|k_inner_cem<[6789]>|pipe<5, (9|12)>|big<256>", name):
+    if re.search(r"<[234],|<[234]>|k_inner_cem<[6789]>|big<256>", name):
         continue
     print("| `%s` | %d | " % (name, sum(c.values())) + " | ".join(str(c.get(x, 0)) for x in keys) + " |")
