@@ -585,8 +585,10 @@ static int enqueue_solve(mpcmmd_handle_s* h, int kind, int n_ep, cudaStream_t s,
 // chains on 1776 resident CTAs): the groups drift out of phase, so one group's tail wave and small kernels are filled by the others' chains.  Measured
 // (tools/overlap_probe.py, mmd_opt solve of 25 / 50 / 100 episodes): 1 group 24.2 / 41.9 / 78.8 ms, 2 groups 22.6 / 41.1 / 79.5, 3 groups 21.6 / 39.9 / 78.2,
 // 4 groups 22.5 / 42.9 / 78.4.
+// MPCMMD_GROUPS overrides the count, except for mmd_opt with large reduced sets (num_reduced > 10): there every chain range of k_inner_cem_big uses the
+// one big_state scratch of the handle, which push_view does not split by episode, so concurrent branches would overwrite each other's chain state.
 static int solve_groups(const mpcmmd_handle_s* h, int kind, int n_ep) {
-    if (n_ep < 2) return 1;
+    if (n_ep < 2 || (kind == MPCMMD_COST_MMD_OPT && h->d.nr > MPCMMD_MAX_NR)) return 1;
     if (h->groups_override >= 1 && h->groups_override <= MAX_GROUPS) return h->groups_override < n_ep ? h->groups_override : n_ep;
     const long long chains = (long long)n_ep * h->d.B;
     if (kind != MPCMMD_COST_MMD_OPT || !inner_cem_is_fast(h->d) || chains <= 6LL * h->sm_count || chains > 36LL * h->sm_count) return 1;
@@ -682,6 +684,7 @@ extern "C" int mpcmmd_solve_host(mpcmmd_handle h, int cost_kind, int n_ep, const
 extern "C" int mpcmmd_last_launch_count(mpcmmd_handle h) { return h ? h->last_launches : 0; }
 extern "C" const char* mpcmmd_inner_cem_path(mpcmmd_handle h) {
     if (!h) return "";
+    if (h->d.nr > MPCMMD_MAX_NR) return "k_inner_cem_big (global chain state, one CTA per chain)";
     if (!inner_cem_is_fast(h->d)) return "k_inner_cem (generic, one CTA per chain)";
     switch (h->inner_mode) {
         case INNER_CTA: return "k_inner_cem_fast (one CTA per chain)";

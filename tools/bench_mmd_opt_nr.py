@@ -24,5 +24,5 @@ for nr, iters in ((5, 20), (10, 20), (20, 4), (40, 1)):
             a.record(); run(); b.record(); torch.cuda.synchronize(); ts.append(a.elapsed_time(b))
         ms = float(np.median(ts)) * 20.0 / iters / E
         fl = scenes.flops_per_sample("mmd_opt", nr, 60, 6); gf = (fl["project"] + fl["risk"]) * 100 * 20 / 1e9
-        print(f"| {nr} | {nr * nr + 1} | {E} | {iters} | {ms:.1f} | {gf:.1f} | {gf / ms:.2f} | {prob.inner_cem_path() if nr <= 5 else ('k_inner_cem<%d> (shared-memory state)' % nr if nr <= 10 else 'k_inner_cem_big (global state)')} |", flush=True)
+        print(f"| {nr} | {nr * nr + 1} | {E} | {iters} | {ms:.1f} | {gf:.1f} | {gf / ms:.2f} | {prob.inner_cem_path()} |", flush=True)
         del prob
