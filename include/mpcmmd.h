@@ -162,6 +162,38 @@ int mpcmmd_validate_threefry_host(int device, int n_ep, int n_roll, int num_prim
                                   const double *state0, const double *x_obs_traj, const double *y_obs_traj, int32_t *count,
                                   int32_t *count_lane, double *acc_out, double *steer_out);
 
+/* Monte-Carlo RISK of each plan (DESIGN.md section 3 item 9) from the per-rollout costs
+ *   c_obs  = max over (obstacle, t < num_prime) of max(0, obstacle cost)  (float32 cost in the static variant, widened; NaN propagates)
+ *   c_lane = max_t max(0, y_lb - y) + max_t max(0, y - y_ub)
+ * p_coll / p_lane = the fraction of rollouts with cost > 0 or NaN (NaN counts as a hit, as in the counts; the solver's saa_cost does not
+ * count NaN); mean_obs; var_obs = v[lo] lw + v[hi] hw at q = alpha (n - 1) over the sorted c_obs (cvar_cost's formula in float64, no FMA);
+ * cvar_obs = the mean of the c_obs >= var_obs; mmd_obs = ker_wt (S / n^2 - 2 E / n), S = sum_ij exp(-|c_i - c_j| / sigma),
+ * E = sum_i exp(-c_i / sigma) (Laplace kernel; the constant term is omitted as in the solver).  Any NaN c_obs makes the four moments NaN.
+ * All HOST pointers; outputs (n_ep,) unless noted.  Bit-reproducible from run to run and at any chunking. */
+typedef struct {
+    double alpha;                 /* VaR / CVaR level, 0..1 (the solver's alpha_quant is 0.98) */
+    double ker_wt;                /* MMD scale (cem.py:165: 1000) */
+    const double *sigma;          /* (n_ep,) Laplace bandwidth per plan (> 0, finite), or NULL: no MMD */
+    double *p_coll, *p_lane, *mean_obs, *var_obs, *cvar_obs;   /* (n_ep,) */
+    double *mmd_obs;              /* (n_ep,), required iff sigma != NULL */
+    double *c_obs, *c_lane;       /* (n_ep, n_roll) per-rollout costs, optional: both or neither */
+} mpcmmd_risk_out;
+/* mpcmmd_validate_host's rollouts and counts (same counts) with the risk statistics; no rollout positions. */
+int mpcmmd_validate_risk_host(int device, int n_ep, int n_roll, int num_prime, int num_obs, int obs_cost_f32, double dt, double wheel_base,
+                              double a_obs, double b_obs, double y_lb, double y_ub, const double *acc, const double *steer,
+                              const double *state0, const double *x_obs_traj, const double *y_obs_traj, int32_t *count,
+                              int32_t *count_lane, const mpcmmd_risk_out *risk);
+/* mpcmmd_validate_threefry_host's rollouts and counts (same counts) with the risk statistics; no perturbed controls. */
+int mpcmmd_validate_threefry_risk_host(int device, int n_ep, int n_roll, int num_prime, int num_obs, int obs_cost_f32, int noise_kind,
+                                       double noise_level, double k_steer, double beta_a, double beta_b, double acc_const_noise,
+                                       double steer_const_noise, double dt, double wheel_base, double a_obs, double b_obs, double y_lb,
+                                       double y_ub, const uint32_t *seed, const double *acc_plan, const double *steer_plan,
+                                       const double *state0, const double *x_obs_traj, const double *y_obs_traj, int32_t *count,
+                                       int32_t *count_lane, const mpcmmd_risk_out *risk);
+/* The statistics of caller-supplied costs: c_obs (n_sets, n), each value >= 0 and finite or NaN; c_lane (n_sets, n) or NULL (p_lane = 0).
+ * risk->c_obs / risk->c_lane are not used. */
+int mpcmmd_risk_stats_host(int device, int n_sets, int n, const double *c_obs, const double *c_lane, const mpcmmd_risk_out *risk);
+
 /* Measured FP32 FMA throughput of the device (TFLOP/s, FMA = 2 flops): the roofline denominator of the FP32-bound kernels. */
 int mpcmmd_fp32_peak(int device, float *tflops, int *sm_count);
 /* Measured special-function-unit peaks (thread-level operations per second / 1e9): gops[0] = ex2.approx (MUFU.EX2), gops[1] = IEEE

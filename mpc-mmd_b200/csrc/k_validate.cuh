@@ -22,8 +22,14 @@ struct ValCfg {
 // Shared counters cnt[(O + 2)][np]: rows 0..O-1 obstacle intersections per (obstacle, timestep), row O lower-lane, row O+1 upper-lane
 // violations per timestep.  val_count adds one rollout state per lane at timestep t; every lane of the warp must call it (ballots).
 // xo, yo: the trajectory's obstacle trajectories (O, np).
+// Risk statistics (DESIGN.md section 3 item 9): a rollout's running maxima of max(0, obstacle cost) over (obstacle, t) and of the two lane
+// violations over t, NaN propagating as np.max(np.maximum(0, .)) does.  Only the RISK instantiations keep them.
+struct ValRisk { double obs, lb, ub; };
+__device__ __forceinline__ double val_nanmax(double m, double v) { return (v > m || v != v) ? v : m; }
+
+template <bool RISK = false>
 __device__ __forceinline__ void val_count(const ValCfg& c, const double* __restrict__ xo, const double* __restrict__ yo, int t, double x,
-                                          double y, bool live, int lane, int* cnt) {
+                                          double y, bool live, int lane, int* cnt, ValRisk* rk = nullptr) {
     const int np = c.np, O = c.O;
     const float a2f = (float)c.a2, b2f = (float)c.b2;
     for (int o = 0; o < O; o++) {
@@ -32,15 +38,18 @@ __device__ __forceinline__ void val_count(const ValCfg& c, const double* __restr
             const float wc = (float)x - (float)xo[o * np + t], ws = (float)y - (float)yo[o * np + t];
             const float cost = ((-(wc * wc)) / a2f - (ws * ws) / b2f) + 1.0f;          // S/validation.py:112
             nz = (cost > 0.0f) || (cost != cost);                                       // np.maximum(0, cost) != 0 (NaN counts)
+            if (RISK) rk->obs = val_nanmax(rk->obs, (double)cost);                      // the float32 maximum, widened exactly
         } else {
             const double wc = x - xo[o * np + t], ws = y - yo[o * np + t];
             const double cost = ((-(wc * wc)) / c.a2 - (ws * ws) / c.b2) + 1.0;
             nz = (cost > 0.0) || (cost != cost);
+            if (RISK) rk->obs = val_nanmax(rk->obs, cost);
         }
         const unsigned m = __ballot_sync(0xffffffffu, live && nz);
         if (lane == 0 && m) atomicAdd(&cnt[o * np + t], __popc(m));
     }
     const double lb = -y + c.y_lb, ub = y - c.y_ub;                                     // S/validation.py:118-119
+    if (RISK) { rk->lb = val_nanmax(rk->lb, lb); rk->ub = val_nanmax(rk->ub, ub); }
     const unsigned ml = __ballot_sync(0xffffffffu, live && ((lb > 0.0) || (lb != lb)));
     const unsigned mu = __ballot_sync(0xffffffffu, live && ((ub > 0.0) || (ub != ub)));
     if (lane == 0 && ml) atomicAdd(&cnt[O * np + t], __popc(ml));
@@ -69,11 +78,15 @@ __device__ __forceinline__ void val_reduce(const int* cnt, int O, int np, int la
     if (lane == 0) { *count = m; *count_lane = l + u; }
 }
 
-// grid = episodes; thread r handles rollouts r, r + VAL_THREADS, ...
+// grid = episodes; thread r handles rollouts r, r + VAL_THREADS, ...  RISK: c_obs, c_lane (n_ep, n_roll) receive each rollout's obstacle and lane
+// costs (DESIGN.md section 3 item 9); the counting is the same.  The two pointers come last, so RISK = false compiles to the counting-only
+// kernel's instructions with the same parameter offsets.
+template <bool RISK>
 __global__ void __launch_bounds__(VAL_THREADS) k_validate(ValCfg c, const double* __restrict__ acc, const double* __restrict__ steer,
                                                           const double* __restrict__ state0, const double* __restrict__ x_obs,
                                                           const double* __restrict__ y_obs, int32_t* __restrict__ count,
-                                                          int32_t* __restrict__ count_lane, double* __restrict__ x_roll, double* __restrict__ y_roll) {
+                                                          int32_t* __restrict__ count_lane, double* __restrict__ x_roll, double* __restrict__ y_roll,
+                                                          double* __restrict__ c_obs, double* __restrict__ c_lane) {
     extern __shared__ int cnt[];
     const int e = blockIdx.x, tid = threadIdx.x, lane = tid & 31;
     const int np = c.np, O = c.O;
@@ -87,12 +100,18 @@ __global__ void __launch_bounds__(VAL_THREADS) k_validate(ValCfg c, const double
         const bool live = r < c.n_roll;
         const size_t row = ((size_t)e * c.n_roll + (live ? r : 0)) * np;
         double x = s0[0], y = s0[1], vx = s0[2], vy = s0[3], psi = s0[4];
+        // the maxima live in shared memory: in registers they would be saved around the double trig slow-path call (local-memory spills)
+        __shared__ ValRisk rks[VAL_THREADS];
+        ValRisk& rk = rks[tid];
+        if constexpr (RISK) rk = ValRisk{0.0, 0.0, 0.0};
         for (int t = 0; t < np; t++) {
             // ---- record the state before the step (S/validation.py:98-100) and count on it
             if (live && x_roll) { x_roll[row + t] = x; y_roll[row + t] = y; }
-            val_count(c, xo, yo, t, x, y, live, lane, cnt);
+            if constexpr (RISK) val_count<true>(c, xo, yo, t, x, y, live, lane, cnt, &rk);
+            else val_count(c, xo, yo, t, x, y, live, lane, cnt);
             val_step(c, live ? acc[row + t] : 0.0, live ? steer[row + t] : 0.0, x, y, vx, vy, psi);
         }
+        if (RISK && live) { c_obs[row / np] = rk.obs; c_lane[row / np] = rk.lb + rk.ub; }
     }
     __syncthreads();
     if (tid < 32) val_reduce(cnt, O, np, lane, count + e, count_lane + e);

@@ -28,11 +28,14 @@ struct ValJaxCfg {
 
 // seed (n_ep,); acc_plan, steer_plan (n_ep, np); state0, x_obs, y_obs as k_validate; cnt_g (n_ep, O + 2, np) zeroed;
 // acc_out, steer_out (n_ep, n_roll, np) the perturbed controls, or null.  Trajectory e = e0 + blockIdx.y.
+// RISK: c_obs, c_lane (gridDim.y, n_roll) -- indexed by blockIdx.y, not e -- receive each rollout's obstacle and lane costs (as k_validate<true>).
+template <bool RISK>
 __global__ void __launch_bounds__(VALJ_THREADS) k_validate_jax(ValCfg c, ValJaxCfg j, int e0, const uint32_t* __restrict__ seed,
                                                                const double* __restrict__ acc_plan, const double* __restrict__ steer_plan,
                                                                const double* __restrict__ state0, const double* __restrict__ x_obs,
                                                                const double* __restrict__ y_obs, int32_t* __restrict__ cnt_g,
-                                                               double* __restrict__ acc_out, double* __restrict__ steer_out) {
+                                                               double* __restrict__ acc_out, double* __restrict__ steer_out,
+                                                               double* __restrict__ c_obs, double* __restrict__ c_lane) {
     extern __shared__ int cnt[];
     const int e = e0 + blockIdx.y, tid = threadIdx.x, lane = tid & 31;
     const int np = c.np, O = c.O;
@@ -51,8 +54,10 @@ __global__ void __launch_bounds__(VALJ_THREADS) k_validate_jax(ValCfg c, ValJaxC
     if (j.noise_kind == 1) { dr::split2(k_acc, ka_acc, kb_acc); dr::split2(k_steer, ka_steer, kb_steer); }
     const size_t row = ((size_t)e * c.n_roll + (live ? r : 0)) * np;
     double x = s0[0], y = s0[1], vx = s0[2], vy = s0[3], psi = s0[4];
+    ValRisk rk = {0.0, 0.0, 0.0};
     for (int t = 0; t < np; t++) {
-        val_count(c, xo, yo, t, x, y, live, lane, cnt);
+        if constexpr (RISK) val_count<true>(c, xo, yo, t, x, y, live, lane, cnt, &rk);
+        else val_count(c, xo, yo, t, x, y, live, lane, cnt);
         double a = 0.0, st = 0.0;
         if (live) {
             const uint32_t el = (uint32_t)r * (uint32_t)np + (uint32_t)t;
@@ -72,6 +77,10 @@ __global__ void __launch_bounds__(VALJ_THREADS) k_validate_jax(ValCfg c, ValJaxC
             if (acc_out) { acc_out[row + t] = a; steer_out[row + t] = st; }
         }
         val_step(c, a, st, x, y, vx, vy, psi);
+    }
+    if (RISK && live) {
+        const size_t i = (size_t)blockIdx.y * c.n_roll + r;
+        c_obs[i] = rk.obs; c_lane[i] = rk.lb + rk.ub;
     }
     __syncthreads();
     int32_t* g = cnt_g + (size_t)e * (O + 2) * np;

@@ -20,6 +20,7 @@
 #include "k_validate.cuh"
 #include "k_validate_noise.cuh"
 #include "k_validate_jax.cuh"
+#include "k_risk_stats.cuh"
 
 static thread_local std::string g_err;
 static int fail(const std::string& m) { g_err = m; return -1; }
@@ -862,13 +863,13 @@ static cudaError_t launch_validate(int n_ep, int n_roll, int num_prime, int num_
                                    const double* d_s0, const double* d_xo, const double* d_yo, int32_t* d_cnt, int32_t* d_lane,
                                    double* d_xr, double* d_yr) {
     if (smem > 48 * 1024) {
-        const cudaError_t e = cudaFuncSetAttribute(k_validate, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        const cudaError_t e = cudaFuncSetAttribute(k_validate<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) return e;
     }
     ValCfg c;
     c.n_roll = n_roll; c.np = num_prime; c.O = num_obs; c.obs_f32 = obs_cost_f32; c.dt = dt; c.wheel_base = wheel_base;
     c.a2 = a_obs * a_obs; c.b2 = b_obs * b_obs; c.y_lb = y_lb; c.y_ub = y_ub;
-    k_validate<<<n_ep, VAL_THREADS, smem>>>(c, d_acc, d_steer, d_s0, d_xo, d_yo, d_cnt, d_lane, d_xr, d_yr);
+    k_validate<false><<<n_ep, VAL_THREADS, smem>>>(c, d_acc, d_steer, d_s0, d_xo, d_yo, d_cnt, d_lane, d_xr, d_yr, nullptr, nullptr);
     return cudaGetLastError();
 }
 
@@ -999,7 +1000,7 @@ extern "C" int mpcmmd_validate_threefry_host(int device, int n_ep, int n_roll, i
         CK(cudaMemcpy(d_s0, state0, (size_t)n_ep * 5 * 8, cudaMemcpyHostToDevice));
         CK(cudaMemcpy(d_xo, x_obs_traj, no * 8, cudaMemcpyHostToDevice)); CK(cudaMemcpy(d_yo, y_obs_traj, no * 8, cudaMemcpyHostToDevice));
         CK(cudaMemset(d_cg, 0, ncnt * 4));
-        if (smem > 48 * 1024) CK(cudaFuncSetAttribute(k_validate_jax, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        if (smem > 48 * 1024) CK(cudaFuncSetAttribute(k_validate_jax<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         ValCfg c;
         c.n_roll = n_roll; c.np = num_prime; c.O = num_obs; c.obs_f32 = obs_cost_f32; c.dt = dt; c.wheel_base = wheel_base;
         c.a2 = a_obs * a_obs; c.b2 = b_obs * b_obs; c.y_lb = y_lb; c.y_ub = y_ub;
@@ -1009,7 +1010,7 @@ extern "C" int mpcmmd_validate_threefry_host(int device, int n_ep, int n_roll, i
         const unsigned chunks = (unsigned)((n_roll + VALJ_THREADS - 1) / VALJ_THREADS);
         for (int e0 = 0; e0 < n_ep; e0 += 65535) {                      // gridDim.y <= 65535 trajectories per launch
             const dim3 grid(chunks, (unsigned)(n_ep - e0 < 65535 ? n_ep - e0 : 65535));
-            k_validate_jax<<<grid, VALJ_THREADS, smem>>>(c, j, e0, d_seed, d_ap, d_sp, d_s0, d_xo, d_yo, d_cg, d_acc, d_steer);
+            k_validate_jax<false><<<grid, VALJ_THREADS, smem>>>(c, j, e0, d_seed, d_ap, d_sp, d_s0, d_xo, d_yo, d_cg, d_acc, d_steer, nullptr, nullptr);
             CK(cudaGetLastError());
         }
         k_validate_finish<<<n_ep, 32>>>(num_obs, num_prime, d_cg, d_cnt, d_lane);
@@ -1021,6 +1022,217 @@ extern "C" int mpcmmd_validate_threefry_host(int device, int n_ep, int n_roll, i
     const int rc = body();
     cudaFree(d_seed); cudaFree(d_ap); cudaFree(d_sp); cudaFree(d_acc); cudaFree(d_steer); cudaFree(d_s0); cudaFree(d_xo); cudaFree(d_yo);
     cudaFree(d_cg); cudaFree(d_cnt); cudaFree(d_lane);
+    return rc;
+}
+
+// ------------------------------------------------------------------------------------------------
+// Monte-Carlo risk statistics (DESIGN.md section 3 item 9): each rollout's obstacle and lane costs (k_validate<true> / k_validate_jax<true>),
+// then k_risk_stats per plan.  The per-rollout arrays (16 B per rollout) live in a fixed device scratch: the plans run in chunks that fit it
+// (one plan at least), like k_inner_cem_big's chain ranges.  Every statistic depends on its plan alone, so the chunking changes no bit.
+static const size_t RISK_SCRATCH_BYTES = (size_t)1 << 30;
+
+// plans per chunk when each rollout takes `per_roll` bytes of device scratch
+static int risk_chunk(int n_ep, long long n_roll, size_t per_roll) {
+    const long long k = (long long)(RISK_SCRATCH_BYTES / per_roll) / n_roll;
+    return (int)(k < 1 ? 1 : (k > n_ep ? n_ep : k));
+}
+
+static int risk_check(const char* fn, const mpcmmd_risk_out* r, int n_sets) {
+    if (!r) return fail(std::string(fn) + ": null risk output");
+    if (!(r->alpha >= 0.0 && r->alpha <= 1.0)) return fail(std::string(fn) + ": alpha must lie in [0, 1]");
+    if (!r->p_coll || !r->p_lane || !r->mean_obs || !r->var_obs || !r->cvar_obs) return fail(std::string(fn) + ": null statistics pointer");
+    if ((r->sigma == nullptr) != (r->mmd_obs == nullptr)) return fail(std::string(fn) + ": sigma and mmd_obs must both be given or both be null");
+    if ((r->c_obs == nullptr) != (r->c_lane == nullptr)) return fail(std::string(fn) + ": c_obs and c_lane must both be given or both be null");
+    if (r->sigma)
+        for (int i = 0; i < n_sets; i++)
+            if (!(r->sigma[i] > 0.0 && isfinite(r->sigma[i]))) return fail(std::string(fn) + ": sigma must be positive and finite");
+    return 0;
+}
+
+// k_risk_stats on plans [e0, e0 + ne) whose per-rollout costs are in d_co / d_cl (ne, n) (overwritten); results to the host arrays of r
+static int risk_run_chunk(const mpcmmd_risk_out* r, int e0, int ne, int n, const double* d_sigma, double* d_co, double* d_cl, double* d_st,
+                          std::vector<double>& h_st) {
+    k_risk_stats<<<ne, RS_THREADS>>>(n, r->alpha, r->ker_wt, d_sigma ? d_sigma + e0 : nullptr, d_co, d_cl, d_st);
+    CK(cudaGetLastError());
+    h_st.resize((size_t)ne * RS_OUT);
+    CK(cudaMemcpy(h_st.data(), d_st, (size_t)ne * RS_OUT * 8, cudaMemcpyDeviceToHost));
+    for (int i = 0; i < ne; i++) {
+        const double* q = &h_st[(size_t)i * RS_OUT];
+        r->p_coll[e0 + i] = q[0]; r->p_lane[e0 + i] = q[1]; r->mean_obs[e0 + i] = q[2]; r->var_obs[e0 + i] = q[3]; r->cvar_obs[e0 + i] = q[4];
+        if (r->mmd_obs) r->mmd_obs[e0 + i] = q[5];
+    }
+    return 0;
+}
+
+// the per-rollout costs of a chunk to the caller (before k_risk_stats overwrites them)
+static int risk_copy_costs(const mpcmmd_risk_out* r, int e0, int ne, int n_roll, const double* d_co, const double* d_cl) {
+    if (!r->c_obs) return 0;
+    const size_t off = (size_t)e0 * n_roll, cnt = (size_t)ne * n_roll * 8;
+    CK(cudaMemcpy(r->c_obs + off, d_co, cnt, cudaMemcpyDeviceToHost));
+    CK(cudaMemcpy(r->c_lane + off, d_cl, cnt, cudaMemcpyDeviceToHost));
+    return 0;
+}
+
+static int risk_upload_sigma(const mpcmmd_risk_out* r, int n_ep, double** d_sigma) {
+    if (!r->sigma) return 0;
+    CK(cudaMalloc(d_sigma, (size_t)n_ep * 8));
+    CK(cudaMemcpy(*d_sigma, r->sigma, (size_t)n_ep * 8, cudaMemcpyHostToDevice));
+    return 0;
+}
+
+// mpcmmd_validate_host's rollouts and counts, plus the risk statistics.  Host-drawn controls take 16 B per knot and rollout on the device,
+// so they are uploaded chunk by chunk as well.
+extern "C" int mpcmmd_validate_risk_host(int device, int n_ep, int n_roll, int num_prime, int num_obs, int obs_cost_f32, double dt, double wheel_base,
+                                         double a_obs, double b_obs, double y_lb, double y_ub, const double* acc, const double* steer,
+                                         const double* state0, const double* x_obs_traj, const double* y_obs_traj, int32_t* count,
+                                         int32_t* count_lane, const mpcmmd_risk_out* risk) {
+    const char* fn = "mpcmmd_validate_risk_host";
+    int ndev = 0;
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) return fail(std::string(fn) + ": no CUDA device (this library has no CPU fallback)");
+    if (device < 0 || device >= ndev) return fail(std::string(fn) + ": bad device index");
+    if (n_ep < 1 || n_roll < 1 || num_prime < 1 || num_prime > MPCMMD_T || num_obs < 1) return fail(std::string(fn) + ": bad sizes");
+    if ((long long)n_roll * num_prime >= (1LL << 31)) return fail(std::string(fn) + ": n_roll * num_prime must be below 2^31");
+    if (!acc || !steer || !state0 || !x_obs_traj || !y_obs_traj || !count || !count_lane) return fail(std::string(fn) + ": null pointer");
+    if (risk_check(fn, risk, n_ep)) return -1;
+    const size_t smem = (size_t)(num_obs + 2) * num_prime * sizeof(int);
+    if (smem > 200 * 1024) return fail(std::string(fn) + ": (num_obs + 2) * num_prime counters do not fit in shared memory");
+    CK(cudaSetDevice(device));
+    const int chunk = risk_chunk(n_ep, n_roll, 16 + 16 * (size_t)num_prime);
+    const size_t rc_ = (size_t)chunk * n_roll, np = (size_t)num_prime, no = (size_t)n_ep * num_obs * np;
+    double *d_acc = nullptr, *d_steer = nullptr, *d_s0 = nullptr, *d_xo = nullptr, *d_yo = nullptr, *d_co = nullptr, *d_cl = nullptr, *d_sigma = nullptr, *d_st = nullptr;
+    int32_t *d_cnt = nullptr, *d_lane = nullptr;
+    std::vector<double> h_st;
+    auto body = [&]() -> int {
+        CK(cudaMalloc(&d_acc, rc_ * np * 8)); CK(cudaMalloc(&d_steer, rc_ * np * 8)); CK(cudaMalloc(&d_s0, (size_t)n_ep * 5 * 8));
+        CK(cudaMalloc(&d_xo, no * 8)); CK(cudaMalloc(&d_yo, no * 8)); CK(cudaMalloc(&d_cnt, (size_t)n_ep * 4)); CK(cudaMalloc(&d_lane, (size_t)n_ep * 4));
+        CK(cudaMalloc(&d_co, rc_ * 8)); CK(cudaMalloc(&d_cl, rc_ * 8)); CK(cudaMalloc(&d_st, (size_t)chunk * RS_OUT * 8));
+        if (risk_upload_sigma(risk, n_ep, &d_sigma)) return -1;
+        CK(cudaMemcpy(d_s0, state0, (size_t)n_ep * 5 * 8, cudaMemcpyHostToDevice));
+        CK(cudaMemcpy(d_xo, x_obs_traj, no * 8, cudaMemcpyHostToDevice)); CK(cudaMemcpy(d_yo, y_obs_traj, no * 8, cudaMemcpyHostToDevice));
+        if (smem > 48 * 1024) CK(cudaFuncSetAttribute(k_validate<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        ValCfg c;
+        c.n_roll = n_roll; c.np = num_prime; c.O = num_obs; c.obs_f32 = obs_cost_f32; c.dt = dt; c.wheel_base = wheel_base;
+        c.a2 = a_obs * a_obs; c.b2 = b_obs * b_obs; c.y_lb = y_lb; c.y_ub = y_ub;
+        for (int e0 = 0; e0 < n_ep; e0 += chunk) {
+            const int ne = n_ep - e0 < chunk ? n_ep - e0 : chunk;
+            const size_t k0 = (size_t)e0 * n_roll * np, nk = (size_t)ne * n_roll * np, oo = (size_t)e0 * num_obs * np;
+            CK(cudaMemcpy(d_acc, acc + k0, nk * 8, cudaMemcpyHostToDevice)); CK(cudaMemcpy(d_steer, steer + k0, nk * 8, cudaMemcpyHostToDevice));
+            k_validate<true><<<ne, VAL_THREADS, smem>>>(c, d_acc, d_steer, d_s0 + (size_t)e0 * 5, d_xo + oo, d_yo + oo, d_cnt + e0, d_lane + e0,
+                                                         nullptr, nullptr, d_co, d_cl);
+            CK(cudaGetLastError());
+            if (risk_copy_costs(risk, e0, ne, n_roll, d_co, d_cl)) return -1;
+            if (risk_run_chunk(risk, e0, ne, n_roll, d_sigma, d_co, d_cl, d_st, h_st)) return -1;
+        }
+        CK(cudaMemcpy(count, d_cnt, (size_t)n_ep * 4, cudaMemcpyDeviceToHost)); CK(cudaMemcpy(count_lane, d_lane, (size_t)n_ep * 4, cudaMemcpyDeviceToHost));
+        return 0;
+    };
+    const int rc = body();
+    cudaFree(d_acc); cudaFree(d_steer); cudaFree(d_s0); cudaFree(d_xo); cudaFree(d_yo); cudaFree(d_cnt); cudaFree(d_lane);
+    cudaFree(d_co); cudaFree(d_cl); cudaFree(d_sigma); cudaFree(d_st);
+    return rc;
+}
+
+// mpcmmd_validate_threefry_host's rollouts and counts, plus the risk statistics
+extern "C" int mpcmmd_validate_threefry_risk_host(int device, int n_ep, int n_roll, int num_prime, int num_obs, int obs_cost_f32, int noise_kind,
+                                                  double noise_level, double k_steer, double beta_a, double beta_b, double acc_const_noise,
+                                                  double steer_const_noise, double dt, double wheel_base, double a_obs, double b_obs, double y_lb,
+                                                  double y_ub, const uint32_t* seed, const double* acc_plan, const double* steer_plan,
+                                                  const double* state0, const double* x_obs_traj, const double* y_obs_traj, int32_t* count,
+                                                  int32_t* count_lane, const mpcmmd_risk_out* risk) {
+    const char* fn = "mpcmmd_validate_threefry_risk_host";
+    int ndev = 0;
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) return fail(std::string(fn) + ": no CUDA device (this library has no CPU fallback)");
+    if (device < 0 || device >= ndev) return fail(std::string(fn) + ": bad device index");
+    if (n_roll < 1) return fail(std::string(fn) + ": n_roll must be >= 1");
+    if (n_ep < 1 || num_prime < 1 || num_prime > MPCMMD_T || num_obs < 1) return fail(std::string(fn) + ": bad sizes");
+    if ((long long)n_roll * num_prime >= (1LL << 31))
+        return fail(std::string(fn) + ": n_roll * num_prime must be below 2^31 (JAX's uint32 element counters)");
+    if (noise_kind != 0 && noise_kind != 1) return fail(std::string(fn) + ": noise_kind must be 0 (gaussian) or 1 (beta)");
+    if (!seed || !acc_plan || !steer_plan || !state0 || !x_obs_traj || !y_obs_traj || !count || !count_lane) return fail(std::string(fn) + ": null pointer");
+    if (risk_check(fn, risk, n_ep)) return -1;
+    const size_t smem = (size_t)(num_obs + 2) * num_prime * sizeof(int);
+    if (smem > 200 * 1024) return fail(std::string(fn) + ": (num_obs + 2) * num_prime counters do not fit in shared memory");
+    CK(cudaSetDevice(device));
+    const int chunk = risk_chunk(n_ep, n_roll, 16);
+    const size_t rc_ = (size_t)chunk * n_roll, no = (size_t)n_ep * num_obs * num_prime, npl = (size_t)n_ep * num_prime;
+    const size_t ncnt = (size_t)n_ep * (num_obs + 2) * num_prime;
+    double *d_ap = nullptr, *d_sp = nullptr, *d_s0 = nullptr, *d_xo = nullptr, *d_yo = nullptr, *d_co = nullptr, *d_cl = nullptr, *d_sigma = nullptr, *d_st = nullptr;
+    uint32_t* d_seed = nullptr;
+    int32_t *d_cg = nullptr, *d_cnt = nullptr, *d_lane = nullptr;
+    std::vector<double> h_st;
+    auto body = [&]() -> int {
+        CK(cudaMalloc(&d_seed, (size_t)n_ep * 4)); CK(cudaMalloc(&d_ap, npl * 8)); CK(cudaMalloc(&d_sp, npl * 8));
+        CK(cudaMalloc(&d_s0, (size_t)n_ep * 5 * 8)); CK(cudaMalloc(&d_xo, no * 8)); CK(cudaMalloc(&d_yo, no * 8));
+        CK(cudaMalloc(&d_cg, ncnt * 4)); CK(cudaMalloc(&d_cnt, (size_t)n_ep * 4)); CK(cudaMalloc(&d_lane, (size_t)n_ep * 4));
+        CK(cudaMalloc(&d_co, rc_ * 8)); CK(cudaMalloc(&d_cl, rc_ * 8)); CK(cudaMalloc(&d_st, (size_t)chunk * RS_OUT * 8));
+        if (risk_upload_sigma(risk, n_ep, &d_sigma)) return -1;
+        CK(cudaMemcpy(d_seed, seed, (size_t)n_ep * 4, cudaMemcpyHostToDevice));
+        CK(cudaMemcpy(d_ap, acc_plan, npl * 8, cudaMemcpyHostToDevice)); CK(cudaMemcpy(d_sp, steer_plan, npl * 8, cudaMemcpyHostToDevice));
+        CK(cudaMemcpy(d_s0, state0, (size_t)n_ep * 5 * 8, cudaMemcpyHostToDevice));
+        CK(cudaMemcpy(d_xo, x_obs_traj, no * 8, cudaMemcpyHostToDevice)); CK(cudaMemcpy(d_yo, y_obs_traj, no * 8, cudaMemcpyHostToDevice));
+        CK(cudaMemset(d_cg, 0, ncnt * 4));
+        if (smem > 48 * 1024) CK(cudaFuncSetAttribute(k_validate_jax<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        ValCfg c;
+        c.n_roll = n_roll; c.np = num_prime; c.O = num_obs; c.obs_f32 = obs_cost_f32; c.dt = dt; c.wheel_base = wheel_base;
+        c.a2 = a_obs * a_obs; c.b2 = b_obs * b_obs; c.y_lb = y_lb; c.y_ub = y_ub;
+        ValJaxCfg j;
+        j.noise_kind = noise_kind; j.nl = noise_level; j.ks = k_steer * noise_level; j.beta_a = beta_a; j.beta_b = beta_b;
+        j.c_acc = acc_const_noise; j.c_steer = steer_const_noise;
+        const unsigned chunks = (unsigned)((n_roll + VALJ_THREADS - 1) / VALJ_THREADS);
+        for (int c0 = 0; c0 < n_ep; c0 += chunk) {
+            const int ne = n_ep - c0 < chunk ? n_ep - c0 : chunk;
+            for (int e0 = c0; e0 < c0 + ne; e0 += 65535) {                    // gridDim.y <= 65535 trajectories per launch
+                const int ny = c0 + ne - e0 < 65535 ? c0 + ne - e0 : 65535;
+                const size_t ro = (size_t)(e0 - c0) * n_roll;
+                k_validate_jax<true><<<dim3(chunks, (unsigned)ny), VALJ_THREADS, smem>>>(c, j, e0, d_seed, d_ap, d_sp, d_s0, d_xo, d_yo, d_cg,
+                                                                                      nullptr, nullptr, d_co + ro, d_cl + ro);
+                CK(cudaGetLastError());
+            }
+            if (risk_copy_costs(risk, c0, ne, n_roll, d_co, d_cl)) return -1;
+            if (risk_run_chunk(risk, c0, ne, n_roll, d_sigma, d_co, d_cl, d_st, h_st)) return -1;
+        }
+        k_validate_finish<<<n_ep, 32>>>(num_obs, num_prime, d_cg, d_cnt, d_lane);
+        CK(cudaGetLastError());
+        CK(cudaMemcpy(count, d_cnt, (size_t)n_ep * 4, cudaMemcpyDeviceToHost)); CK(cudaMemcpy(count_lane, d_lane, (size_t)n_ep * 4, cudaMemcpyDeviceToHost));
+        return 0;
+    };
+    const int rc = body();
+    cudaFree(d_seed); cudaFree(d_ap); cudaFree(d_sp); cudaFree(d_s0); cudaFree(d_xo); cudaFree(d_yo);
+    cudaFree(d_cg); cudaFree(d_cnt); cudaFree(d_lane); cudaFree(d_co); cudaFree(d_cl); cudaFree(d_sigma); cudaFree(d_st);
+    return rc;
+}
+
+// k_risk_stats on caller-supplied costs: n_sets sets of n values each
+extern "C" int mpcmmd_risk_stats_host(int device, int n_sets, int n, const double* c_obs, const double* c_lane, const mpcmmd_risk_out* risk) {
+    const char* fn = "mpcmmd_risk_stats_host";
+    int ndev = 0;
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) return fail(std::string(fn) + ": no CUDA device (this library has no CPU fallback)");
+    if (device < 0 || device >= ndev) return fail(std::string(fn) + ": bad device index");
+    if (n_sets < 1 || n < 1) return fail(std::string(fn) + ": n_sets and n must be >= 1");
+    if (!c_obs) return fail(std::string(fn) + ": null c_obs");
+    if (risk_check(fn, risk, n_sets)) return -1;
+    for (size_t i = 0; i < (size_t)n_sets * n; i++)
+        if (c_obs[i] < 0.0 || c_obs[i] == INFINITY) return fail(std::string(fn) + ": c_obs values must be >= 0 and finite, or NaN");
+    CK(cudaSetDevice(device));
+    const int chunk = risk_chunk(n_sets, n, 16);
+    const size_t rc_ = (size_t)chunk * n;
+    double *d_co = nullptr, *d_cl = nullptr, *d_sigma = nullptr, *d_st = nullptr;
+    std::vector<double> h_st;
+    auto body = [&]() -> int {
+        CK(cudaMalloc(&d_co, rc_ * 8)); CK(cudaMalloc(&d_cl, rc_ * 8)); CK(cudaMalloc(&d_st, (size_t)chunk * RS_OUT * 8));
+        if (risk_upload_sigma(risk, n_sets, &d_sigma)) return -1;
+        for (int e0 = 0; e0 < n_sets; e0 += chunk) {
+            const int ne = n_sets - e0 < chunk ? n_sets - e0 : chunk;
+            const size_t k0 = (size_t)e0 * n, nk = (size_t)ne * n;
+            CK(cudaMemcpy(d_co, c_obs + k0, nk * 8, cudaMemcpyHostToDevice));
+            if (c_lane) CK(cudaMemcpy(d_cl, c_lane + k0, nk * 8, cudaMemcpyHostToDevice));
+            else CK(cudaMemset(d_cl, 0, nk * 8));
+            if (risk_run_chunk(risk, e0, ne, n, d_sigma, d_co, d_cl, d_st, h_st)) return -1;
+        }
+        return 0;
+    };
+    const int rc = body();
+    cudaFree(d_co); cudaFree(d_cl); cudaFree(d_sigma); cudaFree(d_st);
     return rc;
 }
 

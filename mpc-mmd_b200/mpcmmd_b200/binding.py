@@ -33,10 +33,17 @@ class MpcmmdOut(C.Structure):
     _fields_ = [(n, C.c_void_p) for n in ("cx", "cy", "cost_lane", "cost_obs", "beta", "sigma", "res_beta")]
 
 
+class MpcmmdRiskOut(C.Structure):
+    """mpcmmd_risk_out (include/mpcmmd.h): the Monte-Carlo risk statistics of the validation entry points"""
+    _fields_ = [("alpha", C.c_double), ("ker_wt", C.c_double)] + \
+               [(n, C.c_void_p) for n in ("sigma", "p_coll", "p_lane", "mean_obs", "var_obs", "cvar_obs", "mmd_obs", "c_obs", "c_lane")]
+
+
 EXPORTS = ("mpcmmd_last_error", "mpcmmd_version", "mpcmmd_create", "mpcmmd_create_with_kernel", "mpcmmd_destroy", "mpcmmd_solve", "mpcmmd_solve_host",
            "mpcmmd_last_launch_count", "mpcmmd_inner_cem_path", "mpcmmd_profile_solve", "mpcmmd_fp32_peak", "mpcmmd_xu_peaks", "mpcmmd_selfcheck_ieee", "mpcmmd_math_vec", "mpcmmd_rng_normal", "mpcmmd_rng_beta", "mpcmmd_get_tables",
            "mpcmmd_stage_project", "mpcmmd_stage_risk", "mpcmmd_stage_risk_injected", "mpcmmd_stage_init", "mpcmmd_stage_select", "mpcmmd_stage_noise", "mpcmmd_validate_host",
-           "mpcmmd_validate_seeded_host", "mpcmmd_validate_threefry_host")
+           "mpcmmd_validate_seeded_host", "mpcmmd_validate_threefry_host", "mpcmmd_validate_risk_host", "mpcmmd_validate_threefry_risk_host",
+           "mpcmmd_risk_stats_host")
 
 _lib = None
 
@@ -81,6 +88,10 @@ def load():
     lib.mpcmmd_validate_host.argtypes = [C.c_int] * 6 + [C.c_double] * 6 + [V] * 9
     lib.mpcmmd_validate_seeded_host.argtypes = [C.c_int] * 7 + [C.c_double] * 12 + [V] * 11
     lib.mpcmmd_validate_threefry_host.argtypes = [C.c_int] * 7 + [C.c_double] * 12 + [V] * 10
+    RP = C.POINTER(MpcmmdRiskOut)
+    lib.mpcmmd_validate_risk_host.argtypes = [C.c_int] * 6 + [C.c_double] * 6 + [V] * 7 + [RP]
+    lib.mpcmmd_validate_threefry_risk_host.argtypes = [C.c_int] * 7 + [C.c_double] * 12 + [V] * 8 + [RP]
+    lib.mpcmmd_risk_stats_host.argtypes = [C.c_int] * 3 + [V] * 2 + [RP]
     _lib = lib
     return lib
 

@@ -15,7 +15,8 @@ different random numbers: its counts estimate what the reference's estimate, for
 Same command line as the reference, same input files (`./data/{noise}_noise/noise_{L}/ts_{np}/{cost}_{nr}_samples_{O}_obs.npz`), same output
 (`./stats/{noise}_noise/noise_{L}/ts_{np}/{nr}_samples_{O}_obs.npz` with coll_cvar, coll_cvar_lane, coll_mmd_opt, coll_mmd_opt_lane,
 coll_mmd_random, coll_mmd_random_lane; with `--rng jax` or a non-default `--num_rollouts` also rng and num_rollouts, so those counts are
-not taken for the reference's; when the mmd_opt plans carry `kernel` (driver `--kernel gaussian`), so does the stats file).  Trajectory pairs are enumerated exactly like the reference does -- `set(cvar rows) & set(mmd_opt rows)`
+not taken for the reference's; when the mmd_opt plans carry `kernel` (driver `--kernel gaussian`), so does the stats file; with `--risk`
+also each plan's Monte-Carlo risk, `risk_stats_batch`).  Trajectory pairs are enumerated exactly like the reference does -- `set(cvar rows) & set(mmd_opt rows)`
 in Python set-iteration order, position k in that order is the RNG seed of the pair (SURVEY.md Q21) -- so the per-pair draws are the same.
 """
 from __future__ import annotations
@@ -222,6 +223,114 @@ def threefry_stats_batch(prob, items, num_prime, noise_level, noise, num_obs, wa
     return (count, lane, acc, steer) if want_draws else (count, lane)
 
 
+RISK_KEYS = ("p_coll", "p_lane", "mean_obs", "var_obs", "cvar_obs")
+
+
+def _check_alpha(alpha):
+    a = float(alpha)
+    if not 0.0 <= a <= 1.0:
+        raise ValueError("alpha must lie in [0, 1], not %r" % (alpha,))
+    return a
+
+
+def _check_sigma(sigma, n):
+    """sigma as a float64 (n,) array: one Laplace bandwidth per plan (a scalar applies to every plan), each > 0 and finite"""
+    sg = np.asarray(sigma, np.float64)
+    if sg.ndim == 0:
+        sg = np.full(n, float(sg))
+    if sg.shape != (n,):
+        raise ValueError("sigma must be a scalar or have shape (%d,), not %s" % (n, sg.shape))
+    if not np.all(np.isfinite(sg) & (sg > 0)):
+        raise ValueError("sigma must be positive and finite")
+    return np.ascontiguousarray(sg)
+
+
+def _risk_struct(shape, alpha, ker_wt, sigma, costs_shape=None):
+    """(mpcmmd_risk_out, its output arrays): statistics of `shape`, per-rollout costs of costs_shape if given"""
+    out = {k: np.zeros(shape) for k in RISK_KEYS}
+    if sigma is not None:
+        out["mmd_obs"] = np.zeros(shape)
+    if costs_shape is not None:
+        out["c_obs"], out["c_lane"] = np.zeros(costs_shape), np.zeros(costs_shape)
+    p = lambda k: out[k].ctypes.data if k in out else None
+    r = B.MpcmmdRiskOut(alpha, float(ker_wt), None if sigma is None else sigma.ctypes.data, *[p(k) for k in RISK_KEYS + ("mmd_obs", "c_obs", "c_lane")])
+    return r, out
+
+
+def risk_stats_batch(prob, items, num_prime, noise_level, noise, num_obs, n_roll=NUM_ROLLOUTS, rng="host", alpha=0.98, sigma=None,
+                     want_rollout_costs=False, device=None):
+    """Monte-Carlo risk of each plan (DESIGN.md section 3 item 9): the rollouts of `compute_stats_batch` with rng="host" (NumPy's legacy
+    stream, mpcmmd_validate_risk_host) or rng="jax" (counter-based noise, mpcmmd_validate_threefry_risk_host), and per plan the collision
+    and lane probabilities (a NaN cost counts as a hit), the mean, VaR_alpha and CVaR_alpha of the obstacle cost, and with `sigma` (one
+    Laplace bandwidth per plan, or a scalar) its MMD ker_wt (E k(c, c') - 2 E k(c, 0)), ker_wt = prob.ker_wt.
+    Returns a dict: count, count_lane (as compute_stats_batch), p_coll, p_lane, mean_obs, var_obs, cvar_obs (n,) [, mmd_obs (n,)]
+    [, c_obs, c_lane (n, n_roll) per-rollout costs]."""
+    if rng == "device":
+        raise ValueError("risk_stats_batch: rng='device' has no risk statistics (its draws are NumPy's: use rng='host')")
+    if rng not in ("host", "jax"):
+        raise ValueError("risk_stats_batch: rng must be 'host' or 'jax', not %r" % (rng,))
+    if noise not in B.NOISE_KINDS:
+        raise ValueError("noise must be one of %s, not %r" % (sorted(B.NOISE_KINDS), noise))
+    if isinstance(n_roll, bool) or not isinstance(n_roll, (int, np.integer)) or n_roll < 1:
+        raise ValueError("n_roll must be an integer >= 1, not %r" % (n_roll,))
+    if int(n_roll) * int(num_prime) >= 2 ** 31:
+        raise ValueError("n_roll * num_prime must be below 2**31")
+    alpha = _check_alpha(alpha)
+    n = len(items)
+    if sigma is not None:
+        if getattr(prob, "kernel", "laplace") != "laplace":
+            raise ValueError("risk_stats_batch: the Monte-Carlo MMD is the Laplace kernel's; this handle uses kernel=%r" % (prob.kernel,))
+        sigma = _check_sigma(sigma, n)
+    seeds = _seeds(items)
+    n_roll = int(n_roll)
+    r, out = _risk_struct(n, alpha, getattr(prob, "ker_wt", 1000.0), sigma, (n, n_roll) if want_rollout_costs else None)
+    count = np.zeros(n, np.int32); lane = np.zeros(n, np.int32)
+    out.update(count=count, count_lane=lane)
+    if n == 0:
+        return out
+    acc_p, steer_p, state0, xo, yo, static = _inputs(prob, items, num_prime, num_obs)
+    dev = prob.device.index if device is None else int(device)
+    p = lambda a: None if a is None else a.ctypes.data_as(C.c_void_p)
+    geom = (float(prob.t), float(prob.wheel_base), float(prob.a_obs), float(prob.b_obs), float(prob.y_lb), float(prob.y_ub))
+    if rng == "host":
+        acc_all = np.empty((n, n_roll, num_prime)); steer_all = np.empty((n, n_roll, num_prime))
+        for i, it in enumerate(items):
+            acc_all[i], steer_all[i] = perturbed_controls(prob, acc_p[i], steer_p[i], noise_level, num_prime, noise, it["key"], n_roll)
+        B.check(B.load().mpcmmd_validate_risk_host(dev or 0, n, n_roll, num_prime, num_obs, 1 if static else 0, *geom, p(acc_all), p(steer_all),
+                                                   p(state0), p(xo), p(yo), p(count), p(lane), C.byref(r)))
+    else:
+        B.check(B.load().mpcmmd_validate_threefry_risk_host(
+            dev or 0, n, n_roll, num_prime, num_obs, 1 if static else 0, B.NOISE_KINDS[noise], float(noise_level), float(prob.cem_helper.K_steer),
+            float(prob.beta_a), float(prob.beta_b), float(prob.acc_const_noise), float(prob.steer_const_noise), *geom, p(seeds), p(acc_p),
+            p(steer_p), p(state0), p(xo), p(yo), p(count), p(lane), C.byref(r)))
+    return out
+
+
+def risk_stats(c_obs, c_lane=None, alpha=0.98, sigma=None, ker_wt=1000.0, device=0):
+    """the risk statistics of given per-rollout costs (mpcmmd_risk_stats_host): c_obs (n,) or (n_sets, n), each >= 0 and finite or NaN;
+    c_lane the same shape or None (p_lane = 0); sigma a scalar or one bandwidth per set.  Returns a dict of arrays of shape c_obs.shape[:-1]:
+    p_coll, p_lane, mean_obs, var_obs, cvar_obs [, mmd_obs]."""
+    co = np.ascontiguousarray(c_obs, np.float64)
+    if co.ndim not in (1, 2) or co.shape[-1] < 1 or co.size == 0:
+        raise ValueError("c_obs must have shape (n,) or (n_sets, n) with n >= 1, not %s" % (co.shape,))
+    if np.any(co < 0) or np.any(np.isinf(co)):
+        raise ValueError("c_obs values must be >= 0 and finite, or NaN")
+    cl = None
+    if c_lane is not None:
+        cl = np.ascontiguousarray(c_lane, np.float64)
+        if cl.shape != co.shape:
+            raise ValueError("c_lane must have the shape of c_obs %s, not %s" % (co.shape, cl.shape))
+    shape = co.shape[:-1]
+    n_sets, n = (1, co.shape[0]) if co.ndim == 1 else co.shape
+    alpha = _check_alpha(alpha)
+    if sigma is not None:
+        sigma = _check_sigma(np.reshape(sigma, -1) if np.ndim(sigma) else sigma, n_sets)
+    r, out = _risk_struct(shape, alpha, ker_wt, sigma)
+    p = lambda a: None if a is None else a.ctypes.data_as(C.c_void_p)
+    B.check(B.load().mpcmmd_risk_stats_host(int(device), n_sets, n, p(co), p(cl), C.byref(r)))
+    return out
+
+
 def _load(root, noise, noise_level, num_prime, cost, num_reduced, num_obs):
     return np.load(root + "/{}_noise/noise_{}/ts_{}/{}_{}_samples_{}_obs.npz".format(noise, int(noise_level * 100), num_prime, cost, num_reduced, num_obs))
 
@@ -256,6 +365,9 @@ def _item(d, idx, key, dynamic):
 
 
 def run_validation(args, variant="static", device=0, log=print):
+    risk = getattr(args, "risk", False)
+    if risk and args.rng not in ("host", "jax"):
+        raise ValueError("--risk needs --rng host or --rng jax (the legacy-stream device draws are NumPy's: use --rng host)")
     written = []
     dynamic = variant == "dynamic"
     for noise in args.noises:
@@ -271,8 +383,18 @@ def run_validation(args, variant="static", device=0, log=print):
                         log((len(pairs), _matrix(data_cvar, num_obs).shape[1]))                     # the reference prints eset.shape
                         # both costs of a scene share the seed k (validation.py:315-336)
                         items = [_item(data_mmd_opt, im, k, dynamic) for k, _, im in pairs] + [_item(data_cvar, ic, k, dynamic) for k, ic, _ in pairs]
-                        count, lane = compute_stats_batch(prob, items, num_prime, noise_level, noise, num_obs, n_roll=args.num_rollouts, rng=args.rng)
+                        extra = {}
+                        if risk:
+                            rs = risk_stats_batch(prob, items, num_prime, noise_level, noise, num_obs, n_roll=args.num_rollouts, rng=args.rng,
+                                                  alpha=args.risk_alpha)
+                            count, lane = rs["count"], rs["count_lane"]
+                        else:
+                            count, lane = compute_stats_batch(prob, items, num_prime, noise_level, noise, num_obs, n_roll=args.num_rollouts, rng=args.rng)
                         m = len(pairs)
+                        if risk:                                  # the same order as the coll_* arrays: pair k at position k
+                            extra["risk_alpha"] = float(args.risk_alpha)
+                            for k in RISK_KEYS:
+                                extra[k + "_cvar"], extra[k + "_mmd_opt"] = rs[k][m:], rs[k][:m]
                         f = lambda a: np.asarray(a, np.float64)                                   # np.append([], int) yields float64 arrays
                         path = "{}/{}_noise/noise_{}/ts_{}/{}_samples_{}_obs".format(args.stats_root, noise, int(noise_level * 100), num_prime, num_reduced, num_obs)
                         os.makedirs(os.path.dirname(path), exist_ok=True)
@@ -281,7 +403,7 @@ def run_validation(args, variant="static", device=0, log=print):
                         if "kernel" in data_mmd_opt.files:                                        # plans made with a non-reference MMD kernel
                             tag["kernel"] = str(data_mmd_opt["kernel"])
                         np.savez(path, coll_cvar=f(count[m:]), coll_cvar_lane=f(lane[m:]), coll_mmd_opt=f(count[:m]), coll_mmd_opt_lane=f(lane[:m]),
-                                 coll_mmd_random=[], coll_mmd_random_lane=[], **tag)
+                                 coll_mmd_random=[], coll_mmd_random_lane=[], **tag, **extra)
                         written.append(path + ".npz")
                         del prob
     return written
@@ -305,7 +427,18 @@ def build_parser():
                         "rollout on the GPU (same distributions, not the reference's numbers)")
     p.add_argument("--num_rollouts", type=_positive_int, default=NUM_ROLLOUTS,
                    help="noisy rollouts per planned trajectory (default %d, the reference's _num_batch)" % NUM_ROLLOUTS)
+    p.add_argument("--risk", action="store_true",
+                   help="also write each plan's Monte-Carlo risk: p_coll_*, p_lane_*, mean_obs_*, var_obs_*, cvar_obs_* and risk_alpha "
+                        "(needs --rng host or jax)")
+    p.add_argument("--risk_alpha", type=_unit_float, default=0.98, help="VaR / CVaR level of --risk (default 0.98, the solver's alpha_quant)")
     return p
+
+
+def _unit_float(s):
+    v = float(s)
+    if not 0.0 <= v <= 1.0:
+        raise argparse.ArgumentTypeError("must lie in [0, 1], not %s" % s)
+    return v
 
 
 def _positive_int(s):
@@ -316,7 +449,10 @@ def _positive_int(s):
 
 
 def main(argv=None, variant=None):
-    args = build_parser().parse_args(argv)
+    parser = build_parser()
+    args = parser.parse_args(argv)
+    if args.risk and args.rng == "device":
+        parser.error("--risk needs --rng host or --rng jax")
     run_validation(args, variant or args.variant)
 
 
