@@ -29,7 +29,8 @@ extern "C" {
 #define MPCMMD_NVAR 11    /* nvar  (cem.py:50)  Bernstein coefficients */
 #define MPCMMD_NPARAM 8   /* num_params (cem.py:136) */
 #define MPCMMD_MAX_NR 10  /* largest num_reduced of the mmd_opt reduced-set kernels with shared-memory chain state */
-#define MPCMMD_MAX_NR_OPT 40  /* largest num_reduced of mmd_opt (11..40: chain state in global memory, k_inner_cem_big); cvar / saa / mmd_random take up to 64 */
+#define MPCMMD_MAX_NR_OPT 40  /* largest num_reduced of mmd_opt (11..40: chain state in global memory, k_inner_cem_big) */
+#define MPCMMD_MAX_NR_WIDE 1024  /* largest num_reduced of cvar / saa / mmd_random (2..64: warp-wide risk per sample; 65..1024: one CTA per sample, k_rollouts_wide) */
 
 enum { MPCMMD_COST_MMD_OPT = 0, MPCMMD_COST_MMD_RANDOM = 1, MPCMMD_COST_CVAR = 2, MPCMMD_COST_SAA = 3 };
 enum { MPCMMD_NOISE_GAUSSIAN = 0, MPCMMD_NOISE_BETA = 1 };

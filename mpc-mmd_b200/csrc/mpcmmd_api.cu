@@ -21,6 +21,7 @@
 #include "k_validate_noise.cuh"
 #include "k_validate_jax.cuh"
 #include "k_risk_stats.cuh"
+#include "k_risk_wide.cuh"
 
 static thread_local std::string g_err;
 static int fail(const std::string& m) { g_err = m; return -1; }
@@ -75,6 +76,12 @@ struct mpcmmd_handle_s {
     int groups_override = 0;                 // MPCMMD_GROUPS=1..8: force the number of episode groups of a solve graph (0 = automatic)
 };
 
+// num_reduced above the warp paths' bound: cvar / saa / mmd_random run k_rollouts_wide (one CTA per sample), and the noise tables hold one outer
+// iteration per episode, drawn at the start of each iteration by k_noise_wide (see enqueue_solve)
+static bool is_wide(const DCfg& d) { return d.nr > MPCMMD_MAX_NR_DEV; }
+// outer iterations of z1 / z2 / z3 / keys / btab the workspace holds per episode
+static size_t noise_slots(const DCfg& d) { return is_wide(d) ? 1 : (size_t)d.iters; }
+
 // ---- episode-offset view of a handle's workspace: every per-episode array advanced by e0 episodes.  A solve graph can then enqueue disjoint episode
 // ranges on different streams with the unchanged launch code (episodes are independent; sample index g and episode index e stay relative to the view).
 struct ViewSave { DWork w; float *beq_x, *beq_y, *state0, *feat, *ctrl, *bscratch, *rolls_x, *rolls_y, *xroll, *mrisk; int* ridx; };
@@ -82,12 +89,12 @@ static ViewSave push_view(mpcmmd_handle_s* h, int e0) {
     ViewSave sv = {h->w, h->beq_x, h->beq_y, h->state0, h->feat, h->ctrl, h->bscratch, h->rolls_x, h->rolls_y, h->xroll, h->mrisk, h->ridx};
     if (e0 == 0) return sv;
     const DCfg& d = h->d; DWork& w = h->w;
-    const size_t e = (size_t)e0, B = d.B, n = (size_t)d.nr * d.np, ncem = (size_t)(d.B - d.n_el) * NPAR, it = d.iters;
+    const size_t e = (size_t)e0, B = d.B, n = (size_t)d.nr * d.np, ncem = (size_t)(d.B - d.n_el) * NPAR, it = d.iters, zs = noise_slots(d);
 #define ADV(p, stride) if (p) p += e * (stride)
     ADV(w.params, B * NPAR); ADV(w.lam_x, B * NV); ADV(w.lam_y, B * NV); ADV(w.s_lane, B * 2 * NL); ADV(w.mean, NPAR); ADV(w.cov, 64);
     ADV(w.cx, B * NV); ADV(w.cy, B * NV); ADV(w.res_norm, B); ADV(w.cost_base, B); ADV(w.acc, B * T_); ADV(w.steer, B * T_); ADV(w.risk, B); ADV(w.lane, B);
-    ADV(w.beta, B * d.nr); ADV(w.sigma, B); ADV(w.res_beta, B * d.iters_in); ADV(w.z1, it * n); ADV(w.z2, it * n); ADV(w.z3, it * n); ADV(w.zcem, it * ncem);
-    ADV(w.keys, it * 4); ADV(w.btab, it * 4 * GT_FIELDS * n); ADV(w.idx_mpc, 1); ADV(w.init_state, 6); ADV(w.mean0, NPAR); ADV(w.cov0, 64);
+    ADV(w.beta, B * d.nr); ADV(w.sigma, B); ADV(w.res_beta, B * d.iters_in); ADV(w.z1, zs * n); ADV(w.z2, zs * n); ADV(w.z3, zs * n); ADV(w.zcem, it * ncem);
+    ADV(w.keys, zs * 4); ADV(w.btab, zs * 4 * GT_FIELDS * n); ADV(w.idx_mpc, 1); ADV(w.init_state, 6); ADV(w.mean0, NPAR); ADV(w.cov0, 64);
     ADV(w.x_obs, (size_t)d.O * T_); ADV(w.y_obs, (size_t)d.O * T_); ADV(w.v_des, 1);
     ADV(w.sx_obs, (size_t)d.O * T_); ADV(w.sy_obs, (size_t)d.O * T_); ADV(w.obs_nan, T_);
     ADV(w.o_cx, NV); ADV(w.o_cy, NV); ADV(w.o_lane, 1); ADV(w.o_obs, 1); ADV(w.o_beta, d.nr); ADV(w.o_sigma, 1); ADV(w.o_res_beta, d.iters_in); ADV(w.o_sel, it);
@@ -178,6 +185,13 @@ static const void* rollouts_kernel(int mode, int nz, int sorted, int ov = OV_PLA
     return RK_NZ(ROLL_FLY, false, OV_PLAIN);
 #undef RK_NZ
 }
+// k_rollouts_wide instantiation of a launch (num_reduced > 64): noise path (NZ_*), sorted obstacle windows
+static const void* rollouts_wide_kernel(int nz, int sorted) {
+#define RW_NZ(S) (nz == NZ_GAUSS ? (const void*)k_rollouts_wide<WIDE_THREADS, S, NZ_GAUSS> : nz == NZ_BETA_TABLE ? (const void*)k_rollouts_wide<WIDE_THREADS, S, NZ_BETA_TABLE> \
+                                                                                           : (const void*)k_rollouts_wide<WIDE_THREADS, S, NZ_ANY>)
+    return sorted ? RW_NZ(true) : RW_NZ(false);
+#undef RW_NZ
+}
 typedef void (*inner_cem_fn)(DCfg, RollArgs);
 // inner-CEM kernels of mmd_opt.  The k_inner_cem_fast family (one CTA per chain, num_reduced <= 5): CTA (throughput build), CTA_LAT (its latency build),
 // CTA_FASTMATH (MPCMMD_MATH=fast) and LAT512 (k_inner_cem_lat, 16 warps per chain); these leave the chosen reduced set to k_opt_risk.  GENERIC (k_inner_cem,
@@ -264,7 +278,7 @@ extern "C" int mpcmmd_create_with_kernel(const mpcmmd_config* cfg, int mmd_kerne
     if (B < cfg->ellite_num_cost || cfg->ellite_num_cost > 32 || cfg->ellite_num > 8 || cfg->ellite_num > cfg->ellite_num_cost)
         return fail("mpcmmd_create: need ellite_num <= 8, ellite_num <= ellite_num_cost <= min(32, num_batch)");
     if (np < 2 || np > MPCMMD_T) return fail("mpcmmd_create: num_prime must be in [2,100]");
-    if (nr < 2 || nr > MPCMMD_MAX_NR_DEV) return fail("mpcmmd_create: num_reduced must be in [2,64] (mmd_opt: 2..40)");
+    if (nr < 2 || nr > MPCMMD_MAX_NR_WIDE) return fail("mpcmmd_create: num_reduced must be in [2,1024] (mmd_opt: 2..40)");
     if (cfg->num_obs < 1 || E < 1) return fail("mpcmmd_create: num_obs and max_episodes must be >= 1");
     if (cfg->num_obs > MPCMMD_MAX_NR_DEV) return fail("mpcmmd_create: num_obs must be <= 64");
     if (cfg->num_samples_cem > RISKO_THREADS * 8 || cfg->num_ellite_beta < 2 || cfg->num_ellite_beta >= cfg->num_samples_cem)
@@ -341,9 +355,10 @@ static int create_body(mpcmmd_handle_s* h, const mpcmmd_config* cfg, int device)
     AL(params, EB * NPAR) AL(lam_x, EB * NV) AL(lam_y, EB * NV) AL(s_lane, EB * 2 * NL) AL(mean, (size_t)E * NPAR) AL(cov, (size_t)E * 64)
     AL(cx, EB * NV) AL(cy, EB * NV) AL(res_norm, EB) AL(cost_base, EB) AL(acc, EB * T_) AL(steer, EB * T_) AL(risk, EB) AL(lane, EB)
     AL(beta, EB * nr) AL(sigma, EB) AL(res_beta, EB * d.iters_in)
-    AL(z1, (size_t)E * d.iters * n) AL(z2, (size_t)E * d.iters * n) AL(z3, (size_t)E * d.iters * n) AL(zcem, (size_t)E * d.iters * ncem)
-    AL(keys, (size_t)E * d.iters * 4)
-    if (d.noise_kind == 1) { AL(btab, (size_t)E * d.iters * 4 * GT_FIELDS * n) } else w.btab = nullptr;
+    const size_t zs = noise_slots(d);
+    AL(z1, (size_t)E * zs * n) AL(z2, (size_t)E * zs * n) AL(z3, (size_t)E * zs * n) AL(zcem, (size_t)E * d.iters * ncem)
+    AL(keys, (size_t)E * zs * 4)
+    if (d.noise_kind == 1) { AL(btab, (size_t)E * zs * 4 * GT_FIELDS * n) } else w.btab = nullptr;
     AL(idx_mpc, E) AL(init_state, (size_t)E * 6) AL(mean0, (size_t)E * NPAR) AL(cov0, (size_t)E * 64)
     AL(x_obs, (size_t)E * d.O * T_) AL(y_obs, (size_t)E * d.O * T_) AL(v_des, E)
     if (d.O > OBS_SORT_MIN) { AL(sx_obs, (size_t)E * d.O * T_) AL(sy_obs, (size_t)E * d.O * T_) AL(obs_nan, (size_t)E * T_) } else { w.sx_obs = w.sy_obs = nullptr; w.obs_nan = nullptr; }
@@ -351,12 +366,14 @@ static int create_body(mpcmmd_handle_s* h, const mpcmmd_config* cfg, int device)
     AL(o_res_beta, (size_t)E * d.iters_in) AL(o_sel, (size_t)E * d.iters)
 #undef AL
     if (dalloc(h, &h->beq_x, (size_t)E * 3) || dalloc(h, &h->beq_y, (size_t)E * 4) || dalloc(h, &h->state0, (size_t)E * 5)) return -1;
-    // constant normal tables [survey Q8]: every key below derives from PRNGKey(0) only
+    // constant normal tables [survey Q8]: every key below derives from PRNGKey(0) only.  Handles with num_reduced > 64 (no mmd_opt) build only z_init:
+    // the inner-CEM tables have d = num_reduced^2 + 1 columns (about 16 GB at num_reduced 1024)
     {
         const int S = d.S_in, dd = nm + 1, ne = d.n_el_in;
-        float *z_init, *theta0, *zb, *ztmp;
-        if (dalloc(h, &z_init, (size_t)B * NPAR) || dalloc(h, &theta0, (size_t)S * dd) || dalloc(h, &zb, (size_t)d.iters_in * (S - ne) * dd) ||
-            dalloc(h, &ztmp, (size_t)S * dd)) return -1;
+        const bool inner = !is_wide(d);
+        float *z_init, *theta0 = nullptr, *zb = nullptr, *ztmp = nullptr;
+        if (dalloc(h, &z_init, (size_t)B * NPAR)) return -1;
+        if (inner && (dalloc(h, &theta0, (size_t)S * dd) || dalloc(h, &zb, (size_t)d.iters_in * (S - ne) * dd) || dalloc(h, &ztmp, (size_t)S * dd))) return -1;
         // host-side key derivation mirrors the device functions (integer-only Threefry)
         auto tf = [](uint32_t k0, uint32_t k1, uint32_t x0, uint32_t x1, uint32_t* o) {
             auto rotl = [](uint32_t x, int r) { return (x << r) | (x >> (32 - r)); };
@@ -373,28 +390,35 @@ static int create_body(mpcmmd_handle_s* h, const mpcmmd_config* cfg, int device)
         uint32_t key_init[2] = {0u, 0u};
         split0(key_init);                                                         // cem_helper.py:125 / compute_beta.py:108
         k_normal_table<<<64, 256>>>(key_init[0], key_init[1], B * NPAR, z_init);
-        uint32_t kk[2] = {key_init[0], key_init[1]};
-        split0(kk);                                                               // compute_beta.py:44
-        k_normal_table<<<64, 256>>>(kk[0], kk[1], S * dd, ztmp);
-        k_theta0<<<64, 256>>>(ztmp, S, dd, d.sigma_clip, theta0);
-        uint32_t carry[2] = {key_init[0], key_init[1]};
-        for (int it = 0; it < d.iters_in; it++) {
-            split0(carry);                                                        // compute_beta.py:131
-            uint32_t dk[2] = {carry[0], carry[1]};
-            split0(dk);                                                           // compute_beta.py:54
-            k_normal_table<<<64, 256>>>(dk[0], dk[1], (S - ne) * dd, zb + (size_t)it * (S - ne) * dd);
+        d.z_init = z_init; d.theta0 = d.zb_iter = d.zb_iterT = nullptr;
+        if (inner) {
+            uint32_t kk[2] = {key_init[0], key_init[1]};
+            split0(kk);                                                           // compute_beta.py:44
+            k_normal_table<<<64, 256>>>(kk[0], kk[1], S * dd, ztmp);
+            k_theta0<<<64, 256>>>(ztmp, S, dd, d.sigma_clip, theta0);
+            uint32_t carry[2] = {key_init[0], key_init[1]};
+            for (int it = 0; it < d.iters_in; it++) {
+                split0(carry);                                                    // compute_beta.py:131
+                uint32_t dk[2] = {carry[0], carry[1]};
+                split0(dk);                                                       // compute_beta.py:54
+                k_normal_table<<<64, 256>>>(dk[0], dk[1], (S - ne) * dd, zb + (size_t)it * (S - ne) * dd);
+            }
+            float* zbT;
+            if (dalloc(h, &zbT, (size_t)d.iters_in * (S - ne) * dd)) return -1;
+            k_transpose_tables<<<64, 256>>>(zb, zbT, d.iters_in, S - ne, dd);
+            d.theta0 = theta0; d.zb_iter = zb; d.zb_iterT = zbT;
         }
-        float* zbT;
-        if (dalloc(h, &zbT, (size_t)d.iters_in * (S - ne) * dd)) return -1;
-        k_transpose_tables<<<64, 256>>>(zb, zbT, d.iters_in, S - ne, dd);
-        d.z_init = z_init; d.theta0 = theta0; d.zb_iter = zb; d.zb_iterT = zbT;
     }
     // opt-in shared memory sizes (raise-only per (device, kernel): see raise_smem)
     cudaDeviceGetAttribute(&h->sm_count, cudaDevAttrMultiProcessorCount, device);
     if (h->sm_count < 1) h->sm_count = 1;
     if (raise_smem(device, (const void*)k_project, PROJ_SMEM_BYTES)) return fail("k_project smem opt-in failed");
     if (raise_smem(device, (const void*)k_project_tc, ptc::SMEM_BYTES, true)) return fail("k_project_tc smem opt-in failed");
-    {
+    if (is_wide(d)) {
+        const size_t ws = (size_t)wide_layout(nr).total * sizeof(float);
+        for (int so = 0; so < 2; so++) for (int nz = 0; nz < 3; nz++)
+            if (raise_smem(device, rollouts_wide_kernel(nz, so), ws)) return fail("k_rollouts_wide smem opt-in failed");
+    } else {
         size_t rs = nr <= MPCMMD_MAX_NR_OPT ? roll_smem(h, MPCMMD_COST_MMD_OPT) : 0; const size_t rb = roll_smem(h, MPCMMD_COST_CVAR); if (rb > rs) rs = rb;
         if (rs > 227 * 1024) return fail("mpcmmd_create: rollouts of one sample do not fit in shared memory");
         for (int mode = 0; mode < 3; mode++) for (int nz = 0; nz < 3; nz++) for (int so = 0; so < 2; so++) for (int ov = 0; ov < 3; ov++) {
@@ -487,6 +511,16 @@ static int launch_risk(mpcmmd_handle_s* h, const RiskArgs& r, cudaStream_t s, in
     const DCfg& d = h->d;
     const bool opt = r.cost_kind == MPCMMD_COST_MMD_OPT;
     if (r.n_samples > h->E * d.B) return fail("risk stage: more samples than the workspace holds (max_episodes * num_batch)");
+    if (is_wide(d)) {                       // num_reduced 65..1024 (cvar / saa / mmd_random; mmd_opt is refused before it gets here): one CTA per sample
+        if (opt) return fail("mmd_opt: num_reduced must be in [2, 40] (larger reduced sets: cvar / saa / mmd_random only)");
+        const int nz = d.noise_kind == 0 ? NZ_GAUSS : (r.btab && !r.binj1) ? NZ_BETA_TABLE : NZ_ANY;
+        RiskArgs ra = r;
+        void* kargs[] = {(void*)&d, (void*)&ra};
+        CK(cudaLaunchKernel(rollouts_wide_kernel(nz, r.sx_obs != nullptr), dim3(r.n_samples), dim3(WIDE_THREADS), kargs,
+                            (size_t)wide_layout(d.nr).total * sizeof(float), s));
+        if (n_launch) *n_launch = 1;
+        return 0;
+    }
     RollArgs ra;
     ra.r = r; ra.spb = roll_spb(h, r.cost_kind, r.n_samples); ra.R = opt ? d.nm : d.nr; ra.xroll = h->xroll; ra.yroll = h->yroll; ra.feat = h->feat; ra.ridx = h->ridx; ra.bscratch = h->bscratch; ra.ctrl = h->ctrl; ra.write_rolls = 0; ra.fold_risk = 0; ra.mrisk = h->mrisk; ra.stage_ctrl = roll_stage_ctrl(h, r.cost_kind, r.n_samples);
     inner_cem_fn f = nullptr;
@@ -556,16 +590,22 @@ static int enqueue_solve(mpcmmd_handle_s* h, int kind, int n_ep, cudaStream_t s,
     auto mark = [&](int cls) { cnt++; if (marks) { LaunchMark m; cudaEventCreate(&m.ev); cudaEventRecord(m.ev, s); m.cls = cls; marks->push_back(m); } };
     k_boundary<<<(n_ep + 127) / 128, 128, 0, s>>>(w.init_state, h->beq_x, h->beq_y, h->state0, n_ep); mark(0);
     if (w.sx_obs) { k_obs_sort<<<(n_ep * T_ + 127) / 128, 128, 0, s>>>(w.x_obs, w.y_obs, w.sx_obs, w.sy_obs, w.obs_nan, d.O, n_ep * T_); mark(0); }
-    k_noise<<<n_ep * d.iters, d.B <= SEL_RANK_MAX ? 128 : 1024, 0, s>>>(d, w, n_ep, 0, d.iters); mark(0);
+    const bool wide = is_wide(d);
+    if (!wide) { k_noise<<<n_ep * d.iters, d.B <= SEL_RANK_MAX ? 128 : 1024, 0, s>>>(d, w, n_ep, 0, d.iters); mark(0); }
     k_init<<<n_ep, d.B <= SEL_RANK_MAX ? 128 : 1024, 0, s>>>(d, w, n_ep); mark(0);
     for (int it = 0; it < d.iters; it++) {
+        if (wide) {                         // this iteration's tables, after the previous iteration's rollouts have read theirs (same stream)
+            const int chunks = noise_wide_chunks(d);
+            k_noise_wide<<<n_ep * chunks, NOISE_WIDE_THREADS, 0, s>>>(d, w, it, chunks); mark(0);
+        }
         ProjArgs p = proj_args(h, n_ep);
         launch_project(h, p, s); mark(1);
         RiskArgs r;
         r.n_samples = n_ep * d.B; r.B = d.B; r.cost_kind = kind; r.acc = w.acc; r.steer = w.steer; r.state0 = h->state0;
-        r.z1 = w.z1 + it * n; r.z2 = w.z2 + it * n; r.z3 = w.z3 + it * n; r.z_stride = (size_t)d.iters * n;
-        r.keys = w.keys + it * 4; r.key_stride = (size_t)d.iters * 4;
-        r.btab = w.btab ? w.btab + (size_t)it * 4 * GT_FIELDS * n : nullptr; r.btab_stride = (size_t)d.iters * 4 * GT_FIELDS * n; r.binj1 = r.binj2 = nullptr;
+        const int zi = wide ? 0 : it;      // slot of this iteration's noise tables within an episode
+        r.z1 = w.z1 + zi * n; r.z2 = w.z2 + zi * n; r.z3 = w.z3 + zi * n; r.z_stride = noise_slots(d) * n;
+        r.keys = w.keys + zi * 4; r.key_stride = noise_slots(d) * 4;
+        r.btab = w.btab ? w.btab + (size_t)zi * 4 * GT_FIELDS * n : nullptr; r.btab_stride = noise_slots(d) * 4 * GT_FIELDS * n; r.binj1 = r.binj2 = nullptr;
         r.x_obs = w.x_obs; r.y_obs = w.y_obs; r.sx_obs = w.sx_obs; r.sy_obs = w.sy_obs; r.obs_nan = w.obs_nan; r.risk = w.risk; r.lane = w.lane; r.beta = w.beta; r.sigma = w.sigma; r.res_beta = w.res_beta;
         int nl = 0;
         if (launch_risk(h, r, s, &nl)) return -1;
@@ -578,6 +618,7 @@ static int enqueue_solve(mpcmmd_handle_s* h, int kind, int n_ep, cudaStream_t s,
         a.o_sigma = w.o_sigma; a.o_res_beta = w.o_res_beta; a.o_sel = w.o_sel; a.sel_stride = d.iters;
         k_select<<<n_ep, d.B <= SEL_RANK_MAX ? SEL_THREADS : SEL_THREADS_BIG, sel_smem(d), s>>>(d, a); mark(3);
     }
+    if (wide) { k_wide_beta_out<<<n_ep, 256, 0, s>>>(d.nr, d.B, d.iters, w.beta, w.o_sel, w.o_beta); mark(3); }
     *launches = cnt;
     return 0;
 }
@@ -754,6 +795,8 @@ extern "C" int mpcmmd_get_tables(mpcmmd_handle h, float* z_init, float* theta0, 
     if (!h) return fail("null handle");
     CK(cudaSetDevice(h->device));
     const DCfg& d = h->d; const int dd = d.nm + 1;
+    if (is_wide(d) && (theta0 || zb_iter))
+        return fail("mpcmmd_get_tables: a handle with num_reduced > 64 has no inner-CEM tables (theta0, zb_iter: mmd_opt only, num_reduced <= 40)");
     if (z_init) CK(cudaMemcpy(z_init, d.z_init, sizeof(float) * d.B * NPAR, cudaMemcpyDeviceToDevice));
     if (theta0) CK(cudaMemcpy(theta0, d.theta0, sizeof(float) * d.S_in * dd, cudaMemcpyDeviceToDevice));
     if (zb_iter) CK(cudaMemcpy(zb_iter, d.zb_iter, sizeof(float) * d.iters_in * (d.S_in - d.n_el_in) * dd, cudaMemcpyDeviceToDevice));
@@ -844,13 +887,14 @@ extern "C" int mpcmmd_stage_noise(mpcmmd_handle h, int32_t idx_mpc, int32_t iter
     const size_t n = (size_t)d.nr * d.np, ncem = (size_t)(d.B - d.n_el) * NPAR;
     CK(cudaMemcpy(w.idx_mpc, &idx_mpc, sizeof(int32_t), cudaMemcpyHostToDevice));
     DCfg dg = d; dg.noise_kind = 0;                                  // always emit the Gaussian tables here
-    k_noise<<<1, 128>>>(dg, w, 1, iter, 1);
+    if (is_wide(d)) { const int chunks = noise_wide_chunks(dg); k_noise_wide<<<chunks, NOISE_WIDE_THREADS>>>(dg, w, iter, chunks); }
+    else k_noise<<<1, 128>>>(dg, w, 1, iter, 1);
     CK(cudaDeviceSynchronize());
-    const size_t slot = (size_t)iter;
+    const size_t slot = is_wide(d) ? 0 : (size_t)iter;
     if (z1) CK(cudaMemcpy(z1, w.z1 + slot * n, sizeof(float) * n, cudaMemcpyDeviceToDevice));
     if (z2) CK(cudaMemcpy(z2, w.z2 + slot * n, sizeof(float) * n, cudaMemcpyDeviceToDevice));
     if (z3) CK(cudaMemcpy(z3, w.z3 + slot * n, sizeof(float) * n, cudaMemcpyDeviceToDevice));
-    if (z_cem) CK(cudaMemcpy(z_cem, w.zcem + slot * ncem, sizeof(float) * ncem, cudaMemcpyDeviceToDevice));
+    if (z_cem) CK(cudaMemcpy(z_cem, w.zcem + (size_t)iter * ncem, sizeof(float) * ncem, cudaMemcpyDeviceToDevice));
     if (keys) CK(cudaMemcpy(keys, w.keys + slot * 4, sizeof(uint32_t) * 4, cudaMemcpyDeviceToDevice));
     return 0;
 }

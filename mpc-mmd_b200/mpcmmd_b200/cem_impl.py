@@ -44,7 +44,9 @@ class CEM:
     optimizer/ copies to mirror), `max_episodes` (workspace capacity of `solve_batch`), `device`,
     `num_batch` / `maxiter_cem` overrides for scaled or reduced runs, `kernel` ("laplace" as the reference, or
     "gaussian"): the kernel of the MMD risk costs of mmd_opt and mmd_random, fixed for the object's lifetime
-    (DESIGN.md section 3 items 4 and 8)."""
+    (DESIGN.md section 3 items 4 and 8).
+    `num_reduced` is 2..1024 for cvar, saa and mmd_random (above 64 one CTA per sample finishes the risk) and 2..40 for mmd_opt, whose
+    solves and stages refuse larger sets; `tables()` (the mmd_opt inner-CEM tables) is refused above 64."""
 
     def __init__(self, num_reduced, num_obs, noise_level, num_prime, noise, acc_const_noise, steer_const_noise, *,
                  variant="static", max_episodes=1, device=0, num_batch=100, maxiter_cem=20,
