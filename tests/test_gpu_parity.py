@@ -3,6 +3,8 @@
 The arithmetic contract (DESIGN.md section 3) makes every float32 result reproducible, so the bar
 here is `np.array_equal`, which is stricter than the 1e-4 relative tolerance north_star asks for
 (and implies identical elite index sets and identical downstream collision counts)."""
+import os
+
 import numpy as np
 import pytest
 
@@ -577,17 +579,31 @@ def test_solve_scaled_batch_bit_exact(mods, cost, noise, B, kw):
             _eq(got[k][e], ref[k], f"B={B} {cost} ep{e} {k}")
 
 
-@pytest.mark.parametrize("cost,nobs,special", [("cvar", 32, "plain"), ("cvar", 32, "nan_obstacle"), ("mmd_random", 20, "moving"), ("mmd_opt", 32, "edge"),
-                                               ("cvar", 64, "plain")])
-def test_stage_risk_many_obstacles_sorted_window(mods, cost, nobs, special):
-    """num_obs > 8 (configs[4]: 32 obstacles): the rollouts look only at the obstacles inside an x window around the vehicle, found by binary search in the
-    per-knot sorted obstacle lists of k_obs_sort.  Skipped obstacles contribute exactly 0, so the result must equal the oracle's all-pairs maximum bit for bit --
-    with static and moving obstacles, with obstacles placed right at the window edge (|dx| = a_obs +- ulps), and with a NaN obstacle coordinate (plain-loop fallback)."""
+_SORTED_WINDOW_CASES = [("cvar", 32, "plain"), ("cvar", 32, "nan_obstacle"), ("mmd_random", 20, "moving"), ("mmd_opt", 32, "edge"), ("cvar", 64, "plain")]
+
+
+@pytest.mark.parametrize("cost,nobs,special,size", [pytest.param(*c, "staged", id="-".join(map(str, c))) for c in _SORTED_WINDOW_CASES]
+                         + [pytest.param(*c, "fly", id="-".join(map(str, c)) + "-fly") for c in _SORTED_WINDOW_CASES if c[0] != "mmd_opt"]
+                         + [pytest.param("cvar", 32, "edge", "fly", id="cvar-32-edge-fly")])
+def test_stage_risk_many_obstacles_sorted_window(mods, cost, nobs, special, size):
+    """num_obs > 8 (configs[4]: 32 obstacles).  Which kernel reads the obstacles depends on the launch size: cvar / mmd_random launches of fewer
+    than 2 * SMs * 128 rollouts ("staged": 24 samples) run k_rollouts<ROLL_STAGED>, whose plain loop visits every obstacle; larger ones ("fly":
+    just above that) run k_rollouts<ROLL_FLY, SORTED>, which looks only at the obstacles inside an x window around the vehicle, found by binary
+    search in the per-knot sorted obstacle lists of k_obs_sort.  mmd_opt re-rolls its chosen reduced set in k_opt_risk<true>, which searches the
+    window at any size.  Skipped obstacles contribute exactly 0, so the result must equal the oracle's all-pairs maximum bit for bit -- with static
+    and moving obstacles, with obstacles placed right at the window edge (|dx| = a_obs +- ulps), and with a NaN obstacle coordinate (plain-loop
+    fallback).  The kernel each size runs is asserted from the profiler's kernel records."""
+    import torch
+    import kernel_names as KN
     kw = dict(num_samples_cem=40, maxiter_beta_cem=3) if cost == "mmd_opt" else {}
-    prob, ora = _pair(mods, (5, nobs, 0.1, 60, "gaussian", 0.02, 0.01), max_episodes=1, **kw)
+    thr = 2 * torch.cuda.get_device_properties(0).multi_processor_count * 128          # rollouts of the smallest ROLL_FLY launch
+    n = 6 if cost == "mmd_opt" else 24 if size == "staged" else -(-thr // 5) + 7
+    prob, ora = _pair(mods, (5, nobs, 0.1, 60, "gaussian", 0.02, 0.01), max_episodes=-(-n // 100), **kw)
     rng = np.random.default_rng(300 + nobs)
-    n = 24 if cost != "mmd_opt" else 6
-    acc, steer = _controls(ora, rng, n)
+    acc, steer = _controls(ora, rng, min(n, 24))
+    if n > 24:                                                    # scaled copies of the 24 projected control sequences
+        pick = rng.integers(0, 24, n); pick[0] = 0
+        acc = (acc[pick] * rng.uniform(0.5, 1.5, (n, 1))).astype(f32); steer = (steer[pick] * rng.uniform(0.5, 1.5, (n, 1))).astype(f32)
     st0 = np.array([0.0, 1.75, 5.0, 0.0, 0.0], f32)
     noise_t = ora.noise_tables(91, 4)
     t = np.linspace(0.0, 15.0, 100).astype(f32)
@@ -601,10 +617,15 @@ def test_stage_risk_many_obstacles_sorted_window(mods, cost, nobs, special):
             xo[j, :] = xe; yo[j, :] = 1.75
     if special == "nan_obstacle":
         xo[3, 17] = np.nan; yo[5, 40] = np.nan
-    got = prob.stage_risk(cost, acc, steer, st0, noise_t, xo, yo)
-    for i in range(n):
-        ref = ora.risk(cost, acc[i], steer[i], st0, noise_t, xo, yo)
-        _eq(got["risk"][i], ref["risk"], f"{special} risk[{i}]"); _eq(got["lane"][i], ref["lane"], f"{special} lane[{i}]")
+    want = "k_opt_risk<true>" if cost == "mmd_opt" else "k_rollouts<2, false, 0, 0>" if size == "staged" else "k_rollouts<1, true, 0, 0>"
+    got, names = KN.launched(lambda: prob.stage_risk(cost, acc, steer, st0, noise_t, xo, yo))
+    assert want in KN.family(names), (size, want, sorted(KN.family(names)))
+    idx = range(n) if n <= 24 or cost == "cvar" else sorted(set(range(0, n, 53)) | {n - 1})
+    from concurrent.futures import ThreadPoolExecutor
+    with ThreadPoolExecutor(max_workers=max(1, min(len(idx), os.cpu_count() or 1))) as ex:
+        refs = dict(zip(idx, ex.map(lambda i: ora.risk(cost, acc[i], steer[i], st0, noise_t, xo, yo), idx)))
+    for i, ref in refs.items():
+        _eq(got["risk"][i], ref["risk"], f"{special} {size} risk[{i}]"); _eq(got["lane"][i], ref["lane"], f"{special} {size} lane[{i}]")
     if special != "nan_obstacle":
         assert np.isfinite(got["risk"]).all() and np.any(got["risk"] != got["risk"][0])
 
