@@ -901,175 +901,73 @@ extern "C" int mpcmmd_stage_noise(mpcmmd_handle h, int32_t idx_mpc, int32_t iter
 
 // ------------------------------------------------------------------------------------------------
 // Monte-Carlo validation (S/validation.py:134-171): host arrays in, counts out.  Not tied to a handle.
-// k_validate on device arrays: the rollout + counting half shared by both validation entry points (enqueue only).
-static cudaError_t launch_validate(int n_ep, int n_roll, int num_prime, int num_obs, int obs_cost_f32, double dt, double wheel_base, double a_obs,
-                                   double b_obs, double y_lb, double y_ub, size_t smem, const double* d_acc, const double* d_steer,
-                                   const double* d_s0, const double* d_xo, const double* d_yo, int32_t* d_cnt, int32_t* d_lane,
-                                   double* d_xr, double* d_yr) {
-    if (smem > 48 * 1024) {
-        const cudaError_t e = cudaFuncSetAttribute(k_validate<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return e;
+
+// The device buffers of one validation call, freed when the call returns, refused or not.  alloc / upload take counts of T and refuse
+// as CK does (the message names cudaMalloc or cudaMemcpy and the CUDA error).
+struct DeviceBuffers {
+    std::vector<void*> held;
+    DeviceBuffers() = default;
+    DeviceBuffers(const DeviceBuffers&) = delete;
+    DeviceBuffers& operator=(const DeviceBuffers&) = delete;
+    ~DeviceBuffers() { for (void* p : held) cudaFree(p); }
+    template <class T> int alloc(T** d, size_t n) {
+        CK(cudaMalloc(d, n * sizeof(T)));
+        held.push_back(*d);
+        return 0;
     }
+    template <class T> int upload(T** d, const T* h, size_t n) {
+        if (alloc(d, n)) return -1;
+        CK(cudaMemcpy(*d, h, n * sizeof(T), cudaMemcpyHostToDevice));
+        return 0;
+    }
+};
+
+// The checks every validation entry point fn shares, each refusal naming fn: a CUDA device and the index (val_device), the sizes
+// (val_sizes), then -- after fn's own argument checks -- the (num_obs + 2) * num_prime shared-memory counters, whose bytes go to smem,
+// and cudaSetDevice (val_open).
+static int val_device(const char* fn, int device) {
+    int ndev = 0;
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) return fail(std::string(fn) + ": no CUDA device (this library has no CPU fallback)");
+    if (device < 0 || device >= ndev) return fail(std::string(fn) + ": bad device index");
+    return 0;
+}
+static int val_sizes(const char* fn, int n_ep, int n_roll, int num_prime, int num_obs) {
+    if (n_ep < 1 || n_roll < 1 || num_prime < 1 || num_prime > MPCMMD_T || num_obs < 1) return fail(std::string(fn) + ": bad sizes");
+    return 0;
+}
+static int val_open(const char* fn, int device, int num_prime, int num_obs, size_t* smem) {
+    *smem = (size_t)(num_obs + 2) * num_prime * sizeof(int);
+    if (*smem > 200 * 1024) return fail(std::string(fn) + ": (num_obs + 2) * num_prime counters do not fit in shared memory");
+    CK(cudaSetDevice(device));
+    return 0;
+}
+
+static ValCfg val_cfg(int n_roll, int num_prime, int num_obs, int obs_cost_f32, double dt, double wheel_base, double a_obs, double b_obs,
+                      double y_lb, double y_ub) {
     ValCfg c;
     c.n_roll = n_roll; c.np = num_prime; c.O = num_obs; c.obs_f32 = obs_cost_f32; c.dt = dt; c.wheel_base = wheel_base;
     c.a2 = a_obs * a_obs; c.b2 = b_obs * b_obs; c.y_lb = y_lb; c.y_ub = y_ub;
-    k_validate<false><<<n_ep, VAL_THREADS, smem>>>(c, d_acc, d_steer, d_s0, d_xo, d_yo, d_cnt, d_lane, d_xr, d_yr, nullptr, nullptr);
-    return cudaGetLastError();
+    return c;
+}
+static ValJaxCfg val_jax_cfg(int noise_kind, double noise_level, double k_steer, double beta_a, double beta_b, double acc_const_noise,
+                             double steer_const_noise) {
+    ValJaxCfg j;
+    j.noise_kind = noise_kind; j.nl = noise_level; j.ks = k_steer * noise_level; j.beta_a = beta_a; j.beta_b = beta_b;
+    j.c_acc = acc_const_noise; j.c_steer = steer_const_noise;
+    return j;
 }
 
-extern "C" int mpcmmd_validate_host(int device, int n_ep, int n_roll, int num_prime, int num_obs, int obs_cost_f32, double dt, double wheel_base,
-                                    double a_obs, double b_obs, double y_lb, double y_ub, const double* acc, const double* steer,
-                                    const double* state0, const double* x_obs_traj, const double* y_obs_traj, int32_t* count,
-                                    int32_t* count_lane, double* x_roll, double* y_roll) {
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) return fail("mpcmmd_validate_host: no CUDA device (this library has no CPU fallback)");
-    if (device < 0 || device >= ndev) return fail("mpcmmd_validate_host: bad device index");
-    if (n_ep < 1 || n_roll < 1 || num_prime < 1 || num_prime > MPCMMD_T || num_obs < 1) return fail("mpcmmd_validate_host: bad sizes");
-    if (!acc || !steer || !state0 || !x_obs_traj || !y_obs_traj || !count || !count_lane) return fail("mpcmmd_validate_host: null pointer");
-    if ((x_roll == nullptr) != (y_roll == nullptr)) return fail("mpcmmd_validate_host: x_roll and y_roll must both be given or both be null");
-    const size_t smem = (size_t)(num_obs + 2) * num_prime * sizeof(int);
-    if (smem > 200 * 1024) return fail("mpcmmd_validate_host: (num_obs + 2) * num_prime counters do not fit in shared memory");
-    CK(cudaSetDevice(device));
-    const size_t nc = (size_t)n_ep * n_roll * num_prime, no = (size_t)n_ep * num_obs * num_prime;
-    double *d_acc = nullptr, *d_steer = nullptr, *d_s0 = nullptr, *d_xo = nullptr, *d_yo = nullptr, *d_xr = nullptr, *d_yr = nullptr;
-    int32_t *d_cnt = nullptr, *d_lane = nullptr;
-    int rc = 0;
-    auto body = [&]() -> int {
-        CK(cudaMalloc(&d_acc, nc * 8)); CK(cudaMalloc(&d_steer, nc * 8)); CK(cudaMalloc(&d_s0, (size_t)n_ep * 5 * 8));
-        CK(cudaMalloc(&d_xo, no * 8)); CK(cudaMalloc(&d_yo, no * 8)); CK(cudaMalloc(&d_cnt, (size_t)n_ep * 4)); CK(cudaMalloc(&d_lane, (size_t)n_ep * 4));
-        if (x_roll) { CK(cudaMalloc(&d_xr, nc * 8)); CK(cudaMalloc(&d_yr, nc * 8)); }
-        CK(cudaMemcpy(d_acc, acc, nc * 8, cudaMemcpyHostToDevice)); CK(cudaMemcpy(d_steer, steer, nc * 8, cudaMemcpyHostToDevice));
-        CK(cudaMemcpy(d_s0, state0, (size_t)n_ep * 5 * 8, cudaMemcpyHostToDevice));
-        CK(cudaMemcpy(d_xo, x_obs_traj, no * 8, cudaMemcpyHostToDevice)); CK(cudaMemcpy(d_yo, y_obs_traj, no * 8, cudaMemcpyHostToDevice));
-        CK(launch_validate(n_ep, n_roll, num_prime, num_obs, obs_cost_f32, dt, wheel_base, a_obs, b_obs, y_lb, y_ub, smem,
-                           d_acc, d_steer, d_s0, d_xo, d_yo, d_cnt, d_lane, d_xr, d_yr));
-        CK(cudaMemcpy(count, d_cnt, (size_t)n_ep * 4, cudaMemcpyDeviceToHost)); CK(cudaMemcpy(count_lane, d_lane, (size_t)n_ep * 4, cudaMemcpyDeviceToHost));
-        if (x_roll) { CK(cudaMemcpy(x_roll, d_xr, nc * 8, cudaMemcpyDeviceToHost)); CK(cudaMemcpy(y_roll, d_yr, nc * 8, cudaMemcpyDeviceToHost)); }
-        return 0;
-    };
-    rc = body();
-    cudaFree(d_acc); cudaFree(d_steer); cudaFree(d_s0); cudaFree(d_xo); cudaFree(d_yo); cudaFree(d_cnt); cudaFree(d_lane); cudaFree(d_xr); cudaFree(d_yr);
-    return rc;
+// k_validate on device-resident controls of n_ep plans (enqueue only).  Its shared-memory opt-in is raise-only, as the solve path's.
+template <bool RISK>
+static int launch_validate(int device, const ValCfg& c, int n_ep, size_t smem, const double* d_acc, const double* d_steer, const double* d_s0,
+                           const double* d_xo, const double* d_yo, int32_t* d_cnt, int32_t* d_lane, double* d_xr, double* d_yr, double* d_co,
+                           double* d_cl) {
+    if (raise_smem(device, (const void*)k_validate<RISK>, smem)) return -1;
+    k_validate<RISK><<<n_ep, VAL_THREADS, smem>>>(c, d_acc, d_steer, d_s0, d_xo, d_yo, d_cnt, d_lane, d_xr, d_yr, d_co, d_cl);
+    CK(cudaGetLastError());
+    return 0;
 }
 
-// The same with the noise drawn on the device (k_validate_noise): planned controls and per-trajectory seeds in, counts out.
-extern "C" int mpcmmd_validate_seeded_host(int device, int n_ep, int n_roll, int num_prime, int num_obs, int obs_cost_f32, int noise_kind,
-                                           double noise_level, double k_steer, double beta_a, double beta_b, double acc_const_noise,
-                                           double steer_const_noise, double dt, double wheel_base, double a_obs, double b_obs, double y_lb,
-                                           double y_ub, const uint32_t* seed, const double* acc_plan, const double* steer_plan,
-                                           const double* state0, const double* x_obs_traj, const double* y_obs_traj, int32_t* count,
-                                           int32_t* count_lane, double* acc_out, double* steer_out, uint32_t* state_out) {
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) return fail("mpcmmd_validate_seeded_host: no CUDA device (this library has no CPU fallback)");
-    if (device < 0 || device >= ndev) return fail("mpcmmd_validate_seeded_host: bad device index");
-    if (n_ep < 1 || n_roll < 1 || num_prime < 1 || num_prime > MPCMMD_T || num_obs < 1) return fail("mpcmmd_validate_seeded_host: bad sizes");
-    if (noise_kind != 0 && noise_kind != 1) return fail("mpcmmd_validate_seeded_host: noise_kind must be 0 (gaussian) or 1 (beta)");
-    if (!seed || !acc_plan || !steer_plan || !state0 || !x_obs_traj || !y_obs_traj || !count || !count_lane)
-        return fail("mpcmmd_validate_seeded_host: null pointer");
-    if ((acc_out == nullptr) != (steer_out == nullptr)) return fail("mpcmmd_validate_seeded_host: acc_out and steer_out must both be given or both be null");
-    if (noise_kind == 1) {                               // np.random.beta's argument check (NaN passes), before anything is drawn
-        for (size_t i = 0; i < (size_t)n_ep * num_prime; i++) {
-            if (beta_a * fabs(acc_plan[i]) <= 0.0 || beta_a * fabs(steer_plan[i]) + 1e-5 <= 0.0) return fail("mpcmmd_validate_seeded_host: a <= 0");
-            if (beta_b * fabs(acc_plan[i]) <= 0.0 || beta_b * fabs(steer_plan[i]) + 1e-5 <= 0.0) return fail("mpcmmd_validate_seeded_host: b <= 0");
-        }
-    }
-    const size_t smem = (size_t)(num_obs + 2) * num_prime * sizeof(int);
-    if (smem > 200 * 1024) return fail("mpcmmd_validate_seeded_host: (num_obs + 2) * num_prime counters do not fit in shared memory");
-    CK(cudaSetDevice(device));
-    const size_t nc = (size_t)n_ep * n_roll * num_prime, no = (size_t)n_ep * num_obs * num_prime, npl = (size_t)n_ep * num_prime;
-    double *d_ap = nullptr, *d_sp = nullptr, *d_acc = nullptr, *d_steer = nullptr, *d_s0 = nullptr, *d_xo = nullptr, *d_yo = nullptr;
-    uint32_t *d_seed = nullptr, *d_state = nullptr;
-    int32_t *d_cnt = nullptr, *d_lane = nullptr;
-    auto body = [&]() -> int {
-        CK(cudaMalloc(&d_seed, (size_t)n_ep * 4)); CK(cudaMalloc(&d_ap, npl * 8)); CK(cudaMalloc(&d_sp, npl * 8));
-        CK(cudaMalloc(&d_acc, nc * 8)); CK(cudaMalloc(&d_steer, nc * 8)); CK(cudaMalloc(&d_s0, (size_t)n_ep * 5 * 8));
-        CK(cudaMalloc(&d_xo, no * 8)); CK(cudaMalloc(&d_yo, no * 8)); CK(cudaMalloc(&d_cnt, (size_t)n_ep * 4)); CK(cudaMalloc(&d_lane, (size_t)n_ep * 4));
-        if (state_out) CK(cudaMalloc(&d_state, (size_t)n_ep * VALN_STATE_WORDS * 4));
-        CK(cudaMemcpy(d_seed, seed, (size_t)n_ep * 4, cudaMemcpyHostToDevice));
-        CK(cudaMemcpy(d_ap, acc_plan, npl * 8, cudaMemcpyHostToDevice)); CK(cudaMemcpy(d_sp, steer_plan, npl * 8, cudaMemcpyHostToDevice));
-        CK(cudaMemcpy(d_s0, state0, (size_t)n_ep * 5 * 8, cudaMemcpyHostToDevice));
-        CK(cudaMemcpy(d_xo, x_obs_traj, no * 8, cudaMemcpyHostToDevice)); CK(cudaMemcpy(d_yo, y_obs_traj, no * 8, cudaMemcpyHostToDevice));
-        ValNoiseCfg vn;
-        vn.n_roll = n_roll; vn.np = num_prime; vn.noise_kind = noise_kind; vn.nl = noise_level; vn.k_steer = k_steer;
-        vn.beta_a = beta_a; vn.beta_b = beta_b; vn.c_acc = acc_const_noise; vn.c_steer = steer_const_noise;
-        k_validate_noise<<<n_ep, VALN_THREADS>>>(vn, d_seed, d_ap, d_sp, d_acc, d_steer, d_state);
-        CK(cudaGetLastError());
-        CK(launch_validate(n_ep, n_roll, num_prime, num_obs, obs_cost_f32, dt, wheel_base, a_obs, b_obs, y_lb, y_ub, smem,
-                           d_acc, d_steer, d_s0, d_xo, d_yo, d_cnt, d_lane, nullptr, nullptr));
-        CK(cudaMemcpy(count, d_cnt, (size_t)n_ep * 4, cudaMemcpyDeviceToHost)); CK(cudaMemcpy(count_lane, d_lane, (size_t)n_ep * 4, cudaMemcpyDeviceToHost));
-        if (acc_out) { CK(cudaMemcpy(acc_out, d_acc, nc * 8, cudaMemcpyDeviceToHost)); CK(cudaMemcpy(steer_out, d_steer, nc * 8, cudaMemcpyDeviceToHost)); }
-        if (state_out) CK(cudaMemcpy(state_out, d_state, (size_t)n_ep * VALN_STATE_WORDS * 4, cudaMemcpyDeviceToHost));
-        return 0;
-    };
-    const int rc = body();
-    cudaFree(d_seed); cudaFree(d_ap); cudaFree(d_sp); cudaFree(d_acc); cudaFree(d_steer); cudaFree(d_s0); cudaFree(d_xo); cudaFree(d_yo);
-    cudaFree(d_cnt); cudaFree(d_lane); cudaFree(d_state);
-    return rc;
-}
-
-// The same with counter-based noise (k_validate_jax, DESIGN.md section 3 item 7): each rollout draws its JAX-protocol noise while it
-// rolls out, so n_roll is bounded only by JAX's uint32 element counters.
-extern "C" int mpcmmd_validate_threefry_host(int device, int n_ep, int n_roll, int num_prime, int num_obs, int obs_cost_f32, int noise_kind,
-                                             double noise_level, double k_steer, double beta_a, double beta_b, double acc_const_noise,
-                                             double steer_const_noise, double dt, double wheel_base, double a_obs, double b_obs, double y_lb,
-                                             double y_ub, const uint32_t* seed, const double* acc_plan, const double* steer_plan,
-                                             const double* state0, const double* x_obs_traj, const double* y_obs_traj, int32_t* count,
-                                             int32_t* count_lane, double* acc_out, double* steer_out) {
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) return fail("mpcmmd_validate_threefry_host: no CUDA device (this library has no CPU fallback)");
-    if (device < 0 || device >= ndev) return fail("mpcmmd_validate_threefry_host: bad device index");
-    if (n_roll < 1) return fail("mpcmmd_validate_threefry_host: n_roll must be >= 1");
-    if (n_ep < 1 || num_prime < 1 || num_prime > MPCMMD_T || num_obs < 1) return fail("mpcmmd_validate_threefry_host: bad sizes");
-    if ((long long)n_roll * num_prime >= (1LL << 31))
-        return fail("mpcmmd_validate_threefry_host: n_roll * num_prime must be below 2^31 (JAX's uint32 element counters)");
-    if (noise_kind != 0 && noise_kind != 1) return fail("mpcmmd_validate_threefry_host: noise_kind must be 0 (gaussian) or 1 (beta)");
-    if (!seed || !acc_plan || !steer_plan || !state0 || !x_obs_traj || !y_obs_traj || !count || !count_lane)
-        return fail("mpcmmd_validate_threefry_host: null pointer");
-    if ((acc_out == nullptr) != (steer_out == nullptr)) return fail("mpcmmd_validate_threefry_host: acc_out and steer_out must both be given or both be null");
-    const size_t smem = (size_t)(num_obs + 2) * num_prime * sizeof(int);
-    if (smem > 200 * 1024) return fail("mpcmmd_validate_threefry_host: (num_obs + 2) * num_prime counters do not fit in shared memory");
-    CK(cudaSetDevice(device));
-    const size_t nc = (size_t)n_ep * n_roll * num_prime, no = (size_t)n_ep * num_obs * num_prime, npl = (size_t)n_ep * num_prime;
-    const size_t ncnt = (size_t)n_ep * (num_obs + 2) * num_prime;
-    double *d_ap = nullptr, *d_sp = nullptr, *d_acc = nullptr, *d_steer = nullptr, *d_s0 = nullptr, *d_xo = nullptr, *d_yo = nullptr;
-    uint32_t* d_seed = nullptr;
-    int32_t *d_cg = nullptr, *d_cnt = nullptr, *d_lane = nullptr;
-    auto body = [&]() -> int {
-        CK(cudaMalloc(&d_seed, (size_t)n_ep * 4)); CK(cudaMalloc(&d_ap, npl * 8)); CK(cudaMalloc(&d_sp, npl * 8));
-        CK(cudaMalloc(&d_s0, (size_t)n_ep * 5 * 8)); CK(cudaMalloc(&d_xo, no * 8)); CK(cudaMalloc(&d_yo, no * 8));
-        CK(cudaMalloc(&d_cg, ncnt * 4)); CK(cudaMalloc(&d_cnt, (size_t)n_ep * 4)); CK(cudaMalloc(&d_lane, (size_t)n_ep * 4));
-        if (acc_out) { CK(cudaMalloc(&d_acc, nc * 8)); CK(cudaMalloc(&d_steer, nc * 8)); }
-        CK(cudaMemcpy(d_seed, seed, (size_t)n_ep * 4, cudaMemcpyHostToDevice));
-        CK(cudaMemcpy(d_ap, acc_plan, npl * 8, cudaMemcpyHostToDevice)); CK(cudaMemcpy(d_sp, steer_plan, npl * 8, cudaMemcpyHostToDevice));
-        CK(cudaMemcpy(d_s0, state0, (size_t)n_ep * 5 * 8, cudaMemcpyHostToDevice));
-        CK(cudaMemcpy(d_xo, x_obs_traj, no * 8, cudaMemcpyHostToDevice)); CK(cudaMemcpy(d_yo, y_obs_traj, no * 8, cudaMemcpyHostToDevice));
-        CK(cudaMemset(d_cg, 0, ncnt * 4));
-        if (smem > 48 * 1024) CK(cudaFuncSetAttribute(k_validate_jax<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        ValCfg c;
-        c.n_roll = n_roll; c.np = num_prime; c.O = num_obs; c.obs_f32 = obs_cost_f32; c.dt = dt; c.wheel_base = wheel_base;
-        c.a2 = a_obs * a_obs; c.b2 = b_obs * b_obs; c.y_lb = y_lb; c.y_ub = y_ub;
-        ValJaxCfg j;
-        j.noise_kind = noise_kind; j.nl = noise_level; j.ks = k_steer * noise_level; j.beta_a = beta_a; j.beta_b = beta_b;
-        j.c_acc = acc_const_noise; j.c_steer = steer_const_noise;
-        const unsigned chunks = (unsigned)((n_roll + VALJ_THREADS - 1) / VALJ_THREADS);
-        for (int e0 = 0; e0 < n_ep; e0 += 65535) {                      // gridDim.y <= 65535 trajectories per launch
-            const dim3 grid(chunks, (unsigned)(n_ep - e0 < 65535 ? n_ep - e0 : 65535));
-            k_validate_jax<false><<<grid, VALJ_THREADS, smem>>>(c, j, e0, d_seed, d_ap, d_sp, d_s0, d_xo, d_yo, d_cg, d_acc, d_steer, nullptr, nullptr);
-            CK(cudaGetLastError());
-        }
-        k_validate_finish<<<n_ep, 32>>>(num_obs, num_prime, d_cg, d_cnt, d_lane);
-        CK(cudaGetLastError());
-        CK(cudaMemcpy(count, d_cnt, (size_t)n_ep * 4, cudaMemcpyDeviceToHost)); CK(cudaMemcpy(count_lane, d_lane, (size_t)n_ep * 4, cudaMemcpyDeviceToHost));
-        if (acc_out) { CK(cudaMemcpy(acc_out, d_acc, nc * 8, cudaMemcpyDeviceToHost)); CK(cudaMemcpy(steer_out, d_steer, nc * 8, cudaMemcpyDeviceToHost)); }
-        return 0;
-    };
-    const int rc = body();
-    cudaFree(d_seed); cudaFree(d_ap); cudaFree(d_sp); cudaFree(d_acc); cudaFree(d_steer); cudaFree(d_s0); cudaFree(d_xo); cudaFree(d_yo);
-    cudaFree(d_cg); cudaFree(d_cnt); cudaFree(d_lane);
-    return rc;
-}
-
-// ------------------------------------------------------------------------------------------------
 // Monte-Carlo risk statistics (DESIGN.md section 3 item 9): each rollout's obstacle and lane costs (k_validate<true> / k_validate_jax<true>),
 // then k_risk_stats per plan.  The per-rollout arrays (16 B per rollout) live in a fixed device scratch: the plans run in chunks that fit it
 // (one plan at least), like k_inner_cem_big's chain ranges.  Every statistic depends on its plan alone, so the chunking changes no bit.
@@ -1093,15 +991,26 @@ static int risk_check(const char* fn, const mpcmmd_risk_out* r, int n_sets) {
     return 0;
 }
 
-// k_risk_stats on plans [e0, e0 + ne) whose per-rollout costs are in d_co / d_cl (ne, n) (overwritten); results to the host arrays of r
-static int risk_run_chunk(const mpcmmd_risk_out* r, int e0, int ne, int n, const double* d_sigma, double* d_co, double* d_cl, double* d_st,
-                          std::vector<double>& h_st) {
-    k_risk_stats<<<ne, RS_THREADS>>>(n, r->alpha, r->ker_wt, d_sigma ? d_sigma + e0 : nullptr, d_co, d_cl, d_st);
+// k_risk_stats' device side for chunks of `chunk` sets of n values: costs co, cl (chunk, n), results st (chunk, RS_OUT), the bandwidths
+// sigma (n_sets,) if r has them
+struct RiskScratch {
+    double *co = nullptr, *cl = nullptr, *st = nullptr, *sigma = nullptr;
+    std::vector<double> h_st;
+};
+static int risk_scratch(DeviceBuffers& m, const mpcmmd_risk_out* r, int n_sets, int chunk, int n, RiskScratch* s) {
+    const size_t rc = (size_t)chunk * n;
+    if (m.alloc(&s->co, rc) || m.alloc(&s->cl, rc) || m.alloc(&s->st, (size_t)chunk * RS_OUT)) return -1;
+    return r->sigma ? m.upload(&s->sigma, r->sigma, (size_t)n_sets) : 0;
+}
+
+// k_risk_stats on plans [e0, e0 + ne) whose per-rollout costs are in s.co / s.cl (ne, n) (overwritten); results to the host arrays of r
+static int risk_run_chunk(const mpcmmd_risk_out* r, RiskScratch& s, int e0, int ne, int n) {
+    k_risk_stats<<<ne, RS_THREADS>>>(n, r->alpha, r->ker_wt, s.sigma ? s.sigma + e0 : nullptr, s.co, s.cl, s.st);
     CK(cudaGetLastError());
-    h_st.resize((size_t)ne * RS_OUT);
-    CK(cudaMemcpy(h_st.data(), d_st, (size_t)ne * RS_OUT * 8, cudaMemcpyDeviceToHost));
+    s.h_st.resize((size_t)ne * RS_OUT);
+    CK(cudaMemcpy(s.h_st.data(), s.st, (size_t)ne * RS_OUT * 8, cudaMemcpyDeviceToHost));
     for (int i = 0; i < ne; i++) {
-        const double* q = &h_st[(size_t)i * RS_OUT];
+        const double* q = &s.h_st[(size_t)i * RS_OUT];
         r->p_coll[e0 + i] = q[0]; r->p_lane[e0 + i] = q[1]; r->mean_obs[e0 + i] = q[2]; r->var_obs[e0 + i] = q[3]; r->cvar_obs[e0 + i] = q[4];
         if (r->mmd_obs) r->mmd_obs[e0 + i] = q[5];
     }
@@ -1109,71 +1018,180 @@ static int risk_run_chunk(const mpcmmd_risk_out* r, int e0, int ne, int n, const
 }
 
 // the per-rollout costs of a chunk to the caller (before k_risk_stats overwrites them)
-static int risk_copy_costs(const mpcmmd_risk_out* r, int e0, int ne, int n_roll, const double* d_co, const double* d_cl) {
+static int risk_copy_costs(const mpcmmd_risk_out* r, const RiskScratch& s, int e0, int ne, int n_roll) {
     if (!r->c_obs) return 0;
     const size_t off = (size_t)e0 * n_roll, cnt = (size_t)ne * n_roll * 8;
-    CK(cudaMemcpy(r->c_obs + off, d_co, cnt, cudaMemcpyDeviceToHost));
-    CK(cudaMemcpy(r->c_lane + off, d_cl, cnt, cudaMemcpyDeviceToHost));
+    CK(cudaMemcpy(r->c_obs + off, s.co, cnt, cudaMemcpyDeviceToHost));
+    CK(cudaMemcpy(r->c_lane + off, s.cl, cnt, cudaMemcpyDeviceToHost));
     return 0;
 }
 
-static int risk_upload_sigma(const mpcmmd_risk_out* r, int n_ep, double** d_sigma) {
-    if (!r->sigma) return 0;
-    CK(cudaMalloc(d_sigma, (size_t)n_ep * 8));
-    CK(cudaMemcpy(*d_sigma, r->sigma, (size_t)n_ep * 8, cudaMemcpyHostToDevice));
+// Rollouts of host-drawn perturbed controls acc, steer (n_ep, c.n_roll, c.np) with k_validate: the counts, and the rollouts to x_roll,
+// y_roll if given.  With `risk` (checked) also the risk statistics: the plans run in chunks, and since host-drawn controls take 16 B per knot
+// and rollout on the device, they are uploaded chunk by chunk as well.  Without it the plans are one chunk.
+static int validate_host_controls(int device, int n_ep, size_t smem, const ValCfg& c, const double* acc, const double* steer, const double* state0,
+                                  const double* x_obs_traj, const double* y_obs_traj, int32_t* count, int32_t* count_lane, double* x_roll,
+                                  double* y_roll, const mpcmmd_risk_out* risk) {
+    const int chunk = risk ? risk_chunk(n_ep, c.n_roll, 16 + 16 * (size_t)c.np) : n_ep;
+    const size_t np = (size_t)c.np, nk_max = (size_t)chunk * c.n_roll * np, no = (size_t)n_ep * c.O * np;
+    DeviceBuffers m;
+    RiskScratch rs;
+    double *d_acc, *d_steer, *d_s0, *d_xo, *d_yo, *d_xr = nullptr, *d_yr = nullptr;
+    int32_t *d_cnt, *d_lane;
+    if (m.alloc(&d_acc, nk_max) || m.alloc(&d_steer, nk_max) || m.upload(&d_s0, state0, (size_t)n_ep * 5) || m.upload(&d_xo, x_obs_traj, no) ||
+        m.upload(&d_yo, y_obs_traj, no) || m.alloc(&d_cnt, n_ep) || m.alloc(&d_lane, n_ep))
+        return -1;
+    if (x_roll && (m.alloc(&d_xr, nk_max) || m.alloc(&d_yr, nk_max))) return -1;
+    if (risk && risk_scratch(m, risk, n_ep, chunk, c.n_roll, &rs)) return -1;
+    const auto launch = risk ? launch_validate<true> : launch_validate<false>;
+    for (int e0 = 0; e0 < n_ep; e0 += chunk) {
+        const int ne = n_ep - e0 < chunk ? n_ep - e0 : chunk;
+        const size_t k0 = (size_t)e0 * c.n_roll * np, nk = (size_t)ne * c.n_roll * np, oo = (size_t)e0 * c.O * np;
+        CK(cudaMemcpy(d_acc, acc + k0, nk * 8, cudaMemcpyHostToDevice)); CK(cudaMemcpy(d_steer, steer + k0, nk * 8, cudaMemcpyHostToDevice));
+        if (launch(device, c, ne, smem, d_acc, d_steer, d_s0 + (size_t)e0 * 5, d_xo + oo, d_yo + oo, d_cnt + e0, d_lane + e0, d_xr, d_yr, rs.co, rs.cl))
+            return -1;
+        if (risk && (risk_copy_costs(risk, rs, e0, ne, c.n_roll) || risk_run_chunk(risk, rs, e0, ne, c.n_roll))) return -1;
+    }
+    CK(cudaMemcpy(count, d_cnt, (size_t)n_ep * 4, cudaMemcpyDeviceToHost)); CK(cudaMemcpy(count_lane, d_lane, (size_t)n_ep * 4, cudaMemcpyDeviceToHost));
+    if (x_roll) { CK(cudaMemcpy(x_roll, d_xr, nk_max * 8, cudaMemcpyDeviceToHost)); CK(cudaMemcpy(y_roll, d_yr, nk_max * 8, cudaMemcpyDeviceToHost)); }
     return 0;
 }
 
-// mpcmmd_validate_host's rollouts and counts, plus the risk statistics.  Host-drawn controls take 16 B per knot and rollout on the device,
-// so they are uploaded chunk by chunk as well.
+// Counter-based noise (k_validate_jax, DESIGN.md section 3 item 7): each rollout draws its JAX-protocol noise while it rolls out, so n_roll
+// is bounded only by JAX's uint32 element counters.  The counts, and the perturbed controls to acc_out, steer_out if given.  With `risk`
+// (checked) also the risk statistics, the plans in chunks; without it the plans are one chunk.
+static int validate_counter_noise(int device, int n_ep, size_t smem, const ValCfg& c, const ValJaxCfg& j, const uint32_t* seed,
+                                  const double* acc_plan, const double* steer_plan, const double* state0, const double* x_obs_traj,
+                                  const double* y_obs_traj, int32_t* count, int32_t* count_lane, double* acc_out, double* steer_out,
+                                  const mpcmmd_risk_out* risk) {
+    const int chunk = risk ? risk_chunk(n_ep, c.n_roll, 16) : n_ep;
+    const size_t nc = (size_t)n_ep * c.n_roll * c.np, no = (size_t)n_ep * c.O * c.np, npl = (size_t)n_ep * c.np;
+    const size_t ncnt = (size_t)n_ep * (c.O + 2) * c.np;
+    DeviceBuffers m;
+    RiskScratch rs;
+    double *d_ap, *d_sp, *d_s0, *d_xo, *d_yo, *d_acc = nullptr, *d_steer = nullptr;
+    uint32_t* d_seed;
+    int32_t *d_cg, *d_cnt, *d_lane;
+    if (m.upload(&d_seed, seed, n_ep) || m.upload(&d_ap, acc_plan, npl) || m.upload(&d_sp, steer_plan, npl) || m.upload(&d_s0, state0, (size_t)n_ep * 5) ||
+        m.upload(&d_xo, x_obs_traj, no) || m.upload(&d_yo, y_obs_traj, no) || m.alloc(&d_cg, ncnt) || m.alloc(&d_cnt, n_ep) || m.alloc(&d_lane, n_ep))
+        return -1;
+    if (acc_out && (m.alloc(&d_acc, nc) || m.alloc(&d_steer, nc))) return -1;
+    if (risk && risk_scratch(m, risk, n_ep, chunk, c.n_roll, &rs)) return -1;
+    CK(cudaMemset(d_cg, 0, ncnt * 4));
+    const auto kern = risk ? k_validate_jax<true> : k_validate_jax<false>;
+    if (raise_smem(device, (const void*)kern, smem)) return -1;
+    const unsigned chunks = (unsigned)((c.n_roll + VALJ_THREADS - 1) / VALJ_THREADS);
+    for (int c0 = 0; c0 < n_ep; c0 += chunk) {
+        const int ne = n_ep - c0 < chunk ? n_ep - c0 : chunk;
+        for (int e0 = c0; e0 < c0 + ne; e0 += 65535) {                    // gridDim.y <= 65535 trajectories per launch
+            const dim3 grid(chunks, (unsigned)(c0 + ne - e0 < 65535 ? c0 + ne - e0 : 65535));
+            const size_t ro = (size_t)(e0 - c0) * c.n_roll;             // the risk costs are indexed by blockIdx.y
+            kern<<<grid, VALJ_THREADS, smem>>>(c, j, e0, d_seed, d_ap, d_sp, d_s0, d_xo, d_yo, d_cg, d_acc, d_steer, risk ? rs.co + ro : nullptr,
+                                               risk ? rs.cl + ro : nullptr);
+            CK(cudaGetLastError());
+        }
+        if (risk && (risk_copy_costs(risk, rs, c0, ne, c.n_roll) || risk_run_chunk(risk, rs, c0, ne, c.n_roll))) return -1;
+    }
+    k_validate_finish<<<n_ep, 32>>>(c.O, c.np, d_cg, d_cnt, d_lane);
+    CK(cudaGetLastError());
+    CK(cudaMemcpy(count, d_cnt, (size_t)n_ep * 4, cudaMemcpyDeviceToHost)); CK(cudaMemcpy(count_lane, d_lane, (size_t)n_ep * 4, cudaMemcpyDeviceToHost));
+    if (acc_out) { CK(cudaMemcpy(acc_out, d_acc, nc * 8, cudaMemcpyDeviceToHost)); CK(cudaMemcpy(steer_out, d_steer, nc * 8, cudaMemcpyDeviceToHost)); }
+    return 0;
+}
+
+extern "C" int mpcmmd_validate_host(int device, int n_ep, int n_roll, int num_prime, int num_obs, int obs_cost_f32, double dt, double wheel_base,
+                                    double a_obs, double b_obs, double y_lb, double y_ub, const double* acc, const double* steer,
+                                    const double* state0, const double* x_obs_traj, const double* y_obs_traj, int32_t* count,
+                                    int32_t* count_lane, double* x_roll, double* y_roll) {
+    const char* fn = "mpcmmd_validate_host";
+    size_t smem;
+    if (val_device(fn, device) || val_sizes(fn, n_ep, n_roll, num_prime, num_obs)) return -1;
+    if (!acc || !steer || !state0 || !x_obs_traj || !y_obs_traj || !count || !count_lane) return fail(std::string(fn) + ": null pointer");
+    if ((x_roll == nullptr) != (y_roll == nullptr)) return fail(std::string(fn) + ": x_roll and y_roll must both be given or both be null");
+    if (val_open(fn, device, num_prime, num_obs, &smem)) return -1;
+    return validate_host_controls(device, n_ep, smem, val_cfg(n_roll, num_prime, num_obs, obs_cost_f32, dt, wheel_base, a_obs, b_obs, y_lb, y_ub),
+                                  acc, steer, state0, x_obs_traj, y_obs_traj, count, count_lane, x_roll, y_roll, nullptr);
+}
+
+// The same with the noise drawn on the device (k_validate_noise): planned controls and per-trajectory seeds in, counts out.
+extern "C" int mpcmmd_validate_seeded_host(int device, int n_ep, int n_roll, int num_prime, int num_obs, int obs_cost_f32, int noise_kind,
+                                           double noise_level, double k_steer, double beta_a, double beta_b, double acc_const_noise,
+                                           double steer_const_noise, double dt, double wheel_base, double a_obs, double b_obs, double y_lb,
+                                           double y_ub, const uint32_t* seed, const double* acc_plan, const double* steer_plan,
+                                           const double* state0, const double* x_obs_traj, const double* y_obs_traj, int32_t* count,
+                                           int32_t* count_lane, double* acc_out, double* steer_out, uint32_t* state_out) {
+    const char* fn = "mpcmmd_validate_seeded_host";
+    size_t smem;
+    if (val_device(fn, device) || val_sizes(fn, n_ep, n_roll, num_prime, num_obs)) return -1;
+    if (noise_kind != 0 && noise_kind != 1) return fail(std::string(fn) + ": noise_kind must be 0 (gaussian) or 1 (beta)");
+    if (!seed || !acc_plan || !steer_plan || !state0 || !x_obs_traj || !y_obs_traj || !count || !count_lane) return fail(std::string(fn) + ": null pointer");
+    if ((acc_out == nullptr) != (steer_out == nullptr)) return fail(std::string(fn) + ": acc_out and steer_out must both be given or both be null");
+    if (noise_kind == 1) {                               // np.random.beta's argument check (NaN passes), before anything is drawn
+        for (size_t i = 0; i < (size_t)n_ep * num_prime; i++) {
+            if (beta_a * fabs(acc_plan[i]) <= 0.0 || beta_a * fabs(steer_plan[i]) + 1e-5 <= 0.0) return fail(std::string(fn) + ": a <= 0");
+            if (beta_b * fabs(acc_plan[i]) <= 0.0 || beta_b * fabs(steer_plan[i]) + 1e-5 <= 0.0) return fail(std::string(fn) + ": b <= 0");
+        }
+    }
+    if (val_open(fn, device, num_prime, num_obs, &smem)) return -1;
+    const size_t nc = (size_t)n_ep * n_roll * num_prime, no = (size_t)n_ep * num_obs * num_prime, npl = (size_t)n_ep * num_prime;
+    DeviceBuffers m;
+    double *d_ap, *d_sp, *d_acc, *d_steer, *d_s0, *d_xo, *d_yo;
+    uint32_t *d_seed, *d_state = nullptr;
+    int32_t *d_cnt, *d_lane;
+    if (m.upload(&d_seed, seed, n_ep) || m.upload(&d_ap, acc_plan, npl) || m.upload(&d_sp, steer_plan, npl) || m.alloc(&d_acc, nc) ||
+        m.alloc(&d_steer, nc) || m.upload(&d_s0, state0, (size_t)n_ep * 5) || m.upload(&d_xo, x_obs_traj, no) || m.upload(&d_yo, y_obs_traj, no) ||
+        m.alloc(&d_cnt, n_ep) || m.alloc(&d_lane, n_ep))
+        return -1;
+    if (state_out && m.alloc(&d_state, (size_t)n_ep * VALN_STATE_WORDS)) return -1;
+    ValNoiseCfg vn;
+    vn.n_roll = n_roll; vn.np = num_prime; vn.noise_kind = noise_kind; vn.nl = noise_level; vn.k_steer = k_steer;
+    vn.beta_a = beta_a; vn.beta_b = beta_b; vn.c_acc = acc_const_noise; vn.c_steer = steer_const_noise;
+    k_validate_noise<<<n_ep, VALN_THREADS>>>(vn, d_seed, d_ap, d_sp, d_acc, d_steer, d_state);
+    CK(cudaGetLastError());
+    if (launch_validate<false>(device, val_cfg(n_roll, num_prime, num_obs, obs_cost_f32, dt, wheel_base, a_obs, b_obs, y_lb, y_ub), n_ep, smem,
+                               d_acc, d_steer, d_s0, d_xo, d_yo, d_cnt, d_lane, nullptr, nullptr, nullptr, nullptr))
+        return -1;
+    CK(cudaMemcpy(count, d_cnt, (size_t)n_ep * 4, cudaMemcpyDeviceToHost)); CK(cudaMemcpy(count_lane, d_lane, (size_t)n_ep * 4, cudaMemcpyDeviceToHost));
+    if (acc_out) { CK(cudaMemcpy(acc_out, d_acc, nc * 8, cudaMemcpyDeviceToHost)); CK(cudaMemcpy(steer_out, d_steer, nc * 8, cudaMemcpyDeviceToHost)); }
+    if (state_out) CK(cudaMemcpy(state_out, d_state, (size_t)n_ep * VALN_STATE_WORDS * 4, cudaMemcpyDeviceToHost));
+    return 0;
+}
+
+// The same with counter-based noise (validate_counter_noise).
+extern "C" int mpcmmd_validate_threefry_host(int device, int n_ep, int n_roll, int num_prime, int num_obs, int obs_cost_f32, int noise_kind,
+                                             double noise_level, double k_steer, double beta_a, double beta_b, double acc_const_noise,
+                                             double steer_const_noise, double dt, double wheel_base, double a_obs, double b_obs, double y_lb,
+                                             double y_ub, const uint32_t* seed, const double* acc_plan, const double* steer_plan,
+                                             const double* state0, const double* x_obs_traj, const double* y_obs_traj, int32_t* count,
+                                             int32_t* count_lane, double* acc_out, double* steer_out) {
+    const char* fn = "mpcmmd_validate_threefry_host";
+    size_t smem;
+    if (val_device(fn, device)) return -1;
+    if (n_roll < 1) return fail(std::string(fn) + ": n_roll must be >= 1");
+    if (val_sizes(fn, n_ep, n_roll, num_prime, num_obs)) return -1;
+    if ((long long)n_roll * num_prime >= (1LL << 31)) return fail(std::string(fn) + ": n_roll * num_prime must be below 2^31 (JAX's uint32 element counters)");
+    if (noise_kind != 0 && noise_kind != 1) return fail(std::string(fn) + ": noise_kind must be 0 (gaussian) or 1 (beta)");
+    if (!seed || !acc_plan || !steer_plan || !state0 || !x_obs_traj || !y_obs_traj || !count || !count_lane) return fail(std::string(fn) + ": null pointer");
+    if ((acc_out == nullptr) != (steer_out == nullptr)) return fail(std::string(fn) + ": acc_out and steer_out must both be given or both be null");
+    if (val_open(fn, device, num_prime, num_obs, &smem)) return -1;
+    return validate_counter_noise(device, n_ep, smem, val_cfg(n_roll, num_prime, num_obs, obs_cost_f32, dt, wheel_base, a_obs, b_obs, y_lb, y_ub),
+                                  val_jax_cfg(noise_kind, noise_level, k_steer, beta_a, beta_b, acc_const_noise, steer_const_noise), seed, acc_plan,
+                                  steer_plan, state0, x_obs_traj, y_obs_traj, count, count_lane, acc_out, steer_out, nullptr);
+}
+
+// mpcmmd_validate_host's rollouts and counts, plus the risk statistics.
 extern "C" int mpcmmd_validate_risk_host(int device, int n_ep, int n_roll, int num_prime, int num_obs, int obs_cost_f32, double dt, double wheel_base,
                                          double a_obs, double b_obs, double y_lb, double y_ub, const double* acc, const double* steer,
                                          const double* state0, const double* x_obs_traj, const double* y_obs_traj, int32_t* count,
                                          int32_t* count_lane, const mpcmmd_risk_out* risk) {
     const char* fn = "mpcmmd_validate_risk_host";
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) return fail(std::string(fn) + ": no CUDA device (this library has no CPU fallback)");
-    if (device < 0 || device >= ndev) return fail(std::string(fn) + ": bad device index");
-    if (n_ep < 1 || n_roll < 1 || num_prime < 1 || num_prime > MPCMMD_T || num_obs < 1) return fail(std::string(fn) + ": bad sizes");
+    size_t smem;
+    if (val_device(fn, device) || val_sizes(fn, n_ep, n_roll, num_prime, num_obs)) return -1;
     if ((long long)n_roll * num_prime >= (1LL << 31)) return fail(std::string(fn) + ": n_roll * num_prime must be below 2^31");
     if (!acc || !steer || !state0 || !x_obs_traj || !y_obs_traj || !count || !count_lane) return fail(std::string(fn) + ": null pointer");
-    if (risk_check(fn, risk, n_ep)) return -1;
-    const size_t smem = (size_t)(num_obs + 2) * num_prime * sizeof(int);
-    if (smem > 200 * 1024) return fail(std::string(fn) + ": (num_obs + 2) * num_prime counters do not fit in shared memory");
-    CK(cudaSetDevice(device));
-    const int chunk = risk_chunk(n_ep, n_roll, 16 + 16 * (size_t)num_prime);
-    const size_t rc_ = (size_t)chunk * n_roll, np = (size_t)num_prime, no = (size_t)n_ep * num_obs * np;
-    double *d_acc = nullptr, *d_steer = nullptr, *d_s0 = nullptr, *d_xo = nullptr, *d_yo = nullptr, *d_co = nullptr, *d_cl = nullptr, *d_sigma = nullptr, *d_st = nullptr;
-    int32_t *d_cnt = nullptr, *d_lane = nullptr;
-    std::vector<double> h_st;
-    auto body = [&]() -> int {
-        CK(cudaMalloc(&d_acc, rc_ * np * 8)); CK(cudaMalloc(&d_steer, rc_ * np * 8)); CK(cudaMalloc(&d_s0, (size_t)n_ep * 5 * 8));
-        CK(cudaMalloc(&d_xo, no * 8)); CK(cudaMalloc(&d_yo, no * 8)); CK(cudaMalloc(&d_cnt, (size_t)n_ep * 4)); CK(cudaMalloc(&d_lane, (size_t)n_ep * 4));
-        CK(cudaMalloc(&d_co, rc_ * 8)); CK(cudaMalloc(&d_cl, rc_ * 8)); CK(cudaMalloc(&d_st, (size_t)chunk * RS_OUT * 8));
-        if (risk_upload_sigma(risk, n_ep, &d_sigma)) return -1;
-        CK(cudaMemcpy(d_s0, state0, (size_t)n_ep * 5 * 8, cudaMemcpyHostToDevice));
-        CK(cudaMemcpy(d_xo, x_obs_traj, no * 8, cudaMemcpyHostToDevice)); CK(cudaMemcpy(d_yo, y_obs_traj, no * 8, cudaMemcpyHostToDevice));
-        if (smem > 48 * 1024) CK(cudaFuncSetAttribute(k_validate<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        ValCfg c;
-        c.n_roll = n_roll; c.np = num_prime; c.O = num_obs; c.obs_f32 = obs_cost_f32; c.dt = dt; c.wheel_base = wheel_base;
-        c.a2 = a_obs * a_obs; c.b2 = b_obs * b_obs; c.y_lb = y_lb; c.y_ub = y_ub;
-        for (int e0 = 0; e0 < n_ep; e0 += chunk) {
-            const int ne = n_ep - e0 < chunk ? n_ep - e0 : chunk;
-            const size_t k0 = (size_t)e0 * n_roll * np, nk = (size_t)ne * n_roll * np, oo = (size_t)e0 * num_obs * np;
-            CK(cudaMemcpy(d_acc, acc + k0, nk * 8, cudaMemcpyHostToDevice)); CK(cudaMemcpy(d_steer, steer + k0, nk * 8, cudaMemcpyHostToDevice));
-            k_validate<true><<<ne, VAL_THREADS, smem>>>(c, d_acc, d_steer, d_s0 + (size_t)e0 * 5, d_xo + oo, d_yo + oo, d_cnt + e0, d_lane + e0,
-                                                         nullptr, nullptr, d_co, d_cl);
-            CK(cudaGetLastError());
-            if (risk_copy_costs(risk, e0, ne, n_roll, d_co, d_cl)) return -1;
-            if (risk_run_chunk(risk, e0, ne, n_roll, d_sigma, d_co, d_cl, d_st, h_st)) return -1;
-        }
-        CK(cudaMemcpy(count, d_cnt, (size_t)n_ep * 4, cudaMemcpyDeviceToHost)); CK(cudaMemcpy(count_lane, d_lane, (size_t)n_ep * 4, cudaMemcpyDeviceToHost));
-        return 0;
-    };
-    const int rc = body();
-    cudaFree(d_acc); cudaFree(d_steer); cudaFree(d_s0); cudaFree(d_xo); cudaFree(d_yo); cudaFree(d_cnt); cudaFree(d_lane);
-    cudaFree(d_co); cudaFree(d_cl); cudaFree(d_sigma); cudaFree(d_st);
-    return rc;
+    if (risk_check(fn, risk, n_ep) || val_open(fn, device, num_prime, num_obs, &smem)) return -1;
+    return validate_host_controls(device, n_ep, smem, val_cfg(n_roll, num_prime, num_obs, obs_cost_f32, dt, wheel_base, a_obs, b_obs, y_lb, y_ub),
+                                  acc, steer, state0, x_obs_traj, y_obs_traj, count, count_lane, nullptr, nullptr, risk);
 }
 
 // mpcmmd_validate_threefry_host's rollouts and counts, plus the risk statistics
@@ -1184,74 +1202,23 @@ extern "C" int mpcmmd_validate_threefry_risk_host(int device, int n_ep, int n_ro
                                                   const double* state0, const double* x_obs_traj, const double* y_obs_traj, int32_t* count,
                                                   int32_t* count_lane, const mpcmmd_risk_out* risk) {
     const char* fn = "mpcmmd_validate_threefry_risk_host";
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) return fail(std::string(fn) + ": no CUDA device (this library has no CPU fallback)");
-    if (device < 0 || device >= ndev) return fail(std::string(fn) + ": bad device index");
+    size_t smem;
+    if (val_device(fn, device)) return -1;
     if (n_roll < 1) return fail(std::string(fn) + ": n_roll must be >= 1");
-    if (n_ep < 1 || num_prime < 1 || num_prime > MPCMMD_T || num_obs < 1) return fail(std::string(fn) + ": bad sizes");
-    if ((long long)n_roll * num_prime >= (1LL << 31))
-        return fail(std::string(fn) + ": n_roll * num_prime must be below 2^31 (JAX's uint32 element counters)");
+    if (val_sizes(fn, n_ep, n_roll, num_prime, num_obs)) return -1;
+    if ((long long)n_roll * num_prime >= (1LL << 31)) return fail(std::string(fn) + ": n_roll * num_prime must be below 2^31 (JAX's uint32 element counters)");
     if (noise_kind != 0 && noise_kind != 1) return fail(std::string(fn) + ": noise_kind must be 0 (gaussian) or 1 (beta)");
     if (!seed || !acc_plan || !steer_plan || !state0 || !x_obs_traj || !y_obs_traj || !count || !count_lane) return fail(std::string(fn) + ": null pointer");
-    if (risk_check(fn, risk, n_ep)) return -1;
-    const size_t smem = (size_t)(num_obs + 2) * num_prime * sizeof(int);
-    if (smem > 200 * 1024) return fail(std::string(fn) + ": (num_obs + 2) * num_prime counters do not fit in shared memory");
-    CK(cudaSetDevice(device));
-    const int chunk = risk_chunk(n_ep, n_roll, 16);
-    const size_t rc_ = (size_t)chunk * n_roll, no = (size_t)n_ep * num_obs * num_prime, npl = (size_t)n_ep * num_prime;
-    const size_t ncnt = (size_t)n_ep * (num_obs + 2) * num_prime;
-    double *d_ap = nullptr, *d_sp = nullptr, *d_s0 = nullptr, *d_xo = nullptr, *d_yo = nullptr, *d_co = nullptr, *d_cl = nullptr, *d_sigma = nullptr, *d_st = nullptr;
-    uint32_t* d_seed = nullptr;
-    int32_t *d_cg = nullptr, *d_cnt = nullptr, *d_lane = nullptr;
-    std::vector<double> h_st;
-    auto body = [&]() -> int {
-        CK(cudaMalloc(&d_seed, (size_t)n_ep * 4)); CK(cudaMalloc(&d_ap, npl * 8)); CK(cudaMalloc(&d_sp, npl * 8));
-        CK(cudaMalloc(&d_s0, (size_t)n_ep * 5 * 8)); CK(cudaMalloc(&d_xo, no * 8)); CK(cudaMalloc(&d_yo, no * 8));
-        CK(cudaMalloc(&d_cg, ncnt * 4)); CK(cudaMalloc(&d_cnt, (size_t)n_ep * 4)); CK(cudaMalloc(&d_lane, (size_t)n_ep * 4));
-        CK(cudaMalloc(&d_co, rc_ * 8)); CK(cudaMalloc(&d_cl, rc_ * 8)); CK(cudaMalloc(&d_st, (size_t)chunk * RS_OUT * 8));
-        if (risk_upload_sigma(risk, n_ep, &d_sigma)) return -1;
-        CK(cudaMemcpy(d_seed, seed, (size_t)n_ep * 4, cudaMemcpyHostToDevice));
-        CK(cudaMemcpy(d_ap, acc_plan, npl * 8, cudaMemcpyHostToDevice)); CK(cudaMemcpy(d_sp, steer_plan, npl * 8, cudaMemcpyHostToDevice));
-        CK(cudaMemcpy(d_s0, state0, (size_t)n_ep * 5 * 8, cudaMemcpyHostToDevice));
-        CK(cudaMemcpy(d_xo, x_obs_traj, no * 8, cudaMemcpyHostToDevice)); CK(cudaMemcpy(d_yo, y_obs_traj, no * 8, cudaMemcpyHostToDevice));
-        CK(cudaMemset(d_cg, 0, ncnt * 4));
-        if (smem > 48 * 1024) CK(cudaFuncSetAttribute(k_validate_jax<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        ValCfg c;
-        c.n_roll = n_roll; c.np = num_prime; c.O = num_obs; c.obs_f32 = obs_cost_f32; c.dt = dt; c.wheel_base = wheel_base;
-        c.a2 = a_obs * a_obs; c.b2 = b_obs * b_obs; c.y_lb = y_lb; c.y_ub = y_ub;
-        ValJaxCfg j;
-        j.noise_kind = noise_kind; j.nl = noise_level; j.ks = k_steer * noise_level; j.beta_a = beta_a; j.beta_b = beta_b;
-        j.c_acc = acc_const_noise; j.c_steer = steer_const_noise;
-        const unsigned chunks = (unsigned)((n_roll + VALJ_THREADS - 1) / VALJ_THREADS);
-        for (int c0 = 0; c0 < n_ep; c0 += chunk) {
-            const int ne = n_ep - c0 < chunk ? n_ep - c0 : chunk;
-            for (int e0 = c0; e0 < c0 + ne; e0 += 65535) {                    // gridDim.y <= 65535 trajectories per launch
-                const int ny = c0 + ne - e0 < 65535 ? c0 + ne - e0 : 65535;
-                const size_t ro = (size_t)(e0 - c0) * n_roll;
-                k_validate_jax<true><<<dim3(chunks, (unsigned)ny), VALJ_THREADS, smem>>>(c, j, e0, d_seed, d_ap, d_sp, d_s0, d_xo, d_yo, d_cg,
-                                                                                      nullptr, nullptr, d_co + ro, d_cl + ro);
-                CK(cudaGetLastError());
-            }
-            if (risk_copy_costs(risk, c0, ne, n_roll, d_co, d_cl)) return -1;
-            if (risk_run_chunk(risk, c0, ne, n_roll, d_sigma, d_co, d_cl, d_st, h_st)) return -1;
-        }
-        k_validate_finish<<<n_ep, 32>>>(num_obs, num_prime, d_cg, d_cnt, d_lane);
-        CK(cudaGetLastError());
-        CK(cudaMemcpy(count, d_cnt, (size_t)n_ep * 4, cudaMemcpyDeviceToHost)); CK(cudaMemcpy(count_lane, d_lane, (size_t)n_ep * 4, cudaMemcpyDeviceToHost));
-        return 0;
-    };
-    const int rc = body();
-    cudaFree(d_seed); cudaFree(d_ap); cudaFree(d_sp); cudaFree(d_s0); cudaFree(d_xo); cudaFree(d_yo);
-    cudaFree(d_cg); cudaFree(d_cnt); cudaFree(d_lane); cudaFree(d_co); cudaFree(d_cl); cudaFree(d_sigma); cudaFree(d_st);
-    return rc;
+    if (risk_check(fn, risk, n_ep) || val_open(fn, device, num_prime, num_obs, &smem)) return -1;
+    return validate_counter_noise(device, n_ep, smem, val_cfg(n_roll, num_prime, num_obs, obs_cost_f32, dt, wheel_base, a_obs, b_obs, y_lb, y_ub),
+                                  val_jax_cfg(noise_kind, noise_level, k_steer, beta_a, beta_b, acc_const_noise, steer_const_noise), seed, acc_plan,
+                                  steer_plan, state0, x_obs_traj, y_obs_traj, count, count_lane, nullptr, nullptr, risk);
 }
 
 // k_risk_stats on caller-supplied costs: n_sets sets of n values each
 extern "C" int mpcmmd_risk_stats_host(int device, int n_sets, int n, const double* c_obs, const double* c_lane, const mpcmmd_risk_out* risk) {
     const char* fn = "mpcmmd_risk_stats_host";
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) return fail(std::string(fn) + ": no CUDA device (this library has no CPU fallback)");
-    if (device < 0 || device >= ndev) return fail(std::string(fn) + ": bad device index");
+    if (val_device(fn, device)) return -1;
     if (n_sets < 1 || n < 1) return fail(std::string(fn) + ": n_sets and n must be >= 1");
     if (!c_obs) return fail(std::string(fn) + ": null c_obs");
     if (risk_check(fn, risk, n_sets)) return -1;
@@ -1259,25 +1226,18 @@ extern "C" int mpcmmd_risk_stats_host(int device, int n_sets, int n, const doubl
         if (c_obs[i] < 0.0 || c_obs[i] == INFINITY) return fail(std::string(fn) + ": c_obs values must be >= 0 and finite, or NaN");
     CK(cudaSetDevice(device));
     const int chunk = risk_chunk(n_sets, n, 16);
-    const size_t rc_ = (size_t)chunk * n;
-    double *d_co = nullptr, *d_cl = nullptr, *d_sigma = nullptr, *d_st = nullptr;
-    std::vector<double> h_st;
-    auto body = [&]() -> int {
-        CK(cudaMalloc(&d_co, rc_ * 8)); CK(cudaMalloc(&d_cl, rc_ * 8)); CK(cudaMalloc(&d_st, (size_t)chunk * RS_OUT * 8));
-        if (risk_upload_sigma(risk, n_sets, &d_sigma)) return -1;
-        for (int e0 = 0; e0 < n_sets; e0 += chunk) {
-            const int ne = n_sets - e0 < chunk ? n_sets - e0 : chunk;
-            const size_t k0 = (size_t)e0 * n, nk = (size_t)ne * n;
-            CK(cudaMemcpy(d_co, c_obs + k0, nk * 8, cudaMemcpyHostToDevice));
-            if (c_lane) CK(cudaMemcpy(d_cl, c_lane + k0, nk * 8, cudaMemcpyHostToDevice));
-            else CK(cudaMemset(d_cl, 0, nk * 8));
-            if (risk_run_chunk(risk, e0, ne, n, d_sigma, d_co, d_cl, d_st, h_st)) return -1;
-        }
-        return 0;
-    };
-    const int rc = body();
-    cudaFree(d_co); cudaFree(d_cl); cudaFree(d_sigma); cudaFree(d_st);
-    return rc;
+    DeviceBuffers m;
+    RiskScratch rs;
+    if (risk_scratch(m, risk, n_sets, chunk, n, &rs)) return -1;
+    for (int e0 = 0; e0 < n_sets; e0 += chunk) {
+        const int ne = n_sets - e0 < chunk ? n_sets - e0 : chunk;
+        const size_t k0 = (size_t)e0 * n, nk = (size_t)ne * n;
+        CK(cudaMemcpy(rs.co, c_obs + k0, nk * 8, cudaMemcpyHostToDevice));
+        if (c_lane) CK(cudaMemcpy(rs.cl, c_lane + k0, nk * 8, cudaMemcpyHostToDevice));
+        else CK(cudaMemset(rs.cl, 0, nk * 8));
+        if (risk_run_chunk(risk, rs, e0, ne, n)) return -1;
+    }
+    return 0;
 }
 
 // ------------------------------------------------------------------------------------------------

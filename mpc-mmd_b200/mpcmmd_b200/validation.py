@@ -67,6 +67,48 @@ def perturbed_controls(prob, acc, steer, noise_level, num_prime, noise, key, n_r
     return acc + acc_pert + prob.acc_const_noise * z, steer + steer_pert + prob.steer_const_noise * z
 
 
+def _host_draws(prob, items, acc_p, steer_p, noise_level, num_prime, noise, n_roll):
+    """perturbed_controls of every item from its planned controls acc_p[i], steer_p[i] and seed item["key"]: (n, n_roll, num_prime) x2"""
+    acc = np.empty((len(items), n_roll, num_prime)); steer = np.empty((len(items), n_roll, num_prime))
+    for i, it in enumerate(items):
+        acc[i], steer[i] = perturbed_controls(prob, acc_p[i], steer_p[i], noise_level, num_prime, noise, it["key"], n_roll)
+    return acc, steer
+
+
+def _ptr(a):
+    return None if a is None else a.ctypes.data_as(C.c_void_p)
+
+
+def _device_index(prob, device):
+    """the CUDA device of a call: `device` if given, else the handle's"""
+    return (prob.device.index if device is None else int(device)) or 0
+
+
+def _geometry(prob):
+    """dt, wheel_base, a_obs, b_obs, y_lb, y_ub: the rollout and cost arguments of every validation entry point"""
+    return float(prob.t), float(prob.wheel_base), float(prob.a_obs), float(prob.b_obs), float(prob.y_lb), float(prob.y_ub)
+
+
+def _noise_args(prob, noise, noise_level):
+    """noise_kind, noise_level, K_steer, beta_a, beta_b, acc_const_noise, steer_const_noise: the noise arguments of the entry points that
+    draw on the device"""
+    return (B.NOISE_KINDS[noise], float(noise_level), float(prob.cem_helper.K_steer), float(prob.beta_a), float(prob.beta_b),
+            float(prob.acc_const_noise), float(prob.steer_const_noise))
+
+
+def _check_noise(noise):
+    if noise not in B.NOISE_KINDS:
+        raise ValueError("noise must be one of %s, not %r" % (sorted(B.NOISE_KINDS), noise))
+
+
+def _check_n_roll(n_roll, num_prime, why=""):
+    """n_roll an integer >= 1 with n_roll * num_prime below 2**31; `why` closes the second message"""
+    if isinstance(n_roll, bool) or not isinstance(n_roll, (int, np.integer)) or n_roll < 1:
+        raise ValueError("n_roll must be an integer >= 1, not %r" % (n_roll,))
+    if int(n_roll) * int(num_prime) >= 2 ** 31:
+        raise ValueError("n_roll * num_prime must be below 2**31" + why)
+
+
 def _inputs(prob, items, num_prime, num_obs):
     """per-trajectory inputs of the validation entry points: planned controls (n, num_prime) x2, state0 (n, 5), obstacle trajectories
     (n, num_obs, num_prime) x2, and whether the obstacle cost is float32 (static variant)"""
@@ -111,17 +153,13 @@ def compute_stats_batch(prob, items, num_prime, noise_level, noise, num_obs, wan
         z = np.zeros(0, np.int64)
         return (z, z, None, None) if want_rollouts else (z, z)
     acc_p, steer_p, state0, xo, yo, static = _inputs(prob, items, num_prime, num_obs)
-    acc_all = np.empty((n, n_roll, num_prime)); steer_all = np.empty((n, n_roll, num_prime))
-    for i, it in enumerate(items):
-        acc_all[i], steer_all[i] = perturbed_controls(prob, acc_p[i], steer_p[i], noise_level, num_prime, noise, it["key"], n_roll)
+    acc_all, steer_all = _host_draws(prob, items, acc_p, steer_p, noise_level, num_prime, noise, n_roll)
     count = np.zeros(n, np.int32); lane = np.zeros(n, np.int32)
     xr = np.empty((n, n_roll, num_prime)) if want_rollouts else None
     yr = np.empty((n, n_roll, num_prime)) if want_rollouts else None
-    dev = prob.device.index if device is None else int(device)
-    p = lambda a: None if a is None else a.ctypes.data_as(C.c_void_p)
-    B.check(B.load().mpcmmd_validate_host(dev or 0, n, n_roll, num_prime, num_obs, 1 if static else 0, float(prob.t), float(prob.wheel_base),
-                                          float(prob.a_obs), float(prob.b_obs), float(prob.y_lb), float(prob.y_ub), p(acc_all), p(steer_all),
-                                          p(state0), p(xo), p(yo), p(count), p(lane), p(xr), p(yr)))
+    B.check(B.load().mpcmmd_validate_host(_device_index(prob, device), n, n_roll, num_prime, num_obs, 1 if static else 0, *_geometry(prob),
+                                          _ptr(acc_all), _ptr(steer_all), _ptr(state0), _ptr(xo), _ptr(yo), _ptr(count), _ptr(lane), _ptr(xr),
+                                          _ptr(yr)))
     return (count, lane, xr, yr) if want_rollouts else (count, lane)
 
 
@@ -165,8 +203,7 @@ def seeded_stats_batch(prob, items, num_prime, noise_level, noise, num_obs, want
     the planned controls are computed here, each trajectory's stream is np.random.seed(item["key"]) restated on the device.
     Returns count, count_lane (n,) [, acc, steer (n, n_roll, num_prime) perturbed controls, state (n, 628) uint32 streams after the
     last draw = np.random.get_state()[1:] packed as key[624], pos, has_gauss, gauss bits]."""
-    if noise not in B.NOISE_KINDS:
-        raise ValueError("noise must be one of %s, not %r" % (sorted(B.NOISE_KINDS), noise))
+    _check_noise(noise)
     n = len(items)
     if n == 0:
         z = np.zeros(0, np.int64)
@@ -182,13 +219,9 @@ def seeded_stats_batch(prob, items, num_prime, noise_level, noise, num_obs, want
     acc = np.empty((n, n_roll, num_prime)) if want_draws else None
     steer = np.empty((n, n_roll, num_prime)) if want_draws else None
     state = np.empty((n, STATE_WORDS), np.uint32) if want_draws else None
-    dev = prob.device.index if device is None else int(device)
-    p = lambda a: None if a is None else a.ctypes.data_as(C.c_void_p)
     B.check(B.load().mpcmmd_validate_seeded_host(
-        dev or 0, n, n_roll, num_prime, num_obs, 1 if static else 0, B.NOISE_KINDS[noise], float(noise_level), float(prob.cem_helper.K_steer),
-        float(prob.beta_a), float(prob.beta_b), float(prob.acc_const_noise), float(prob.steer_const_noise), float(prob.t), float(prob.wheel_base),
-        float(prob.a_obs), float(prob.b_obs), float(prob.y_lb), float(prob.y_ub), p(seeds), p(acc_p), p(steer_p), p(state0), p(xo), p(yo),
-        p(count), p(lane), p(acc), p(steer), p(state)))
+        _device_index(prob, device), n, n_roll, num_prime, num_obs, 1 if static else 0, *_noise_args(prob, noise, noise_level), *_geometry(prob),
+        _ptr(seeds), _ptr(acc_p), _ptr(steer_p), _ptr(state0), _ptr(xo), _ptr(yo), _ptr(count), _ptr(lane), _ptr(acc), _ptr(steer), _ptr(state)))
     return (count, lane, acc, steer, state) if want_draws else (count, lane)
 
 
@@ -198,12 +231,8 @@ def threefry_stats_batch(prob, items, num_prime, noise_level, noise, num_obs, wa
     array, drawn by each rollout as it rolls out.  No shape parameter check (JAX makes none: at num_prime = 100 the acceleration
     draws of the last knot are NaN and reach only the discarded final state).  Returns count, count_lane (n,) [, acc, steer
     (n, n_roll, num_prime) perturbed controls]."""
-    if noise not in B.NOISE_KINDS:
-        raise ValueError("noise must be one of %s, not %r" % (sorted(B.NOISE_KINDS), noise))
-    if isinstance(n_roll, bool) or not isinstance(n_roll, (int, np.integer)) or n_roll < 1:
-        raise ValueError("n_roll must be an integer >= 1, not %r" % (n_roll,))
-    if int(n_roll) * int(num_prime) >= 2 ** 31:
-        raise ValueError("n_roll * num_prime must be below 2**31 (JAX's uint32 element counters)")
+    _check_noise(noise)
+    _check_n_roll(n_roll, num_prime, " (JAX's uint32 element counters)")
     n = len(items)
     if n == 0:
         z = np.zeros(0, np.int64)
@@ -213,13 +242,9 @@ def threefry_stats_batch(prob, items, num_prime, noise_level, noise, num_obs, wa
     count = np.zeros(n, np.int32); lane = np.zeros(n, np.int32)
     acc = np.empty((n, n_roll, num_prime)) if want_draws else None
     steer = np.empty((n, n_roll, num_prime)) if want_draws else None
-    dev = prob.device.index if device is None else int(device)
-    p = lambda a: None if a is None else a.ctypes.data_as(C.c_void_p)
     B.check(B.load().mpcmmd_validate_threefry_host(
-        dev or 0, n, int(n_roll), num_prime, num_obs, 1 if static else 0, B.NOISE_KINDS[noise], float(noise_level), float(prob.cem_helper.K_steer),
-        float(prob.beta_a), float(prob.beta_b), float(prob.acc_const_noise), float(prob.steer_const_noise), float(prob.t), float(prob.wheel_base),
-        float(prob.a_obs), float(prob.b_obs), float(prob.y_lb), float(prob.y_ub), p(seeds), p(acc_p), p(steer_p), p(state0), p(xo), p(yo),
-        p(count), p(lane), p(acc), p(steer)))
+        _device_index(prob, device), n, int(n_roll), num_prime, num_obs, 1 if static else 0, *_noise_args(prob, noise, noise_level), *_geometry(prob),
+        _ptr(seeds), _ptr(acc_p), _ptr(steer_p), _ptr(state0), _ptr(xo), _ptr(yo), _ptr(count), _ptr(lane), _ptr(acc), _ptr(steer)))
     return (count, lane, acc, steer) if want_draws else (count, lane)
 
 
@@ -269,12 +294,8 @@ def risk_stats_batch(prob, items, num_prime, noise_level, noise, num_obs, n_roll
         raise ValueError("risk_stats_batch: rng='device' has no risk statistics (its draws are NumPy's: use rng='host')")
     if rng not in ("host", "jax"):
         raise ValueError("risk_stats_batch: rng must be 'host' or 'jax', not %r" % (rng,))
-    if noise not in B.NOISE_KINDS:
-        raise ValueError("noise must be one of %s, not %r" % (sorted(B.NOISE_KINDS), noise))
-    if isinstance(n_roll, bool) or not isinstance(n_roll, (int, np.integer)) or n_roll < 1:
-        raise ValueError("n_roll must be an integer >= 1, not %r" % (n_roll,))
-    if int(n_roll) * int(num_prime) >= 2 ** 31:
-        raise ValueError("n_roll * num_prime must be below 2**31")
+    _check_noise(noise)
+    _check_n_roll(n_roll, num_prime)
     alpha = _check_alpha(alpha)
     n = len(items)
     if sigma is not None:
@@ -289,20 +310,15 @@ def risk_stats_batch(prob, items, num_prime, noise_level, noise, num_obs, n_roll
     if n == 0:
         return out
     acc_p, steer_p, state0, xo, yo, static = _inputs(prob, items, num_prime, num_obs)
-    dev = prob.device.index if device is None else int(device)
-    p = lambda a: None if a is None else a.ctypes.data_as(C.c_void_p)
-    geom = (float(prob.t), float(prob.wheel_base), float(prob.a_obs), float(prob.b_obs), float(prob.y_lb), float(prob.y_ub))
+    dev = _device_index(prob, device)
     if rng == "host":
-        acc_all = np.empty((n, n_roll, num_prime)); steer_all = np.empty((n, n_roll, num_prime))
-        for i, it in enumerate(items):
-            acc_all[i], steer_all[i] = perturbed_controls(prob, acc_p[i], steer_p[i], noise_level, num_prime, noise, it["key"], n_roll)
-        B.check(B.load().mpcmmd_validate_risk_host(dev or 0, n, n_roll, num_prime, num_obs, 1 if static else 0, *geom, p(acc_all), p(steer_all),
-                                                   p(state0), p(xo), p(yo), p(count), p(lane), C.byref(r)))
+        acc_all, steer_all = _host_draws(prob, items, acc_p, steer_p, noise_level, num_prime, noise, n_roll)
+        B.check(B.load().mpcmmd_validate_risk_host(dev, n, n_roll, num_prime, num_obs, 1 if static else 0, *_geometry(prob), _ptr(acc_all),
+                                                   _ptr(steer_all), _ptr(state0), _ptr(xo), _ptr(yo), _ptr(count), _ptr(lane), C.byref(r)))
     else:
         B.check(B.load().mpcmmd_validate_threefry_risk_host(
-            dev or 0, n, n_roll, num_prime, num_obs, 1 if static else 0, B.NOISE_KINDS[noise], float(noise_level), float(prob.cem_helper.K_steer),
-            float(prob.beta_a), float(prob.beta_b), float(prob.acc_const_noise), float(prob.steer_const_noise), *geom, p(seeds), p(acc_p),
-            p(steer_p), p(state0), p(xo), p(yo), p(count), p(lane), C.byref(r)))
+            dev, n, n_roll, num_prime, num_obs, 1 if static else 0, *_noise_args(prob, noise, noise_level), *_geometry(prob), _ptr(seeds),
+            _ptr(acc_p), _ptr(steer_p), _ptr(state0), _ptr(xo), _ptr(yo), _ptr(count), _ptr(lane), C.byref(r)))
     return out
 
 
@@ -326,8 +342,7 @@ def risk_stats(c_obs, c_lane=None, alpha=0.98, sigma=None, ker_wt=1000.0, device
     if sigma is not None:
         sigma = _check_sigma(np.reshape(sigma, -1) if np.ndim(sigma) else sigma, n_sets)
     r, out = _risk_struct(shape, alpha, ker_wt, sigma)
-    p = lambda a: None if a is None else a.ctypes.data_as(C.c_void_p)
-    B.check(B.load().mpcmmd_risk_stats_host(int(device), n_sets, n, p(co), p(cl), C.byref(r)))
+    B.check(B.load().mpcmmd_risk_stats_host(int(device), n_sets, n, _ptr(co), _ptr(cl), C.byref(r)))
     return out
 
 

@@ -163,8 +163,7 @@ def _validate_host(V, B, prob, items, num_prime, num_obs, acc, steer):
     _, _, state0, xo, yo, static = V._inputs(prob, items, num_prime, num_obs)
     n, n_roll = acc.shape[:2]
     count, lane = np.zeros(n, np.int32), np.zeros(n, np.int32)
-    B.check(B.load().mpcmmd_validate_host(0, n, n_roll, num_prime, num_obs, 1 if static else 0, float(prob.t), float(prob.wheel_base),
-                                          float(prob.a_obs), float(prob.b_obs), float(prob.y_lb), float(prob.y_ub), _p(np.ascontiguousarray(acc)),
+    B.check(B.load().mpcmmd_validate_host(0, n, n_roll, num_prime, num_obs, 1 if static else 0, *V._geometry(prob), _p(np.ascontiguousarray(acc)),
                                           _p(np.ascontiguousarray(steer)), _p(state0), _p(xo), _p(yo), _p(count), _p(lane), None, None))
     return count, lane
 

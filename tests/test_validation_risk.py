@@ -268,25 +268,40 @@ def test_stats_kernel_edge_cases(built):
     assert float(one["var_obs"]) == 0.25 and float(one["p_lane"]) == 0.0 and "mmd_obs" not in one
 
 
-@pytest.mark.gpu
-def test_chunked_call_equals_separate_calls(built):
-    """700 plans x 10^5 rollouts of counter-based noise (1.1 GB of per-rollout costs, beyond the 1 GiB scratch: two chunks) give the
-    statistics, bit for bit, of the same plans validated in separate calls, on both sides of the chunk boundary"""
+def _chunked_equals_separate(rng, n_roll, knot_bytes):
+    """700 plans of S_beta at n_roll rollouts, each rollout taking 16 B of costs plus knot_bytes per knot of device scratch, more than the
+    1 GiB scratch (two chunks): the statistics and counts, bit for bit, of the same plans validated in separate calls, on both sides of
+    the chunk boundary"""
     _need_gpu()
     from mpcmmd_b200 import validation as V
     g, _ = _cases()
     names, prob, num_obs, noise_level, num_prime, noise = _group(g, "S_beta")
     base = _items(g, names[:1])[0]
     items = [dict(base, key=k) for k in range(700)]
-    n_roll = 100000
-    assert len(items) * n_roll * 16 > 2 ** 30
-    kw = dict(n_roll=n_roll, rng="jax", sigma=0.05, device=0)
+    per_roll = 16 + knot_bytes * num_prime
+    assert len(items) * n_roll * per_roll > 2 ** 30
+    edge = 2 ** 30 // per_roll // n_roll                                  # plans per chunk
+    kw = dict(n_roll=n_roll, rng=rng, sigma=0.05, device=0)
     full = V.risk_stats_batch(prob, items, num_prime, noise_level, noise, num_obs, **kw)
     assert np.any(full["p_coll"] > 0)
-    for lo, hi in ((0, 3), (668, 674), (697, 700)):
+    for lo, hi in ((0, 3), (edge - 3, edge + 3), (697, 700)):
         part = V.risk_stats_batch(prob, items[lo:hi], num_prime, noise_level, noise, num_obs, **kw)
         for k in STATS + ("mmd_obs", "count", "count_lane"):
             assert full[k][lo:hi].tobytes() == part[k].tobytes(), (k, lo, hi)
+
+
+@pytest.mark.gpu
+def test_chunked_call_equals_separate_calls(built):
+    """700 plans x 10^5 rollouts of counter-based noise (1.1 GB of per-rollout costs, beyond the 1 GiB scratch: two chunks of 671 and 29
+    plans) give the statistics, bit for bit, of the same plans validated in separate calls, on both sides of the chunk boundary"""
+    _chunked_equals_separate("jax", 100000, 0)
+
+
+@pytest.mark.gpu
+def test_chunked_host_draws_equal_separate_calls(built):
+    """the same with NumPy's noise drawn on the host: 700 plans x 2000 rollouts, each taking 16 B of per-rollout costs plus 16 B per knot
+    of uploaded controls (1.1 GB at num_prime = 50: two chunks of 657 and 43 plans)"""
+    _chunked_equals_separate("host", 2000, 16)
 
 
 @pytest.mark.gpu

@@ -161,8 +161,7 @@ def _host_counts(V, B, prob, items, num_prime, acc, steer):
     _, _, state0, xo, yo, static = V._inputs(prob, items, num_prime, prob.num_obs)
     n = len(items)
     count, lane = np.zeros(n, np.int32), np.zeros(n, np.int32)
-    B.check(B.load().mpcmmd_validate_host(prob.device.index or 0, n, 1000, num_prime, prob.num_obs, 1 if static else 0, float(prob.t),
-                                          float(prob.wheel_base), float(prob.a_obs), float(prob.b_obs), float(prob.y_lb), float(prob.y_ub),
+    B.check(B.load().mpcmmd_validate_host(prob.device.index or 0, n, 1000, num_prime, prob.num_obs, 1 if static else 0, *V._geometry(prob),
                                           _p(acc), _p(steer), _p(state0), _p(xo), _p(yo), _p(count), _p(lane), None, None))
     return count, lane
 
